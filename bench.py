@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the restrictive-hierarchy head + loss + metrics path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 One "step" = the body of the reference's train_epoch (train.py:201-241) minus the donor backbone and the optimiser,
 on synthetic per-level donor features:
@@ -9,8 +9,15 @@ on synthetic per-level donor features:
     CE + Dice per level + consistency  ->  backward to per-level dfeats and head / FiLM parameter gradients.
 `value` is whole-job Mpixel/s (B*H*W pixels per step per GPU) with inputs resident in HBM; `e2e` is the same step
 driven from pinned HOST buffers (H2D of the step's features and targets and D2H of the loss + metrics inside the timed
-region).  The timed block of K steps is repeated (>= 10 times, >= 100 ms in total) and the MEDIAN block is reported.
-`configs` holds one short measurement of every other BASELINE.json configuration (same step, same timing).
+region).  The headline (`value`, `ms_per_step`) times exactly K steps, back to back, with a CUDA event between
+consecutive steps, and reports the MEDIAN step; the secondary timings (`e2e`, `dropin_modules`, `roofline`) take their
+own step counts, derived from K.  `configs` holds one short measurement of every other BASELINE.json configuration.
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float32, or float64 for
+the int64 confusion matrices and fp64 buffers): loss, scalars, per-level ratios / confusion / probs / logits, and the
+gradients of every input.  Arrays too large to keep whole are stored as a fixed, seeded sample of their flattened
+elements (files named *_sampled.npy), at most 64 MB in all.  Inputs are seeded, so two builds run with the same
+arguments can be compared file for file.
 
 Prints ONE JSON line on rank 0.  `--impl reference` times the reference's own modules (oracle/_ref: byte copies of
 Models/, Metrics/, train.py staged by tools/stage_reference.py) on the host cores, same workload, same batch.
@@ -23,10 +30,12 @@ import subprocess
 import sys
 import tempfile
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import torch  # noqa: E402
 
@@ -165,7 +174,8 @@ class GpuStep:
         h = data["host"]
         self.target = h["target"].to(device)
         self.one = torch.ones((), device=device)  # d(loss)/d(loss), allocated once instead of a fill per step
-        self.result = self.global_summary = None
+        self.result = self.global_summary = self.maps = None
+        self.keep_maps = False  # hold the step's probabilities and logits for --dump-outputs
         if self.flat:
             self.logits = h["logits"].to(device).requires_grad_(True)
             self.fused = rhseg_b200.FusedFlatStep(wl["K"], data["weights"][0])
@@ -194,7 +204,7 @@ class GpuStep:
 
     def step(self):
         """Fused step (rhseg_b200.FusedHierStep / FusedFlatStep): the whole train_epoch body in one autograd node."""
-        self.grads = None  # free the previous step's gradient tensors first (they are GBs for the large batches)
+        self.grads = self.maps = None  # free the previous step's gradient tensors first (they are GBs for the large batches)
         if self.flat:
             out = self.fused(self.logits, self.target)
             self.grads = torch.autograd.grad(out.loss, [self.logits], grad_outputs=self.one)
@@ -204,6 +214,8 @@ class GpuStep:
             leaves = self.feats + [p for grp in self.params for p in grp]
             self.grads = torch.autograd.grad(out.loss, leaves, grad_outputs=self.one)  # dfeats per level + head / FiLM parameter grads
         self.result = (out.scalars, out.ratios)
+        if self.keep_maps:  # not out.loss: it would keep the autograd graph of the step alive
+            self.maps = (out.probs, out.logits)
         self.confusion, self.summary, self.exchange, self.global_summary = out.confusion, out.summary, out.exchange, out.global_summary
         return self.result
 
@@ -382,25 +394,20 @@ class Harness:
         else:
             self.full_step()
 
-    def timed_blocks(self, steps, min_blocks=10, min_total_ms=100.0, max_blocks=60):
-        """Blocks of exactly `steps` steps, each bracketed by barrier + synchronize on both sides and timed with CUDA
-        events on the launching stream; max over ranks per block.  Returns the per-step ms of every block."""
-        out = []
-        total = 0.0
-        while len(out) < min_blocks or (total < min_total_ms and len(out) < max_blocks):
-            self.barrier()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(steps):
-                self.one_step()
-            e1.record()
-            self.barrier()
-            t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=self.dev)
-            if self.world > 1:
-                torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
-            out.append(t.item() / steps)
-            total += t.item()
-        return out
+    def timed_steps(self, steps):
+        """Exactly `steps` steps back to back between one barrier + synchronize on each side, a CUDA event on the
+        launching stream before the first and after every step; max over ranks per step.  Returns the ms of every step."""
+        self.barrier()
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(steps + 1)]
+        ev[0].record()
+        for i in range(steps):
+            self.one_step()
+            ev[i + 1].record()
+        self.barrier()
+        t = torch.tensor([ev[i].elapsed_time(ev[i + 1]) for i in range(steps)], dtype=torch.float64, device=self.dev)
+        if self.world > 1:
+            torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
+        return t.tolist()
 
     def close(self):
         self.graph = None
@@ -528,9 +535,9 @@ def measure_extra(args, name, rank, world, dev, peaks):
         hz.one_step()
     torch.cuda.synchronize()
     big = wl.get("strong") and world < 4
-    steps = 3 if big else 10
-    blocks = hz.timed_blocks(steps, min_blocks=5 if big else 10, min_total_ms=60.0, max_blocks=30)
-    ms = statistics.median(blocks)
+    steps = 15 if big else 100
+    times = hz.timed_steps(steps)
+    ms = statistics.median(times)
     alg = algorithmic_bytes(wl, hz.B)
     px_total = sum(local_batch(wl, world, r) for r in range(world)) * wl["H"] * wl["W"]
     # dominant kernel, timed alone as back-to-back launches
@@ -538,7 +545,7 @@ def measure_extra(args, name, rank, world, dev, peaks):
     graph_used = hz.graph is not None
     hz.close()
     res = {"workload": name, "baseline_config": wl["cfg"], "scaling": "strong" if wl.get("strong") else "weak",
-           "batch_per_gpu": hz.B, "ms_per_step": ms, "ms_per_step_min": min(blocks), "blocks": len(blocks), "steps_per_block": steps,
+           "batch_per_gpu": hz.B, "ms_per_step": ms, "ms_per_step_min": min(times), "timed_steps": steps,
            "Mpx/s": px_total / (ms * 1e-3) / 1e6,
            "whole_step_frac": (alg["step"] + alg["metrics"]) / (ms * 1e-3) / 1e9 / peaks["hbm_gbs"],
            "head_loss_fwd_bwd_frac": alg["step"] / (ms * 1e-3) / 1e9 / peaks["hbm_gbs"],
@@ -632,6 +639,7 @@ def run_ours(args, rank, world, local_rank):
     strong_big = wl.get("strong") and world < 4
     hz = Harness(args, name, rank, world, dev, pin_host=not strong_big)
     st, B = hz.st, hz.B
+    st.keep_maps = bool(args.dump_outputs) and rank == 0
     upsampled = wl["scale"] != 1
     alg = algorithmic_bytes(wl, B)
 
@@ -678,8 +686,10 @@ def run_ours(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    blocks = hz.timed_blocks(args.steps)
-    ms = statistics.median(blocks)
+    times = hz.timed_steps(args.steps)
+    ms = statistics.median(times)
+    dumped = collect_outputs(hz) if st.keep_maps else None
+    st.keep_maps, st.maps = False, None
     counted["n"] = 0
     hz.full_step()  # one eager step: the launches of a step, counted
     launches_per_step = counted["n"]
@@ -769,9 +779,9 @@ def run_ours(args, rank, world, local_rank):
         "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": ms,
         "higher_is_better": True, "scaling": "strong" if wl.get("strong") else "weak", "vs_baseline": None, "dtype": "f32",
         "data": "synthetic", "config": config_of(name, wl, world),
-        "timing": {"blocks": len(blocks), "steps_per_block": args.steps, "ms_per_step_median": ms, "ms_per_step_min": min(blocks),
-                   "ms_per_step_max": max(blocks), "timed_ms_total": sum(blocks) * args.steps,
-                   "how": "each block: barrier + synchronize, CUDA events around K graph replays, barrier + synchronize; max over ranks; median block reported"},
+        "timing": {"timed_steps": len(times), "ms_per_step_median": ms, "ms_per_step_min": min(times),
+                   "ms_per_step_max": max(times), "timed_ms_total": sum(times),
+                   "how": "barrier + synchronize, K steps (graph replays when captured) back to back with a CUDA event before the first and after each, barrier + synchronize; max over ranks per step; median step reported"},
         "run": {"api": "fused step (rhseg_b200.FusedHierStep)" if not st.flat else "fused flat step (rhseg_b200.FusedFlatStep)",
                 "cuda_graph": graph_used, "loss": loss_value,
                 "collective": ("summary all-reduce between fwd and bwd + head/FiLM gradient all-reduce after bwd, %s"
@@ -822,6 +832,8 @@ def run_ours(args, rank, world, local_rank):
                 line["configs"].append(measure_extra(args, extra, rank, world, dev, peaks))
     if world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_reference(name, wl, B, steps=3, warmup=1)  # ~20-30 s of host work
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     return line
 
 
@@ -910,6 +922,56 @@ def time_e2e(args, hz):
             "h2d_GBps_per_rank": [h2d / (m * 1e-3) / 1e9 for m in per_rank],
             "note": "features (fp32) + ternary targets (int8, widened on the device) copied from pinned host memory every step "
                     "(copy of step i+1 overlaps step i); PCIe-bound"}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def collect_outputs(hz):
+    """Host copies of what the last step returned to its caller, name -> tensor (float32, or float64 for int64 and fp64
+    results).  Arrays beyond a fair share of DUMP_BYTES keep a sample of their flattened elements at fixed, seeded
+    positions: the same positions in every run with the same arguments."""
+    st = hz.st
+    scalars, ratios = st.result
+    arrays = {"loss": scalars[:1], "scalars": scalars}  # StepOutput.loss is scalars[0]
+    for L in range(len(ratios)):
+        arrays["ratios_L%d" % L] = ratios[L]
+        arrays["confusion_L%d" % L] = st.confusion[L]
+    if st.flat:
+        arrays["grad_logits"] = st.grads[0]
+    else:
+        for L in range(len(ratios)):
+            arrays["probs_L%d" % L] = st.maps[0][L]
+            arrays["logits_L%d" % L] = st.maps[1][L]
+            arrays["grad_feats_L%d" % L] = st.grads[L]
+        names = ["grad_%s_%d" % (key, i) for key, grp in zip(("head_w", "head_b", "film_w", "film_b"), st.params)
+                 for i in range(len(grp))]
+        arrays.update(zip(names, st.grads[len(st.feats):]))
+        if hz.world > 1:
+            arrays["exchange"] = st.exchange  # the step summary and the parameter gradients summed over the ranks
+    large = [k for k, t in arrays.items() if t.numel() > 65536]
+    small_bytes = sum(t.numel() * 8 for k, t in arrays.items() if k not in large)
+    share = (DUMP_BYTES - small_bytes) // max(len(large), 1)  # bytes per large array
+    res = {}
+    for k, t in arrays.items():
+        t = t.detach()
+        wide = t.dtype in (torch.float64, torch.int64, torch.int32)
+        n = share // (8 if wide else 4)
+        if k in large and t.numel() > n:
+            # n seeded draws, duplicates removed: distinct positions in increasing order (a permutation of all the
+            # positions would take GBs of host memory for the largest outputs)
+            g = torch.Generator().manual_seed(zlib.crc32(k.encode()))
+            idx = torch.unique(torch.randint(0, t.numel(), (n,), generator=g))
+            t, k = t.reshape(-1)[idx.to(t.device)], k + "_sampled"
+        res[k] = t.to(torch.float64 if wide else torch.float32).cpu()
+    return res
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for k, t in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), t.numpy())
 
 
 def load_peaks():
@@ -1016,7 +1078,7 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline measurement (>= 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -1027,7 +1089,10 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the short measurement of the other BASELINE.json configurations")
     ap.add_argument("--workload-only", action="store_true", help="alias of --no-configs")
     ap.add_argument("--no-dp-check", action="store_true", help="N > 1: skip the sharded-vs-global-batch check before timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -231,8 +231,10 @@ def _dist_worker(rank, world, port, q):
         dist.destroy_process_group()
 
 
-def test_batch_sharded_summary_exchange_gloo_world2():
+def test_batch_sharded_summary_exchange_gloo_world2(monkeypatch):
     import torch.multiprocessing as mp
+    # host logic: the workers see no GPU, also on a machine that has one (they check that PeerExchange refuses to run)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()

@@ -1,10 +1,12 @@
-"""Checks that need the reference tree (/root/reference): run in the build container, skipped on
-the GPU box.  They pin the donor backbones and the module drop-in mechanics against the unmodified
-reference."""
+"""The donor backbones, the flat -> hierarchy stitching and ProcessClasses against what the unmodified reference computes
+for the same seeded inputs, stored in tests/golden/reference_pins.npz (tests/golden/make_reference_golden.py).  Where
+the reference tree is present (oracle/ref_loader.py) they are also compared with the reference itself; the module
+drop-in check imports the reference's train.py and runs only there."""
 import json
 import os
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -12,10 +14,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import ref_loader  # noqa: E402
 
-# /root/reference in the build container, the staged byte copies (oracle/_ref, tools/stage_reference.py) elsewhere
-REF = ref_loader.reference_root() or "/root/reference"
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
+REF = ref_loader.reference_root()
+needs_reference = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_reference_golden as G  # noqa: E402
+from helpers import close  # noqa: E402
+
+PINS = np.load(G.PINS, allow_pickle=False)
 
 
 def _ref():
@@ -23,47 +28,45 @@ def _ref():
     return ref_shim, ref_shim.load_reference()
 
 
+def _check_backbone(rec, prefix):
+    """A record of make_reference_golden against the stored one: identical key lists, outputs within 1e-5."""
+    for k in [k for k in PINS.files if k.startswith(prefix + ".") and k.endswith("keys")]:
+        assert json.loads(rec[k]) == json.loads(str(PINS[k])), k
+    for out in sorted({k.rsplit(".", 1)[0] for k in PINS.files if k.startswith(prefix + ".") and k.endswith(".sample")}):
+        assert list(rec[out + ".shape"]) == list(PINS[out + ".shape"]), out
+        assert np.array_equal(rec[out + ".index"], PINS[out + ".index"]), out
+        close(torch.from_numpy(rec[out + ".sample"]), torch.from_numpy(PINS[out + ".sample"]), what=out + " sample")
+        close(torch.from_numpy(rec[out + ".channel_sums"]), torch.from_numpy(PINS[out + ".channel_sums"]), what=out + " channel sums")
+
+
 def test_unet_donor_matches_reference_backbone():
-    ref_shim, (rmodels, _, _) = _ref()
     from rhseg_b200.Models import models
-    tree = json.load(open(os.path.join(REF, "class_tree_tl_extended.json")))
-    torch.manual_seed(0)
-    theirs = rmodels.UNet(size=64, n_channels=3, hierarchy=tree, model_type=1).eval()
-    ours = models.UNet(size=64, n_channels=3, hierarchy=tree, model_type=1).eval()
-    assert set(ours.state_dict()) == set(theirs.state_dict())
-    assert all(ours.state_dict()[k].shape == v.shape for k, v in theirs.state_dict().items())
-    ours.load_state_dict(theirs.state_dict())
-    x = torch.randn(2, 3, 40, 56)
-    with torch.no_grad():
-        assert torch.equal(ours._run_unet(x), theirs._run_unet(x))
-    assert ours.levels == theirs.levels and ours.parent_of == theirs.parent_of
-    assert ours.child_groups == theirs.child_groups and ours.children_of == theirs.children_of
+    tree = G.trees()["ext"]
+    ours = G.unet_record(models, tree)
+    _check_backbone(ours, "unet")
+    assert json.loads(ours["unet.tables"]) == json.loads(str(PINS["unet.tables"]))
+    if ref_loader.available():  # the reference itself, same parameters and input: bit for bit
+        _, (rmodels, _, _) = _ref()
+        theirs = G.unet_record(rmodels, tree)
+        assert ours["unet.keys"] == theirs["unet.keys"] and ours["unet.tables"] == theirs["unet.tables"]
+        assert np.array_equal(ours["unet.out.sample"], theirs["unet.out.sample"])
+        assert np.array_equal(ours["unet.out.channel_sums"], theirs["unet.out.channel_sums"])
 
 
 def test_hrnet_donor_matches_reference_backbone():
-    ref_shim, (rmodels, _, _) = _ref()
     from rhseg_b200.Models import models
-    cfg = ref_shim.hrnet_config()
-    tree = json.load(open(os.path.join(REF, "class_tree_tl.json")))
-    torch.manual_seed(0)
-    theirs = rmodels.HighResolutionNet(cfg, hierarchy=tree, model_type=1).eval()
-    ours = models.HighResolutionNet(cfg, hierarchy=tree, model_type=1).eval()
-    sd = theirs.state_dict()
-    assert set(ours.state_dict()) == set(sd)
-    assert all(ours.state_dict()[k].shape == v.shape for k, v in sd.items())
-    ours.load_state_dict(sd)
-    x = torch.randn(1, 3, 64, 96)
-    with torch.no_grad():
-        a, b = ours._forward_backbone(x), theirs._forward_backbone(x)
-    assert a.shape == b.shape == (1, 720, 16, 24)
-    assert torch.allclose(a, b, rtol=1e-5, atol=1e-6), float((a - b).abs().max())
-    flat_o = models.HighResolutionNet(cfg, hierarchy=tree, model_type=0).eval()
-    flat_t = rmodels.HighResolutionNet(cfg, hierarchy=tree, model_type=0).eval()
-    flat_o.load_state_dict(flat_t.state_dict())
-    with torch.no_grad():
-        assert torch.allclose(flat_o(x)[1], flat_t(x)[1], rtol=1e-5, atol=1e-6)
+    tree = G.trees()["tl"]
+    ours = G.hrnet_record(models, tree, G.hrnet_config())
+    assert list(ours["hrnet.out.shape"]) == [1, 720, 16, 24]
+    _check_backbone(ours, "hrnet")
+    if ref_loader.available():  # the reference's own config and modules
+        ref_shim, (rmodels, _, _) = _ref()
+        theirs = G.hrnet_record(rmodels, tree, ref_shim.hrnet_config())
+        _check_backbone(theirs, "hrnet")
+        assert ours["hrnet.keys"] == theirs["hrnet.keys"] and ours["hrnet.flat_keys"] == theirs["hrnet.flat_keys"]
 
 
+@needs_reference
 def test_module_dropin_shadows_reference_modules():
     """INTEGRATION.md section 1: with the package directory ahead of the reference root, the reference's
     train.py imports OUR Models / Metrics / tree_util."""
@@ -94,49 +97,25 @@ print("ok")
 
 def test_oracle_stitching_matches_reference_predicteval():
     """oracle.stitch_flat_to_levels == predictEval.get_parent_masks + combine_levels on both shipped trees."""
-    import importlib
-    ref_shim, _ = _ref()
-    for n in ("matplotlib.colors", "skimage.measure", "skimage.color", "scipy", "sklearn"):
-        ref_shim._stub(n)
-    pe = importlib.import_module("predictEval")
     from oracle import hier_oracle as O
-    for fname in ("class_tree_tl.json", "class_tree_tl_extended.json"):
-        tree = json.load(open(os.path.join(REF, fname)))
-        names = [n for n in pe.bfs_order(tree) if not pe.children_map(tree).get(n)]
-        idx = {n: i for i, n in enumerate(names)}
-        g = torch.Generator().manual_seed(3)
-        lab = torch.randint(0, len(names), (2, 9, 11), generator=g)
-        flat = torch.nn.functional.one_hot(lab, len(names)).permute(0, 3, 1, 2).float()
-        tgt = torch.nn.functional.one_hot(torch.randint(0, len(names), (2, 9, 11), generator=g), len(names)).permute(0, 3, 1, 2).float()
-        par, par_t, _ = pe.get_parent_masks([flat], [tgt], tree, idx)
-        parent_order = [n for n in pe.bfs_order(tree) if pe.children_map(tree).get(n)]
-        want = pe.combine_levels([flat], par, tree, names, parent_order)
-        got = O.stitch_flat_to_levels(flat, tree)
-        assert len(want) == len(got) and all(torch.equal(a, b) for a, b in zip(want, got))
+    ours = G.stitch_record(lambda flat, tgt, tree: O.stitch_flat_to_levels(flat, tree))
+    want = {k: PINS[k] for k in PINS.files if k.startswith("stitch.")}
+    assert sorted(ours) == sorted(want) and all(np.array_equal(ours[k], want[k]) for k in want)
+    if ref_loader.available():
+        _ref()
+        theirs = G.stitch_record(G.reference_stitch())
+        assert sorted(theirs) == sorted(want) and all(np.array_equal(theirs[k], want[k]) for k in want)
 
 
 def test_oracle_process_classes_pinned_to_reference():
-    """ProcessClasses (Metrics/performance_metrics.py:27-47) is torch-only: the reference's own class, imported with the
-    torchmetrics import stubbed, pins the oracle's restatement (and through it the CUDA confusion kernels) on the three
-    kinds of input that reach it (SURVEY.md 3.4): masked one-hots, composed probabilities, ties / all-zero pixels."""
-    ref_shim, _ = _ref()
-    rpm = ref_loader.load_reference_module("Metrics.performance_metrics")
+    """ProcessClasses (Metrics/performance_metrics.py:27-47) is torch-only: the reference's own class pins the oracle's
+    restatement (and through it the CUDA confusion kernels) on the three kinds of input that reach it (SURVEY.md 3.4):
+    masked one-hots, composed probabilities, ties / all-zero pixels."""
     from oracle import hier_oracle as O
-    theirs = rpm.ProcessClasses()
-    g = torch.Generator().manual_seed(9)
-    for K in (1, 2, 3, 4, 7):
-        B, H, W = 2, 13, 17
-        lab = torch.randint(0, K, (B, H, W), generator=g)
-        onehot = torch.nn.functional.one_hot(lab, K).permute(0, 3, 1, 2).float()
-        ignore = torch.rand(B, 1, H, W, generator=g) < 0.3
-        masked = torch.where(ignore, torch.zeros_like(onehot), onehot)            # train.py:230
-        probs = torch.rand(B, K, H, W, generator=g)
-        probs[:, :, :2] = 0.0                                                     # nothing positive
-        probs[:, :, 2:4] = probs[:, :1, 2:4]                                      # exact ties
-        tgt = torch.nn.functional.one_hot(torch.randint(0, K, (B, H, W), generator=g), K).permute(0, 3, 1, 2).float()
-        tgt = torch.where(torch.rand(B, 1, H, W, generator=g) < 0.4, torch.zeros_like(tgt), tgt)
-        for p in (masked, probs):
-            for child in (False, True):
-                a, b = theirs(p, tgt, child)
-                c, d = O.process_classes(p, tgt, child)
-                assert torch.equal(a, c.to(a.dtype)) and torch.equal(b, d.to(b.dtype)), (K, child)
+    ours = G.process_classes_record(O.process_classes)
+    want = {k: PINS[k] for k in PINS.files if k.startswith("process_classes.")}
+    assert sorted(ours) == sorted(want) and all(np.array_equal(ours[k], want[k]) for k in want)
+    if ref_loader.available():
+        _ref()
+        theirs = G.process_classes_record(ref_loader.load_reference_module("Metrics.performance_metrics").ProcessClasses())
+        assert all(np.array_equal(theirs[k], want[k]) for k in want)
