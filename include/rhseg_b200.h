@@ -33,6 +33,13 @@ extern "C" {
 #define RHSEG_KERNEL_MAX_K 8     /* channels per level the fused kernels are built for    */
 #define RHSEG_TABLE_INTS (4 + 5 * RHSEG_MAX_K)
 #define RHSEG_EVAL_PREZEROED 1   /* rhseg_level_eval / rhseg_head_level_fwd_eval flag       */
+/* Feature element type flag of rhseg_head_level_fwd (zero_psum), rhseg_head_level_fwd_eval (flags),
+ * rhseg_head_conv_bwd (zero_sums) and rhseg_head_conv_bwd_params (flags): set, feats (and dfeats) are
+ * bf16 [B,C,Hf,Wf], 2-byte aligned (autocast-trained donors); clear, fp32.  Each bf16 value is converted
+ * to fp32 exactly; every other tensor and every sum keeps its type, and dfeats is formed in fp32 and
+ * rounded to bf16 (nearest even) once, when stored.  So the results equal the fp32 path's on the
+ * upcast features.                                                                             */
+#define RHSEG_FEATS_BF16 0x10
 #define RHSEG_NSTAT 5            /* per (sample, class) loss statistics, see loss_stats   */
 #define RHSEG_MAX_LEVELS 8       /* tree depth rhseg_step_finalize handles in one launch  */
 #define RHSEG_STITCH_MAX_LEAVES 16 /* leaf channels of a flat model rhseg_stitch_levels reads */
@@ -105,7 +112,7 @@ int rhseg_film_fold(const float* head_w, const float* head_b, const float* film_
  * Outputs: logits [B,K,H,W], probs [B,K,H,W], psum [B,K] fp64 = sum over pixels of probs
  * (accumulated with atomics: zeroed here when zero_psum != 0, otherwise the caller passes a
  * zeroed buffer; it is the FiLM pool of the next level).                                  */
-int rhseg_head_level_fwd(const float* feats, const float* eff_w, const float* eff_b,
+int rhseg_head_level_fwd(const void* feats, const float* eff_w, const float* eff_b,
                          const float* prev_probs, const int32_t* table,
                          int B, int C, int Hf, int Wf, int H, int W, int K, int K_prev, int act_mode,
                          float* z_lo, float* logits, float* probs, double* psum, int zero_psum,
@@ -113,14 +120,15 @@ int rhseg_head_level_fwd(const float* feats, const float* eff_w, const float* ef
 /* zero_psum bit 1 (value 2): z_lo was zeroed by the caller (one fill for all levels); without it the
  * low-res pass zeroes z_lo itself whenever pixel tiles are split between CTAs.
  * zero_psum bit 2 (value 4): eff_w / eff_b are ONE [K,C] / [K] pair shared by all samples (a level without
- * FiLM, i.e. level 0: pass the head's own weight and bias, no rhseg_film_fold launch).       */
+ * FiLM, i.e. level 0: pass the head's own weight and bias, no rhseg_film_fold launch).
+ * zero_psum & RHSEG_FEATS_BF16: feats holds bf16 values (see RHSEG_FEATS_BF16).             */
 
 /* Level forward of an UPSAMPLED head (HRNet) fused with rhseg_level_eval: the hi-res pass that
  * interpolates and activates the logits also evaluates them against the ternary targets while
  * they are in registers.  Arguments = rhseg_head_level_fwd (psum must be zeroed by the caller) +
  * rhseg_level_eval (child is derived from act_mode).  Returns RHSEG_ERR_UNSUPPORTED for heads at
  * feature resolution: call the two functions separately there.                              */
-int rhseg_head_level_fwd_eval(const float* feats, const float* eff_w, const float* eff_b,
+int rhseg_head_level_fwd_eval(const void* feats, const float* eff_w, const float* eff_b,
                               const float* prev_probs, const int32_t* table,
                               int B, int C, int Hf, int Wf, int H, int W, int K, int K_prev, int act_mode,
                               float* z_lo, float* logits, float* probs, double* psum,
@@ -173,10 +181,11 @@ int rhseg_head_dz_lowres_fused(const float* logits, const float* targets, long t
  * S[b,k,c] = sum_n dz[b,k,n] feats[b,c,n]; s[b,k] = sum_n dz[b,k,n]  (fp64, accumulated with
  * atomics: zeroed here when zero_sums != 0, otherwise the caller passes zeroed buffers).
  * dfeats may be NULL (features do not require grad).
- * zero_sums bit 0: zero S / s here; bit 1 (value 2): eff_w is one [K,C] matrix shared by all samples.  */
-int rhseg_head_conv_bwd(const float* feats, const float* dz, const float* eff_w,
+ * zero_sums bit 0: zero S / s here; bit 1 (value 2): eff_w is one [K,C] matrix shared by all samples;
+ * RHSEG_FEATS_BF16: feats and dfeats are bf16.                                                       */
+int rhseg_head_conv_bwd(const void* feats, const float* dz, const float* eff_w,
                         int B, int C, int K, int n_pix,
-                        float* dfeats, double* S, double* s, int zero_sums, void* stream);
+                        void* dfeats, double* S, double* s, int zero_sums, void* stream);
 
 /* rhseg_head_conv_bwd followed by rhseg_head_param_grads in ONE launch: the last CTA to finish forms the parameter
  * gradients from the complete sums (no second kernel on the level chain).  Arguments: those of the two functions;
@@ -188,8 +197,8 @@ int rhseg_head_conv_bwd(const float* feats, const float* dz, const float* eff_w,
  * the conv kernel registers and, for 16-byte-aligned planes, its second CTA per SM).  Exception: a level WITHOUT FiLM
  * (film_w == NULL: d_head_w = sum_b S_b, d_head_b = sum_b s_b) of a narrow donor (B*C*K <= 4096) is always ONE launch,
  * the sums being formed by the conv kernel's last CTA.                                                            */
-int rhseg_head_conv_bwd_params(const float* feats, const float* dz, const float* eff_w, int B, int C, int K,
-                               int n_pix, float* dfeats, double* S, double* s, int flags, const float* head_w,
+int rhseg_head_conv_bwd_params(const void* feats, const float* dz, const float* eff_w, int B, int C, int K,
+                               int n_pix, void* dfeats, double* S, double* s, int flags, const float* head_w,
                                const float* film_w, const float* gamma_beta, const double* prev_psum,
                                double n_pix_out, int K_prev, float* d_head_w, float* d_head_b, float* d_film_w,
                                float* d_film_b, double* g_prev, unsigned* ticket, void* stream);

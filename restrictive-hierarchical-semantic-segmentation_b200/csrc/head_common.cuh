@@ -28,6 +28,13 @@ int fwd_upsampled_dispatch(int K, int act_arg, const float* z_lo, const float* p
                            int Hf, int Wf, int H, int W, int K_prev, float* logits, float* probs, double* psum,
                            cudaStream_t st, const EvalArgs* ea, bool* need_eval);
 
+// feature conv of the level forward for bf16 features (head_fwd_bf16.cu).  z_lo == nullptr: a head at feature
+// resolution, conv + activation into logits / probs / psum; otherwise the low-res conv of an upsampled head into
+// z_lo [B,K,Nf] (zeroed by the caller when zlo_zeroed).  feats = bf16 bit patterns, 2-byte aligned.
+int level_conv_bf16(const uint16_t* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
+                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
+                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
+
 // ------------------------------------------------------------------------------------
 // Activation epilogue shared by the fused and the upsampled path.  P pixels per thread.
 // ------------------------------------------------------------------------------------

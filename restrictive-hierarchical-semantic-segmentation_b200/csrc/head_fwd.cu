@@ -4,9 +4,7 @@
 // :269/:288-302 (sigmoid, restrictive softmax, composition, concat), :766/:776 (upsample).
 #include <algorithm>
 #include <cstdlib>
-#include "common.cuh"
-#include "pipeline.cuh"
-#include "head_common.cuh"
+#include "head_fwd_kernel.cuh"
 
 namespace rhseg {
 
@@ -63,319 +61,10 @@ __global__ void film_fold_kernel(const float* __restrict__ head_w, const float* 
   }
 }
 
-// ------------------------------------------------------------------------------------
-// Fused 1x1 conv (+ activation): TMA-fed, warp-specialised, persistent.
-//
-//   producer warp : streams [PIPE_CH channels x T pixels] stages of the feature planes into a
-//                   shared-memory ring with 1-D bulk async copies (pipeline.cuh)
-//   4 consumer warps: each thread owns J vectors of VEC pixels of the tile, accumulates
-//                   K logits over the stages (weights [C][KP] in shared memory, one broadcast
-//                   vector load per channel), then runs the activation epilogue
-//
-// Work unit = (sample, pixel tile, channel stage); the unit space is split EVENLY over one
-// resident wave of CTAs.  MODE 0-2 (fused activation) splits on tile boundaries; MODE 3 (conv
-// only, HRNet low-res pass, few pixels x many channels) splits anywhere: a tile shared by two
-// CTAs is finished with fp32 atomics into the zero-initialised output (at most two partial
-// sums per pixel, so the result does not depend on arrival order).
-// ------------------------------------------------------------------------------------
-constexpr int MODE_CONV_ONLY = 3;
-
-template <int K, int VEC, int J, int MODE, typename CFG>
-__global__ void __launch_bounds__(CFG::THREADS)
-head_fwd_kernel(const float* __restrict__ feats, const float* __restrict__ eff_w,
-                const float* __restrict__ eff_b, const float* __restrict__ prev_probs,
-                const int32_t* __restrict__ table, int C, int N, int K_prev, int n_tiles, int n_stages,
-                long units_total, int a0, int w_shared, float* __restrict__ logits, float* __restrict__ probs,
-                double* __restrict__ psum) {
-  pdl_wait();
-  constexpr int KP = pad_k(K);
-  constexpr int P = J * VEC;
-  constexpr int NCONS = CFG::CONSUMERS;
-  constexpr int T = NCONS * P;
-  constexpr int ROWP = T + 4;
-  constexpr int CH = CFG::CH;
-  constexpr int NS = CFG::NS;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw);            // full[NS], empty[NS]  (2*NS*8 bytes, padded to 128)
-  float* ring = reinterpret_cast<float*>(smem_raw + 128);            // [NS][CH][ROWP]
-  float* w_t = ring + (size_t)NS * CH * ROWP;                        // [C][KP]
-  float* red = w_t + (size_t)C * KP;                                 // [NCW][K]
-  static_assert(2 * NS * 8 <= 128, "barrier block");
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-
-  long u_begin, u_end;
-  if constexpr (MODE == MODE_CONV_ONLY) {
-    u_begin = units_total * blockIdx.x / gridDim.x;
-    u_end = units_total * (blockIdx.x + 1) / gridDim.x;
-  } else {
-    const long tiles_total = units_total / n_stages;
-    u_begin = (tiles_total * blockIdx.x / gridDim.x) * n_stages;
-    u_end = (tiles_total * (blockIdx.x + 1) / gridDim.x) * n_stages;
-  }
-  if (tid == 0) {
-    for (int i = 0; i < NS; ++i) {
-      mbar_init(smem_u32(&bars[i]), CFG::NPW);
-      mbar_init(smem_u32(&bars[NS + i]), CFG::NCW);
-    }
-    mbar_fence_init();
-  }
-  __syncthreads();
-
-  // unit u = (b * n_tiles + tile) * n_stages + stage; decoded once, then advanced incrementally
-  int stage, tile, b;
-  {
-    const long tile_lin = u_begin / n_stages;
-    stage = (int)(u_begin - tile_lin * n_stages);
-    b = (int)(tile_lin / n_tiles);
-    tile = (int)(tile_lin - (long)b * n_tiles);
-  }
-  auto advance = [&]() {
-    if (++stage == n_stages) {
-      stage = 0;
-      if (++tile == n_tiles) { tile = 0; ++b; }
-    }
-  };
-
-  if (warp >= CFG::NCW) {
-    // ------------------------------ producers ------------------------------
-    if (lane == 0) {
-      const int pw = warp - CFG::NCW;
-      const uint64_t pol = l2_evict_first_policy();
-      int slot = 0;
-      uint32_t phase = 1;  // parity of the "slot is free" wait; flips every NS units
-      for (long u = u_begin; u < u_end; ++u) {
-        mbar_wait(smem_u32(&bars[NS + slot]), phase);
-        const int p0 = tile * T;
-        const int c0 = stage * CH;
-        issue_stage_rows(feats, ((long)b * C + c0) * N + p0, N, min(T, N - p0), min(CH, C - c0), pw, CFG::NPW, a0,
-                         smem_u32(ring + (size_t)slot * CH * ROWP), ROWP * 4, smem_u32(&bars[slot]), pol);
-        if (++slot == NS) { slot = 0; phase ^= 1u; }
-        advance();
-      }
-    }
-    return;
-  }
-
-  // -------------------------------- consumers --------------------------------
-  auto csync = [] { consumer_sync(NCONS); };
-  LevelInfo li;
-  if constexpr (MODE != MODE_CONV_ONLY) li = load_level_info<K>(MODE == RHSEG_ACT_GROUPED ? table : nullptr);
-  int cur_b = -1;
-  float bias[K], ps[K], acc[K][P];
-#pragma unroll
-  for (int k = 0; k < K; ++k) {
-    bias[k] = 0.f;
-    ps[k] = 0.f;
-#pragma unroll
-    for (int p = 0; p < P; ++p) acc[k][p] = 0.f;
-  }
-  const int sN = N & 3;
-  bool from_stage0 = false;
-  int slot = 0;
-  uint32_t phase = 0;
-  for (long u = u_begin; u < u_end; ++u) {
-    const int p0 = tile * T;
-    const int t_act = min(T, N - p0);
-    if (stage == 0 || u == u_begin) {  // first unit of this tile in this CTA (uniform)
-      if (b != cur_b) {
-        if constexpr (MODE != MODE_CONV_ONLY) {
-          if (cur_b >= 0) {
-            block_psum<K, CFG::NCW>(ps, psum + (size_t)cur_b * K, red, csync);
-#pragma unroll
-            for (int k = 0; k < K; ++k) ps[k] = 0.f;
-          }
-        }
-        csync();
-        const float* wsrc = w_shared ? eff_w : eff_w + (size_t)b * K * C;  // level 0: the head's own [K,C] weights
-        for (int k = 0; k < K; ++k)
-          for (int c = tid; c < C; c += NCONS) w_t[c * KP + k] = wsrc[(size_t)k * C + c];
-        if constexpr (KP > K)
-          for (int k = K; k < KP; ++k)
-            for (int c = tid; c < C; c += NCONS) w_t[c * KP + k] = 0.f;
-#pragma unroll
-        for (int k = 0; k < K; ++k) bias[k] = eff_b[(w_shared ? 0 : b * K) + k];
-        cur_b = b;
-        csync();
-      }
-      from_stage0 = stage == 0;
-#pragma unroll
-      for (int k = 0; k < K; ++k)
-#pragma unroll
-        for (int p = 0; p < P; ++p) acc[k][p] = from_stage0 ? bias[k] : 0.f;
-    }
-
-    const int c0 = stage * CH;
-    const int ccnt = min(CH, C - c0);
-    // shift of stage row cc is (sh0 + cc*sN) & 3: only four distinct values, indexed by cc & 3
-    int off[4] = {0, 0, 0, 0};
-    int sh0 = 0;
-    if constexpr (VEC == 1) {
-      sh0 = row_shift(((long)b * C + c0) * N + p0, a0);
-#pragma unroll
-      for (int q = 0; q < 4; ++q) off[q] = ((sh0 + q * sN) & 3) + tid;
-    }
-    const float* wrow = w_t + (size_t)c0 * KP;
-    mbar_wait(smem_u32(&bars[slot]), phase);
-    const float* stage_base = ring + (size_t)slot * CH * ROWP;
-
-    auto channel = [&](int cc, int offv) {
-      const float* row = stage_base + cc * ROWP;
-      float w[KP];
-      if constexpr (KP == 4) {
-        const float4 t = *reinterpret_cast<const float4*>(wrow + cc * KP);
-        w[0] = t.x; w[1] = t.y; w[2] = t.z; w[3] = t.w;
-      } else if constexpr (KP == 8) {
-        const float4 t0 = *reinterpret_cast<const float4*>(wrow + cc * KP);
-        const float4 t1 = *reinterpret_cast<const float4*>(wrow + cc * KP + 4);
-        w[0] = t0.x; w[1] = t0.y; w[2] = t0.z; w[3] = t0.w; w[4] = t1.x; w[5] = t1.y; w[6] = t1.z; w[7] = t1.w;
-      } else if constexpr (KP == 2) {
-        const float2 t = *reinterpret_cast<const float2*>(wrow + cc * KP);
-        w[0] = t.x; w[1] = t.y;
-      } else {
-        w[0] = wrow[cc];
-      }
-#pragma unroll
-      for (int j = 0; j < J; ++j) {
-        float f[VEC];
-        if constexpr (VEC == 4) {
-          const float4 t = *reinterpret_cast<const float4*>(row + (j * NCONS + tid) * 4);
-          f[0] = t.x; f[1] = t.y; f[2] = t.z; f[3] = t.w;
-        } else {
-          f[0] = row[offv + j * NCONS];
-        }
-#pragma unroll
-        for (int k = 0; k < K; ++k)
-#pragma unroll
-          for (int v = 0; v < VEC; ++v) acc[k][j * VEC + v] = fmaf(w[k], f[v], acc[k][j * VEC + v]);
-      }
-    };
-    if (ccnt == CH) {  // full stage: branch-free, loads can be batched ahead of the FMAs
-#pragma unroll
-      for (int cc = 0; cc < CH; ++cc) channel(cc, off[cc & 3]);
-    } else {
-      for (int cc = 0; cc < ccnt; ++cc) channel(cc, ((sh0 + cc * sN) & 3) + tid);
-    }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(smem_u32(&bars[NS + slot]));
-
-    if (stage == n_stages - 1 || u == u_end - 1) {  // last unit of this tile in this CTA: epilogue
-      int lp[J];
-      bool ok[J];
-#pragma unroll
-      for (int j = 0; j < J; ++j) {
-        lp[j] = (j * NCONS + tid) * VEC;
-        ok[j] = lp[j] < t_act;
-      }
-      float* zb = logits + (size_t)b * K * N + p0;
-      if constexpr (MODE == MODE_CONV_ONLY) {
-        const bool complete = from_stage0 && stage == n_stages - 1;
-#pragma unroll
-        for (int j = 0; j < J; ++j) {
-          if (!ok[j]) continue;
-#pragma unroll
-          for (int k = 0; k < K; ++k) {
-            float* dst = zb + (size_t)k * N + lp[j];
-            if (complete) {
-              Vec<VEC> o;
-#pragma unroll
-              for (int v = 0; v < VEC; ++v) o.v[v] = acc[k][j * VEC + v];
-              *reinterpret_cast<Vec<VEC>*>(dst) = o;
-            } else {
-#pragma unroll
-              for (int v = 0; v < VEC; ++v) atomicAdd(dst + v, acc[k][j * VEC + v]);
-            }
-          }
-        }
-      } else {
-        float pp[K][P];
-        if constexpr (MODE == RHSEG_ACT_GROUPED) {
-          const float* pb = prev_probs + (size_t)b * K_prev * N + p0;
-#pragma unroll
-          for (int k = 0; k < K; ++k) {
-            if ((li.start_mask >> k) & 1) {
-#pragma unroll
-              for (int j = 0; j < J; ++j) {
-                Vec<VEC> t;
-                if (ok[j]) t = ld_cached<VEC>(pb + (size_t)li.parent[k] * N + lp[j]);
-                else {
-#pragma unroll
-                  for (int v = 0; v < VEC; ++v) t.v[v] = 0.f;
-                }
-#pragma unroll
-                for (int v = 0; v < VEC; ++v) pp[k][j * VEC + v] = t.v[v];
-              }
-            } else {
-#pragma unroll
-              for (int p = 0; p < P; ++p) pp[k][p] = pp[k > 0 ? k - 1 : 0][p];
-            }
-          }
-        }
-        float prob[K][P];
-        activate<K, P, MODE>(acc, pp, li.start_mask, prob);
-        float* pb_out = probs + (size_t)b * K * N + p0;
-#pragma unroll
-        for (int k = 0; k < K; ++k) {
-#pragma unroll
-          for (int j = 0; j < J; ++j) {
-            if (!ok[j]) continue;
-            Vec<VEC> zo, po;
-#pragma unroll
-            for (int v = 0; v < VEC; ++v) {
-              zo.v[v] = acc[k][j * VEC + v];
-              po.v[v] = prob[k][j * VEC + v];
-              ps[k] += po.v[v];
-            }
-            *reinterpret_cast<Vec<VEC>*>(zb + (size_t)k * N + lp[j]) = zo;
-            *reinterpret_cast<Vec<VEC>*>(pb_out + (size_t)k * N + lp[j]) = po;
-          }
-        }
-      }
-    }
-    if (++slot == NS) { slot = 0; phase ^= 1u; }
-    advance();
-  }
-  if constexpr (MODE != MODE_CONV_ONLY) {
-    if (cur_b >= 0) block_psum<K, CFG::NCW>(ps, psum + (size_t)cur_b * K, red, csync);
-  }
-}
-
-template <int K, int VEC, int J, int MODE, typename CFG>
-static int launch_fwd(const float* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                      const int32_t* table, int B, int C, int N, int K_prev, float* logits, float* probs,
-                      double* psum, cudaStream_t st, bool out_prezeroed = false, int w_shared = 0) {
-  constexpr int KP = pad_k(K);
-  constexpr int T = CFG::CONSUMERS * J * VEC;
-  const size_t smem = 128 + ((size_t)CFG::NS * CFG::CH * (T + 4) + (size_t)C * KP + CFG::NCW * K) * sizeof(float);
-  auto kern = head_fwd_kernel<K, VEC, J, MODE, CFG>;
-  int per_sm = 0;
-  RHSEG_CUDA(cached_launch_prep(reinterpret_cast<const void*>(kern), CFG::THREADS, smem, smem, &per_sm));
-  if (per_sm < 1) return RHSEG_ERR_UNSUPPORTED;
-  const int n_tiles = (N + T - 1) / T;
-  const int n_stages = (C + CFG::CH - 1) / CFG::CH;
-  const long tiles_total = (long)B * n_tiles;
-  const long units_total = tiles_total * n_stages;
-  long grid = (long)device_sm_count() * per_sm;
-  grid = std::min<long>(grid, tiles_total);  // every CTA owns >= n_stages units: a split tile has <= 2 owners
-  if (grid < 1) grid = 1;
-  if (MODE == MODE_CONV_ONLY && grid > 1 && !out_prezeroed)
-    RHSEG_CUDA(cudaMemsetAsync(logits, 0, sizeof(float) * (size_t)B * K * N, st));
-  const int a0 = (int)((reinterpret_cast<uintptr_t>(feats) >> 2) & 3);
-  launch_pdl(kern, dim3((unsigned)grid), dim3(CFG::THREADS), smem, st, feats, eff_w, eff_b, prev_probs, table, C, N, K_prev, n_tiles, n_stages,
-                                                  units_total, a0, w_shared, logits, probs, psum);
-  RHSEG_LAUNCH_CHECK();
-  return RHSEG_OK;
-}
-
-static bool rows_vec4(const float* p, int N) { return (N % 4 == 0) && ((reinterpret_cast<uintptr_t>(p) & 15u) == 0); }
 static int tune_env(const char* name) {
   const char* v = getenv(name);
   return v ? atoi(v) : 0;
 }
-
-// pipeline shapes (see DESIGN.md "conv kernels"): vec4 rows = full-resolution donors (UNet);
-// scalar rows = planes whose pitch is not a multiple of 16 bytes (HRNet 155x155)
-using FwdCfgV4 = PipeCfg<8, 8, 3>;      // 8 consumer warps x float4 -> T = 1024 px, 4 KB row copies
-using FwdCfgS1 = PipeCfg<4, 16, 4, 2>;  // scalar rows, T = 128*J px, two producer warps (1 KB row copies)
 
 template <int K, int MODE>
 static int fwd_fullres(const float* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
@@ -385,13 +74,13 @@ static int fwd_fullres(const float* feats, const float* eff_w, const float* eff_
   if (v4) {
     if constexpr (K == 4) {
       const int t = tune_env("RHSEG_TUNE_FWD_V4");
-      if (t == 1) return launch_fwd<K, 4, 1, MODE, PipeCfg<4, 8, 4>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-      if (t == 2) return launch_fwd<K, 4, 1, MODE, PipeCfg<8, 16, 2>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-      if (t == 3) return launch_fwd<K, 4, 1, MODE, PipeCfg<8, 16, 3>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
+      if (t == 1) return launch_fwd<float, K, 4, 1, MODE, PipeCfg<4, 8, 4>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
+      if (t == 2) return launch_fwd<float, K, 4, 1, MODE, PipeCfg<8, 16, 2>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
+      if (t == 3) return launch_fwd<float, K, 4, 1, MODE, PipeCfg<8, 16, 3>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
     }
-    return launch_fwd<K, 4, 1, MODE, FwdCfgV4>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
+    return launch_fwd<float, K, 4, 1, MODE, FwdCfgV4>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
   }
-  return launch_fwd<K, 1, 2, MODE, FwdCfgS1>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
+  return launch_fwd<float, K, 1, 2, MODE, FwdCfgS1>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
 }
 
 }  // namespace rhseg
@@ -415,13 +104,13 @@ extern "C" int rhseg_film_fold(const float* head_w, const float* head_b, const f
   return RHSEG_OK;
 }
 
-static int level_fwd_impl(const float* feats, const float* eff_w, const float* eff_b,
+static int level_fwd_impl(const void* feats_v, const float* eff_w, const float* eff_b,
                           const float* prev_probs, const int32_t* table, int B, int C, int Hf, int Wf,
                           int H, int W, int K, int K_prev, int act_arg, float* z_lo, float* logits,
                           float* probs, double* psum, int zero_psum, void* stream, const EvalArgs* ea, bool* need_eval) {
   const int act_mode = act_arg & 0xff;
   if (need_eval) *need_eval = false;
-  if (!feats || !eff_w || !eff_b || !logits || !probs || !psum) return RHSEG_ERR_ARG;
+  if (!feats_v || !eff_w || !eff_b || !logits || !probs || !psum) return RHSEG_ERR_ARG;
   if (B <= 0 || C <= 0 || Hf <= 0 || Wf <= 0 || H <= 0 || W <= 0) return RHSEG_ERR_ARG;
   if (K < 1 || K > RHSEG_KERNEL_MAX_K) return RHSEG_ERR_UNSUPPORTED;
   if (act_mode == RHSEG_ACT_GROUPED && (!prev_probs || !table || K_prev < 1)) return RHSEG_ERR_ARG;
@@ -434,41 +123,51 @@ static int level_fwd_impl(const float* feats, const float* eff_w, const float* e
   if (ea && !up) return RHSEG_ERR_UNSUPPORTED;
   if (act_mode == RHSEG_ACT_GROUPED && table == nullptr) return RHSEG_ERR_ARG;
   const int Nf = Hf * Wf;
-  if (!up) {
+  if (zero_psum & RHSEG_FEATS_BF16) {
+    const uint16_t* fb = static_cast<const uint16_t*>(feats_v);
+    if (reinterpret_cast<uintptr_t>(fb) & 1u) return RHSEG_ERR_ARG;
+    if (up && !z_lo) return RHSEG_ERR_ARG;
+    const int rc = level_conv_bf16(fb, eff_w, eff_b, prev_probs, table, B, C, Nf, K, K_prev, act_mode, up ? z_lo : nullptr,
+                                   zlo_zeroed, logits, probs, psum, w_shared, st);
+    if (rc != RHSEG_OK || !up) return rc;
+  } else {
+    const float* feats = static_cast<const float*>(feats_v);
+    if (!up) {
+      RHSEG_DISPATCH_K(K, {
+        if (act_mode == RHSEG_ACT_SIGMOID)
+          return fwd_fullres<KK, RHSEG_ACT_SIGMOID>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
+        if (act_mode == RHSEG_ACT_GROUPED)
+          return fwd_fullres<KK, RHSEG_ACT_GROUPED>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
+        return fwd_fullres<KK, RHSEG_ACT_ZEROS>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
+      });
+    }
+    if (!z_lo) return RHSEG_ERR_ARG;
     RHSEG_DISPATCH_K(K, {
-      if (act_mode == RHSEG_ACT_SIGMOID)
-        return fwd_fullres<KK, RHSEG_ACT_SIGMOID>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
-      if (act_mode == RHSEG_ACT_GROUPED)
-        return fwd_fullres<KK, RHSEG_ACT_GROUPED>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
-      return fwd_fullres<KK, RHSEG_ACT_ZEROS>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
+      int rc;
+      if (rows_vec4(feats, Nf) && rows_vec4(z_lo, Nf)) {
+        rc = launch_fwd<float, KK, 4, 1, MODE_CONV_ONLY, FwdCfgV4>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
+      } else {
+        int t = 0;
+        if constexpr (KK == 4) t = tune_env("RHSEG_TUNE_FWD_S1");
+        if constexpr (KK == 4) {
+          if (t == 1) rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, PipeCfg<8, 16, 3, 2>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
+          else if (t == 2) rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, PipeCfg<8, 8, 4, 2>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
+          else if (t == 3) rc = launch_fwd<float, KK, 1, 4, MODE_CONV_ONLY, PipeCfg<4, 16, 4, 1>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
+          else rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, FwdCfgS1>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
+        } else {
+          rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, FwdCfgS1>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
+        }
+      }
+      if (rc != RHSEG_OK) return rc;
     });
   }
-  if (!z_lo) return RHSEG_ERR_ARG;
-  RHSEG_DISPATCH_K(K, {
-    int rc;
-    if (rows_vec4(feats, Nf) && rows_vec4(z_lo, Nf)) {
-      rc = launch_fwd<KK, 4, 1, MODE_CONV_ONLY, FwdCfgV4>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
-    } else {
-      int t = 0;
-      if constexpr (KK == 4) t = tune_env("RHSEG_TUNE_FWD_S1");
-      if constexpr (KK == 4) {
-        if (t == 1) rc = launch_fwd<KK, 1, 2, MODE_CONV_ONLY, PipeCfg<8, 16, 3, 2>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
-        else if (t == 2) rc = launch_fwd<KK, 1, 2, MODE_CONV_ONLY, PipeCfg<8, 8, 4, 2>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
-        else if (t == 3) rc = launch_fwd<KK, 1, 4, MODE_CONV_ONLY, PipeCfg<4, 16, 4, 1>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
-        else rc = launch_fwd<KK, 1, 2, MODE_CONV_ONLY, FwdCfgS1>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
-      } else {
-        rc = launch_fwd<KK, 1, 2, MODE_CONV_ONLY, FwdCfgS1>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
-      }
-    }
-    if (rc != RHSEG_OK) return rc;
-  });
   bool ne = false;
   const int rc = fwd_upsampled_dispatch(K, act_arg, z_lo, prev_probs, table, B, Hf, Wf, H, W, K_prev, logits, probs, psum, st, ea, &ne);
   if (need_eval) *need_eval = ne;
   return rc;
 }
 
-extern "C" int rhseg_head_level_fwd(const float* feats, const float* eff_w, const float* eff_b,
+extern "C" int rhseg_head_level_fwd(const void* feats, const float* eff_w, const float* eff_b,
                                     const float* prev_probs, const int32_t* table, int B, int C, int Hf, int Wf,
                                     int H, int W, int K, int K_prev, int act_mode, float* z_lo, float* logits,
                                     float* probs, double* psum, int zero_psum, void* stream) {
@@ -476,7 +175,7 @@ extern "C" int rhseg_head_level_fwd(const float* feats, const float* eff_w, cons
                         psum, zero_psum, stream, nullptr, nullptr);
 }
 
-extern "C" int rhseg_head_level_fwd_eval(const float* feats, const float* eff_w, const float* eff_b,
+extern "C" int rhseg_head_level_fwd_eval(const void* feats, const float* eff_w, const float* eff_b,
                                          const float* prev_probs, const int32_t* table, int B, int C, int Hf, int Wf,
                                          int H, int W, int K, int K_prev, int act_mode, float* z_lo, float* logits,
                                          float* probs, double* psum, const float* targets, long t_bstride,
@@ -495,7 +194,7 @@ extern "C" int rhseg_head_level_fwd_eval(const float* feats, const float* eff_w,
               reinterpret_cast<unsigned long long*>(cons + RHSEG_MAX_K), idx_out};
   bool need_eval = false;
   const int rc = level_fwd_impl(feats, eff_w, eff_b, prev_probs, table, B, C, Hf, Wf, H, W, K, K_prev, act_mode, z_lo, logits,
-                                probs, psum, (flags & (2 | 4)), stream, &ea, &need_eval);
+                                probs, psum, (flags & (2 | 4 | RHSEG_FEATS_BF16)), stream, &ea, &need_eval);
   if (rc != RHSEG_OK || !need_eval) return rc;
   // shapes the band kernel does not take: the evaluation runs as its own kernel on the finished logits
   return rhseg_level_eval(logits, targets, t_bstride, t_cstride, parent_targets, pt_bstride, pt_cstride, prev_idx, table, B, K,

@@ -1,17 +1,35 @@
 // mbarrier + TMA bulk-copy (cp.async.bulk) primitives for the feature-streaming kernels.
 //
-// The donor feature maps are [B, C, N] fp32 planes.  A producer warp streams [CH channels x
-// T pixels] stages into a shared-memory ring with 1-D bulk async copies (one per channel row,
-// completion counted on an mbarrier); consumer warps read the stage from shared memory.  Rows
-// whose start is only 4-byte aligned (HRNet: N = 155*155 is odd) are fetched as the enclosing
-// 16-byte-aligned span and indexed with a per-row shift of 0..3 elements, so the same
-// pipeline serves every plane size.  The span never leaves the 16-byte granules that hold
-// valid bytes of the tensor.
+// The donor feature maps are [B, C, N] planes of fp32, or of bf16 held as raw 16-bit values
+// (autocast-trained donors; converted exactly to fp32 in registers by feat_f32).  A producer warp
+// streams [CH channels x T pixels] stages into a shared-memory ring with 1-D bulk async copies
+// (one per channel row, completion counted on an mbarrier); consumer warps read the stage from
+// shared memory.  Rows whose start is only element-aligned (HRNet: N = 155*155 is odd) are
+// fetched as the enclosing 16-byte-aligned span and indexed with a per-row shift of
+// 0..FeatElem<FT>::G-1 elements (0..3 fp32, 0..7 bf16), so the same pipeline serves every plane
+// size.  The span never leaves the 16-byte granules that hold valid bytes of the tensor.
 #pragma once
 #include <cuda_runtime.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 
 namespace rhseg {
+
+// Feature element types: float, or uint16_t = the bit pattern of a bf16 value.  G = elements per 16-byte granule.
+template <typename FT> struct FeatElem;
+template <> struct FeatElem<float> { static constexpr int G = 4, LOG2_G = 2, LOG2_SIZE = 2; };
+template <> struct FeatElem<uint16_t> { static constexpr int G = 8, LOG2_G = 3, LOG2_SIZE = 1; };
+
+__device__ __forceinline__ float feat_f32(float v) { return v; }
+__device__ __forceinline__ float feat_f32(uint16_t v) { return __uint_as_float((uint32_t)v << 16); }  // exact
+__device__ __forceinline__ float bf16_lo(uint32_t w) { return __uint_as_float(w << 16); }       // element 2i of a pair
+__device__ __forceinline__ float bf16_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }  // element 2i+1
+// fp32 pair -> two bf16 (round to nearest even, cvt.rn.bf16x2.f32); `lo` goes to the lower address
+__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const uint32_t*>(&h);
+}
+__device__ __forceinline__ uint16_t to_bf16_bits(float v) { return __bfloat16_as_ushort(__float2bfloat16_rn(v)); }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -66,7 +84,13 @@ __device__ __forceinline__ void consumer_sync(int nthreads) {
 
 // shift (elements) of the 16-byte-aligned span that contains element `e` of a tensor whose base
 // pointer sits `a0` elements past a 16-byte boundary
-__device__ __forceinline__ int row_shift(long e, int a0) { return (int)((e + a0) & 3); }
+template <typename FT = float>
+__device__ __forceinline__ int row_shift(long e, int a0) { return (int)((e + a0) & (FeatElem<FT>::G - 1)); }
+// a0 of a feature tensor (host side)
+template <typename FT>
+inline int base_shift(const void* p) {
+  return (int)((reinterpret_cast<uintptr_t>(p) >> FeatElem<FT>::LOG2_SIZE) & (FeatElem<FT>::G - 1));
+}
 
 // Pipeline shape: NCW consumer warps + NPW producer warps, CH channel rows per stage, NS stages.
 // One elected lane per producer warp issues the row copies of its share of a stage (measured:
@@ -83,14 +107,16 @@ struct PipeCfg {
 
 // Issues the row copies r = first, first+step, ... < ccnt of one stage (rows N elements apart,
 // starting at element e0 of `base`) and arrives on `bar` with the byte count.  Single thread.
-__device__ __forceinline__ void issue_stage_rows(const float* base, long e0, int N, int t_act, int ccnt, int first,
+template <typename FT>
+__device__ __forceinline__ void issue_stage_rows(const FT* base, long e0, int N, int t_act, int ccnt, int first,
                                                  int step, int a0, uint32_t dst_row0, uint32_t row_pitch_bytes,
                                                  uint32_t bar, uint64_t pol) {
+  constexpr int G = FeatElem<FT>::G, LOG2_G = FeatElem<FT>::LOG2_G;
   uint32_t total = 0;
   for (int r = first; r < ccnt; r += step) {
     const long e = e0 + (long)r * N;
-    const int sh = row_shift(e, a0);
-    const uint32_t bytes = (uint32_t)(((sh + t_act + 3) >> 2) << 4);
+    const int sh = row_shift<FT>(e, a0);
+    const uint32_t bytes = (uint32_t)(((sh + t_act + G - 1) >> LOG2_G) << 4);
     bulk_g2s(dst_row0 + (uint32_t)r * row_pitch_bytes, base + (e - sh), bytes, bar, pol);
     total += bytes;
   }

@@ -25,6 +25,16 @@ def _f32c(t: torch.Tensor) -> torch.Tensor:
     return t if t.is_contiguous() else t.contiguous()
 
 
+def _feats_c(feats: Sequence[torch.Tensor]) -> Tuple[List[torch.Tensor], int]:
+    """Contiguous per-level features and the kernels' element-type flag: float32, or bfloat16 on every level (donors
+    trained under torch.autocast; the kernels convert each value to fp32 exactly and store dfeats as bf16)."""
+    dt = feats[0].dtype
+    if dt not in (torch.float32, torch.bfloat16) or any(f.dtype != dt for f in feats):
+        raise native.NativeError("rhseg_b200 head expects float32 or bfloat16 features (one dtype for every level), got %s"
+                                 % ", ".join(sorted({str(f.dtype) for f in feats})))
+    return [f if f.is_contiguous() else f.contiguous() for f in feats], (native.FEATS_BF16 if dt == torch.bfloat16 else 0)
+
+
 _SIDE_STREAMS = {}
 # Upsampled heads, fused training step: which levels are evaluated INSIDE their hi-res forward kernel
 # (rhseg_head_level_fwd_eval) instead of by rhseg_level_eval on a side stream, concurrent with the next level's forward.
@@ -43,7 +53,8 @@ def _side_stream(dev):
 
 def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words: int = 0, with_backward: bool = False):
     """Runs the per-level forward kernels.  `tensors` = feats[n] + head_w[n] + head_b[n] + film_w[n-1] +
-    film_b[n-1].  Returns a dict with the inputs (contiguous fp32) and probs / logits / psums / eff_w /
+    film_b[n-1]; the features are fp32 or bf16 (_feats_c), everything else fp32.  Returns a dict with the inputs
+    (contiguous) and probs / logits / psums / eff_w /
     gamma_beta per level plus the shape tuple.
     `evaluate(L, dims)` (fused training step) returns the rhseg_level_eval arguments of level L:
     (targets_ptr, t_bs, t_cs, parent_ptr, prev_idx_ptr, out_words_ptr, idx_out_ptr); the evaluation then runs
@@ -52,7 +63,7 @@ def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words
     `evaluate` as its third argument (the fused step's statistics workspace).  with_backward: the same fill also
     zeroes the accumulators of the backward pass (r["bwd"], see backward_buffers): ONE fill per training step."""
     n = tree.num_levels
-    feats = [_f32c(t) for t in tensors[0:n]]
+    feats, fbf = _feats_c(tensors[0:n])
     head_w = [_f32c(t) for t in tensors[n:2 * n]]
     head_b = [_f32c(t) for t in tensors[2 * n:3 * n]]
     film_w = [_f32c(t) for t in tensors[3 * n:4 * n - 1]]
@@ -122,11 +133,11 @@ def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words
             call("rhseg_head_level_fwd_eval", ptr(f), ptr(eff_w), ptr(eff_b),
                  ptr(probs[L - 1]) if L > 0 else None, ptr(tables[L]),
                  B, C, Hf, Wf, H, W, K, K_prev, tree.act_mode[L] | hint, ptr(z_lo), ptr(z), ptr(p), ptr(psum),
-                 t_ptr, t_bs, t_cs, pt_ptr, t_bs, t_cs, pidx_ptr, words_ptr, idx_ptr, 1 | 2 | shared, st)
+                 t_ptr, t_bs, t_cs, pt_ptr, t_bs, t_cs, pidx_ptr, words_ptr, idx_ptr, 1 | 2 | shared | fbf, st)
         else:
             call("rhseg_head_level_fwd", ptr(f), ptr(eff_w), ptr(eff_b),
                  ptr(probs[L - 1]) if L > 0 else None, ptr(tables[L]),
-                 B, C, Hf, Wf, H, W, K, K_prev, tree.act_mode[L] | hint, ptr(z_lo), ptr(z), ptr(p), ptr(psum), (2 if upsampled else 0) | shared, st)
+                 B, C, Hf, Wf, H, W, K, K_prev, tree.act_mode[L] | hint, ptr(z_lo), ptr(z), ptr(p), ptr(psum), (2 if upsampled else 0) | shared | fbf, st)
             if ev is not None:
                 t_ptr, t_bs, t_cs, pt_ptr, pidx_ptr, words_ptr, idx_ptr = ev
                 if overlap:
@@ -166,8 +177,9 @@ def level_weight_backward(tree, L, dims, feats_L, dz_feat, eff_w_L, head_w_L, fi
         d_fw = torch.empty_like(film_w_prev)
         d_fb = torch.empty((2 * C,), dtype=torch.float32, device=dev)
         g_prev = buf["gp"]
+    fbf = native.FEATS_BF16 if feats_L.dtype == torch.bfloat16 else 0  # d_feats: same dtype as the features
     call("rhseg_head_conv_bwd_params", ptr(feats_L), ptr(dz_feat), ptr(eff_w_L), B, C, K, Hf * Wf, ptr(d_feats),
-         ptr(buf["S"]), ptr(buf["s"]), (2 if L == 0 else 0) | 4, ptr(head_w_L), ptr(film_w_prev) if L > 0 else None, ptr(gb_L),
+         ptr(buf["S"]), ptr(buf["s"]), (2 if L == 0 else 0) | 4 | fbf, ptr(head_w_L), ptr(film_w_prev) if L > 0 else None, ptr(gb_L),
          ptr(psum_prev) if L > 0 else None, float(H * W), K_prev, ptr(d_hw), ptr(d_hb), ptr(d_fw), ptr(d_fb), ptr(g_prev),
          ptr(buf["ticket"]), st)
     return d_feats, d_hw, d_hb, d_fw, d_fb, g_prev

@@ -18,6 +18,7 @@ TABLE_INTS = 4 + 5 * MAX_K
 NSTAT = 5
 XCHG_HANDLE_BYTES = 64
 DZ_PREZEROED = 1
+FEATS_BF16 = 0x10  # RHSEG_FEATS_BF16: the feature (and dfeats) tensors of the call are bf16
 ACT_SIGMOID, ACT_GROUPED, ACT_ZEROS = 0, 1, 2
 
 _c = ctypes
