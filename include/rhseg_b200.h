@@ -40,6 +40,15 @@ extern "C" {
  * rounded to bf16 (nearest even) once, when stored.  So the results equal the fp32 path's on the
  * upcast features.                                                                             */
 #define RHSEG_FEATS_BF16 0x10
+/* Feature layout flag of the same four calls: set, feats (and dfeats) are channels-last, [B,Hf,Wf,C] in
+ * memory (what a donor converted with torch.channels_last returns); clear, [B,C,Hf,Wf].  Combines with
+ * RHSEG_FEATS_BF16.  Requires C * element size to be a multiple of 16 bytes and a 16-byte aligned
+ * feats (and dfeats) base (every pixel then starts on a 16-byte granule), and in the conv backward at
+ * most 4096 bytes per pixel; a call that misses one returns RHSEG_ERR_UNSUPPORTED.  Every other tensor
+ * keeps its layout.  Full-resolution logits and probabilities are formed in the [B,C,Hf,Wf] kernels'
+ * order, and dfeats too for the same dz; see DESIGN.md 3.8 for when they are bit-identical.  The
+ * low-resolution logits of upsampled heads and the fp64 sums agree to rounding.                */
+#define RHSEG_FEATS_NHWC 0x20
 #define RHSEG_NSTAT 5            /* per (sample, class) loss statistics, see loss_stats   */
 #define RHSEG_MAX_LEVELS 8       /* tree depth rhseg_step_finalize handles in one launch  */
 #define RHSEG_STITCH_MAX_LEAVES 16 /* leaf channels of a flat model rhseg_stitch_levels reads */
@@ -121,7 +130,8 @@ int rhseg_head_level_fwd(const void* feats, const float* eff_w, const float* eff
  * low-res pass zeroes z_lo itself whenever pixel tiles are split between CTAs.
  * zero_psum bit 2 (value 4): eff_w / eff_b are ONE [K,C] / [K] pair shared by all samples (a level without
  * FiLM, i.e. level 0: pass the head's own weight and bias, no rhseg_film_fold launch).
- * zero_psum & RHSEG_FEATS_BF16: feats holds bf16 values (see RHSEG_FEATS_BF16).             */
+ * zero_psum & RHSEG_FEATS_BF16: feats holds bf16 values (see RHSEG_FEATS_BF16).
+ * zero_psum & RHSEG_FEATS_NHWC: feats is channels-last (see RHSEG_FEATS_NHWC).                */
 
 /* Level forward of an UPSAMPLED head (HRNet) fused with rhseg_level_eval: the hi-res pass that
  * interpolates and activates the logits also evaluates them against the ternary targets while
@@ -182,7 +192,7 @@ int rhseg_head_dz_lowres_fused(const float* logits, const float* targets, long t
  * atomics: zeroed here when zero_sums != 0, otherwise the caller passes zeroed buffers).
  * dfeats may be NULL (features do not require grad).
  * zero_sums bit 0: zero S / s here; bit 1 (value 2): eff_w is one [K,C] matrix shared by all samples;
- * RHSEG_FEATS_BF16: feats and dfeats are bf16.                                                       */
+ * RHSEG_FEATS_BF16: feats and dfeats are bf16; RHSEG_FEATS_NHWC: feats and dfeats are channels-last.      */
 int rhseg_head_conv_bwd(const void* feats, const float* dz, const float* eff_w,
                         int B, int C, int K, int n_pix,
                         void* dfeats, double* S, double* s, int zero_sums, void* stream);

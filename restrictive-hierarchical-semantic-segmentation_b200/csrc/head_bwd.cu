@@ -9,6 +9,10 @@
 
 namespace rhseg {
 
+// conv backward for channels-last features and dfeats (head_bwd_nhwc.cu): K dispatch included
+int conv_bwd_nhwc(bool bf16, int K, const void* feats, const float* dz, const float* eff_w, int B, int C, int N,
+                  void* dfeats, double* S, double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt);
+
 // ------------------------------------------------------------------------------------
 // activation backward, output resolution, elementwise
 // ------------------------------------------------------------------------------------
@@ -240,6 +244,13 @@ static int conv_bwd_impl(const void* feats_v, const float* dz, const float* eff_
     RHSEG_CUDA(cudaMemsetAsync(s, 0, sizeof(double) * (size_t)B * K, st));
   }
   const int sms = device_sm_count();
+  if (zero_sums & RHSEG_FEATS_NHWC) {
+    const bool bf16 = (zero_sums & RHSEG_FEATS_BF16) != 0;
+    if (((size_t)C * (bf16 ? 2 : 4)) % 16 != 0 ||
+        ((reinterpret_cast<uintptr_t>(feats_v) | reinterpret_cast<uintptr_t>(dfeats_v)) & 15u) != 0)
+      return RHSEG_ERR_UNSUPPORTED;
+    return conv_bwd_nhwc(bf16, K, feats_v, dz, eff_w, B, C, n_pix, dfeats_v, S, s, sms, st, w_shared, pt);
+  }
   if (zero_sums & RHSEG_FEATS_BF16) {
     if ((reinterpret_cast<uintptr_t>(feats_v) | reinterpret_cast<uintptr_t>(dfeats_v)) & 1u) return RHSEG_ERR_ARG;
     return conv_bwd_bf16(K, static_cast<const uint16_t*>(feats_v), dz, eff_w, B, C, n_pix, static_cast<uint16_t*>(dfeats_v),

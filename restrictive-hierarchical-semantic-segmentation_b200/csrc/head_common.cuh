@@ -35,6 +35,15 @@ int level_conv_bf16(const uint16_t* feats, const float* eff_w, const float* eff_
                     const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
                     bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
 
+// the same for channels-last features [B,Nf,C] (head_fwd_nhwc.cu, head_fwd_nhwc_bf16.cu): C * element size and the base
+// address are multiples of 16 bytes (checked by the caller)
+int level_conv_nhwc(const float* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
+                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
+                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
+int level_conv_nhwc(const uint16_t* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
+                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
+                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
+
 // ------------------------------------------------------------------------------------
 // Activation epilogue shared by the fused and the upsampled path.  P pixels per thread.
 // ------------------------------------------------------------------------------------

@@ -123,7 +123,17 @@ static int level_fwd_impl(const void* feats_v, const float* eff_w, const float* 
   if (ea && !up) return RHSEG_ERR_UNSUPPORTED;
   if (act_mode == RHSEG_ACT_GROUPED && table == nullptr) return RHSEG_ERR_ARG;
   const int Nf = Hf * Wf;
-  if (zero_psum & RHSEG_FEATS_BF16) {
+  if (zero_psum & RHSEG_FEATS_NHWC) {
+    const bool bf16 = (zero_psum & RHSEG_FEATS_BF16) != 0;
+    const size_t esz = bf16 ? 2 : 4;
+    if (((size_t)C * esz) % 16 != 0 || (reinterpret_cast<uintptr_t>(feats_v) & 15u) != 0) return RHSEG_ERR_UNSUPPORTED;
+    if (up && !z_lo) return RHSEG_ERR_ARG;
+    const int rc = bf16 ? level_conv_nhwc(static_cast<const uint16_t*>(feats_v), eff_w, eff_b, prev_probs, table, B, C, Nf, K,
+                                          K_prev, act_mode, up ? z_lo : nullptr, zlo_zeroed, logits, probs, psum, w_shared, st)
+                        : level_conv_nhwc(static_cast<const float*>(feats_v), eff_w, eff_b, prev_probs, table, B, C, Nf, K,
+                                          K_prev, act_mode, up ? z_lo : nullptr, zlo_zeroed, logits, probs, psum, w_shared, st);
+    if (rc != RHSEG_OK || !up) return rc;
+  } else if (zero_psum & RHSEG_FEATS_BF16) {
     const uint16_t* fb = static_cast<const uint16_t*>(feats_v);
     if (reinterpret_cast<uintptr_t>(fb) & 1u) return RHSEG_ERR_ARG;
     if (up && !z_lo) return RHSEG_ERR_ARG;
@@ -194,7 +204,7 @@ extern "C" int rhseg_head_level_fwd_eval(const void* feats, const float* eff_w, 
               reinterpret_cast<unsigned long long*>(cons + RHSEG_MAX_K), idx_out};
   bool need_eval = false;
   const int rc = level_fwd_impl(feats, eff_w, eff_b, prev_probs, table, B, C, Hf, Wf, H, W, K, K_prev, act_mode, z_lo, logits,
-                                probs, psum, (flags & (2 | 4 | RHSEG_FEATS_BF16)), stream, &ea, &need_eval);
+                                probs, psum, (flags & (2 | 4 | RHSEG_FEATS_BF16 | RHSEG_FEATS_NHWC)), stream, &ea, &need_eval);
   if (rc != RHSEG_OK || !need_eval) return rc;
   // shapes the band kernel does not take: the evaluation runs as its own kernel on the finished logits
   return rhseg_level_eval(logits, targets, t_bstride, t_cstride, parent_targets, pt_bstride, pt_cstride, prev_idx, table, B, K,

@@ -25,14 +25,33 @@ def _f32c(t: torch.Tensor) -> torch.Tensor:
     return t if t.is_contiguous() else t.contiguous()
 
 
-def _feats_c(feats: Sequence[torch.Tensor]) -> Tuple[List[torch.Tensor], int]:
-    """Contiguous per-level features and the kernels' element-type flag: float32, or bfloat16 on every level (donors
-    trained under torch.autocast; the kernels convert each value to fp32 exactly and store dfeats as bf16)."""
+def _nhwc_native(f: torch.Tensor) -> bool:
+    """Features the kernels read channels-last as they are (RHSEG_FEATS_NHWC): channels-last-contiguous but not
+    contiguous (so C = 1 and 1x1 planes, which are both, keep the NCHW path), a pixel's channels a multiple of 16 bytes
+    and at most 4096, a 16-byte aligned base."""
+    if f.dim() != 4 or f.is_contiguous() or not f.is_contiguous(memory_format=torch.channels_last):
+        return False
+    row = f.shape[1] * f.element_size()
+    return row % 16 == 0 and row <= 4096 and f.data_ptr() % 16 == 0
+
+
+def _feats_flag(f: torch.Tensor) -> int:
+    """Feature flags of the kernel calls for a tensor _feats_c returned: dtype, and layout (it returned only contiguous
+    tensors and the channels-last ones the kernels read natively)."""
+    return (native.FEATS_BF16 if f.dtype == torch.bfloat16 else 0) | (0 if f.is_contiguous() else native.FEATS_NHWC)
+
+
+def _feats_c(feats: Sequence[torch.Tensor]) -> Tuple[List[torch.Tensor], List[int]]:
+    """Per-level features as the kernels read them, and each level's flags (_feats_flag).  dtype: float32, or bfloat16
+    on every level (donors trained under torch.autocast; the kernels convert each value to fp32 exactly and store dfeats
+    as bf16).  Layout, per level: channels-last features (donors converted with torch.channels_last) are read in place
+    when _nhwc_native allows it, and their dfeats comes back channels-last; anything else is made contiguous."""
     dt = feats[0].dtype
     if dt not in (torch.float32, torch.bfloat16) or any(f.dtype != dt for f in feats):
         raise native.NativeError("rhseg_b200 head expects float32 or bfloat16 features (one dtype for every level), got %s"
                                  % ", ".join(sorted({str(f.dtype) for f in feats})))
-    return [f if f.is_contiguous() else f.contiguous() for f in feats], (native.FEATS_BF16 if dt == torch.bfloat16 else 0)
+    out = [f if f.is_contiguous() or _nhwc_native(f) else f.contiguous() for f in feats]
+    return out, [_feats_flag(f) for f in out]
 
 
 _SIDE_STREAMS = {}
@@ -53,8 +72,8 @@ def _side_stream(dev):
 
 def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words: int = 0, with_backward: bool = False):
     """Runs the per-level forward kernels.  `tensors` = feats[n] + head_w[n] + head_b[n] + film_w[n-1] +
-    film_b[n-1]; the features are fp32 or bf16 (_feats_c), everything else fp32.  Returns a dict with the inputs
-    (contiguous) and probs / logits / psums / eff_w /
+    film_b[n-1]; the features are fp32 or bf16, contiguous or channels-last (_feats_c), everything else fp32.
+    Returns a dict with the inputs (as the kernels read them) and probs / logits / psums / eff_w /
     gamma_beta per level plus the shape tuple.
     `evaluate(L, dims)` (fused training step) returns the rhseg_level_eval arguments of level L:
     (targets_ptr, t_bs, t_cs, parent_ptr, prev_idx_ptr, out_words_ptr, idx_out_ptr); the evaluation then runs
@@ -63,7 +82,7 @@ def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words
     `evaluate` as its third argument (the fused step's statistics workspace).  with_backward: the same fill also
     zeroes the accumulators of the backward pass (r["bwd"], see backward_buffers): ONE fill per training step."""
     n = tree.num_levels
-    feats, fbf = _feats_c(tensors[0:n])
+    feats, fflags = _feats_c(tensors[0:n])
     head_w = [_f32c(t) for t in tensors[n:2 * n]]
     head_b = [_f32c(t) for t in tensors[2 * n:3 * n]]
     film_w = [_f32c(t) for t in tensors[3 * n:4 * n - 1]]
@@ -95,7 +114,7 @@ def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words
     for L in range(n):
         K = tree.head_channels[L]
         K_prev = tree.head_channels[L - 1] if L > 0 else 0
-        f = feats[L]
+        f, fbf = feats[L], fflags[L]
         if tuple(f.shape) != (B, C, Hf, Wf):
             raise native.NativeError("per-level feature tensors must share one shape")
         if tuple(head_w[L].shape[:2]) != (K, C):
@@ -177,7 +196,7 @@ def level_weight_backward(tree, L, dims, feats_L, dz_feat, eff_w_L, head_w_L, fi
         d_fw = torch.empty_like(film_w_prev)
         d_fb = torch.empty((2 * C,), dtype=torch.float32, device=dev)
         g_prev = buf["gp"]
-    fbf = native.FEATS_BF16 if feats_L.dtype == torch.bfloat16 else 0  # d_feats: same dtype as the features
+    fbf = _feats_flag(feats_L)  # d_feats: same dtype and layout as the features (empty_like keeps channels-last)
     call("rhseg_head_conv_bwd_params", ptr(feats_L), ptr(dz_feat), ptr(eff_w_L), B, C, K, Hf * Wf, ptr(d_feats),
          ptr(buf["S"]), ptr(buf["s"]), (2 if L == 0 else 0) | 4 | fbf, ptr(head_w_L), ptr(film_w_prev) if L > 0 else None, ptr(gb_L),
          ptr(psum_prev) if L > 0 else None, float(H * W), K_prev, ptr(d_hw), ptr(d_hb), ptr(d_fw), ptr(d_fb), ptr(g_prev),

@@ -19,6 +19,7 @@ NSTAT = 5
 XCHG_HANDLE_BYTES = 64
 DZ_PREZEROED = 1
 FEATS_BF16 = 0x10  # RHSEG_FEATS_BF16: the feature (and dfeats) tensors of the call are bf16
+FEATS_NHWC = 0x20  # RHSEG_FEATS_NHWC: the feature (and dfeats) tensors of the call are channels-last [B,H,W,C]
 ACT_SIGMOID, ACT_GROUPED, ACT_ZEROS = 0, 1, 2
 
 _c = ctypes
