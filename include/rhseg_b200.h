@@ -197,16 +197,12 @@ int rhseg_head_conv_bwd(const void* feats, const float* dz, const float* eff_w,
                         int B, int C, int K, int n_pix,
                         void* dfeats, double* S, double* s, int zero_sums, void* stream);
 
-/* rhseg_head_conv_bwd followed by rhseg_head_param_grads in ONE launch: the last CTA to finish forms the parameter
- * gradients from the complete sums (no second kernel on the level chain).  Arguments: those of the two functions;
- * flags = zero_sums of rhseg_head_conv_bwd | 4 when g_prev is zero on entry (part of a larger zero fill; otherwise it is
- * zeroed here); n_pix_out = H*W of the output (the FiLM pool size); ticket = a device counter that is zero on entry (left
- * zero).  Two forms, same results: conv kernel + 12-CTA parameter kernel behind a programmatic dependent launch
- * (default, measured faster for C = 720), or the parameter gradients as the tail of the conv kernel's last CTA
- * (library built with -DRHSEG_WITH_PARAM_TAIL and RHSEG_PARAM_TAIL=1; compiled out by default because the tail costs
- * the conv kernel registers and, for 16-byte-aligned planes, its second CTA per SM).  Exception: a level WITHOUT FiLM
- * (film_w == NULL: d_head_w = sum_b S_b, d_head_b = sum_b s_b) of a narrow donor (B*C*K <= 4096) is always ONE launch,
- * the sums being formed by the conv kernel's last CTA.                                                            */
+/* rhseg_head_conv_bwd followed by rhseg_head_param_grads.  Arguments: those of the two functions; flags = zero_sums of
+ * rhseg_head_conv_bwd | 4 when g_prev is zero on entry (part of a larger zero fill; otherwise it is zeroed here);
+ * n_pix_out = H*W of the output (the FiLM pool size); ticket = a device counter that is zero on entry (left zero).
+ * Two forms, same results: a level WITHOUT FiLM (film_w == NULL: d_head_w = sum_b S_b, d_head_b = sum_b s_b) of a
+ * narrow donor (B*C*K <= 4096) is ONE launch, the sums being formed by the conv kernel's last CTA; every other level
+ * is the conv kernel + the 12-CTA parameter kernel behind a programmatic dependent launch.                         */
 int rhseg_head_conv_bwd_params(const void* feats, const float* dz, const float* eff_w, int B, int C, int K,
                                int n_pix, void* dfeats, double* S, double* s, int flags, const float* head_w,
                                const float* film_w, const float* gamma_beta, const double* prev_psum,

@@ -182,6 +182,25 @@ __device__ __forceinline__ Vec<VEC> ld_cached(const float* p) {
   return r;
 }
 
+// the KP weights of one channel in a [C][KP] shared-memory table of the conv kernels (p = its row): vector loads that
+// every thread of a warp reads at the same address (broadcast)
+template <int KP>
+__device__ __forceinline__ void ld_wvec(const float* p, float (&w)[KP]) {
+  if constexpr (KP == 4) {
+    const float4 t = *reinterpret_cast<const float4*>(p);
+    w[0] = t.x; w[1] = t.y; w[2] = t.z; w[3] = t.w;
+  } else if constexpr (KP == 8) {
+    const float4 t0 = *reinterpret_cast<const float4*>(p);
+    const float4 t1 = *reinterpret_cast<const float4*>(p + 4);
+    w[0] = t0.x; w[1] = t0.y; w[2] = t0.z; w[3] = t0.w; w[4] = t1.x; w[5] = t1.y; w[6] = t1.z; w[7] = t1.w;
+  } else if constexpr (KP == 2) {
+    const float2 t = *reinterpret_cast<const float2*>(p);
+    w[0] = t.x; w[1] = t.y;
+  } else {
+    w[0] = p[0];
+  }
+}
+
 template <int VEC>
 __device__ __forceinline__ void st_stream(float* p, const Vec<VEC>& r) {
   if constexpr (VEC == 4) {

@@ -38,102 +38,40 @@ __device__ __forceinline__ void st_feats(uint16_t* p, const Vec<VEC>& r) {
 // (KP-1 + 5-log2(KP) shuffles).  The per-channel sums of the current (sample, stage) segment
 // stay in registers across tiles and leave the warp as fp64 atomics when the segment ends.
 // ------------------------------------------------------------------------------------
-// ------------------------------------------------------------------------------------
-// Parameter gradients as the TAIL of the conv backward (no second launch, no launch gap on the level chain):
-// every CTA takes a ticket when its share of S / s has been added; the last one forms, from the complete sums,
-//   d_head_w = sum_b (S_b diag(gamma_b) + s_b beta_b^T),  d_head_b = sum_b s_b,
-//   dgamma_b[c] = sum_k S_b[k,c] W[k,c],  dbeta_b = W^T s_b,  d_film_w = sum_b [dgamma|dbeta]_b cond_b^T,
-//   d_film_b = sum_b [dgamma|dbeta]_b,  g_prev[b] = film_w^T [dgamma|dbeta]_b
-// (closed forms: DESIGN.md 3.5).  Same arguments as rhseg_head_param_grads; all sums in fp64.
-// ------------------------------------------------------------------------------------
+
+// Level WITHOUT FiLM (level 0): its parameter gradients are plain sums over the batch, d_head_w = sum_b S_b and
+// d_head_b = sum_b s_b.  With a ticket, the last CTA of the conv backward forms them (a few thousand L2 loads) instead of
+// a second kernel at the very end of the step.  Levels with FiLM take rhseg_head_param_grads.
 struct ParamTail {
   unsigned* ticket;  // device counter, zero on entry, left zero; nullptr = no tail
-  const float* head_w;
-  const float* film_w;
-  const float* gamma_beta;
-  const double* prev_psum;
-  double n_pix;
-  int B, K_prev;
+  int B;
   float* d_head_w;
   float* d_head_b;
-  float* d_film_w;
-  float* d_film_b;
-  double* g_prev;
 };
 
+// called by the nthr consumer threads of every CTA once its share of S / s has been added
 template <int K>
-__device__ __noinline__ void param_grads_tail(const ParamTail& pt, const double* __restrict__ S, const double* __restrict__ s, int C,
-                                              double* sm /* shared: B*K_prev + 2*B*C doubles */, int tid, int nthr) {
-  const int B = pt.B, Kp = pt.film_w ? pt.K_prev : 0;
-  const int lane = tid & 31, warp = tid >> 5, nwarp = nthr >> 5;
-  double* cond = sm;                    // [B][Kp]  pooled probabilities of the previous level (fp32 values, as in the forward)
-  double* dg = sm + (size_t)B * Kp;     // [B][C]   dgamma
-  double* db = dg + (size_t)B * C;      // [B][C]   dbeta
-  for (int i = tid; i < B * Kp; i += nthr) cond[i] = (double)(float)fast_div(pt.prev_psum[i], pt.n_pix);
+__device__ __forceinline__ void level0_param_tail(const ParamTail& pt, const double* __restrict__ S,
+                                                  const double* __restrict__ s, int C, int nthr) {
+  __shared__ int last_cta;
+  const int tid = threadIdx.x;
+  __threadfence();
   consumer_sync(nthr);
-  // phase 1: thread <-> channel; every load of a channel is independent of the others (no barrier inside)
-  for (int c = tid; c < C; c += nthr) {
-    float w[K];
-#pragma unroll
-    for (int k = 0; k < K; ++k) w[k] = pt.head_w[(size_t)k * C + c];
-    double dw[K], dfb_g = 0.0, dfb_b = 0.0, dfw_g[RHSEG_MAX_K], dfw_b[RHSEG_MAX_K];
-#pragma unroll
-    for (int k = 0; k < K; ++k) dw[k] = 0.0;
-#pragma unroll
-    for (int j = 0; j < RHSEG_MAX_K; ++j) { dfw_g[j] = 0.0; dfw_b[j] = 0.0; }
-    for (int b = 0; b < B; ++b) {
-      const double gam = Kp ? (double)pt.gamma_beta[(size_t)b * 2 * C + c] : 1.0;
-      const double bet = Kp ? (double)pt.gamma_beta[(size_t)b * 2 * C + C + c] : 0.0;
-      double dgam = 0.0, dbet = 0.0;
-#pragma unroll
-      for (int k = 0; k < K; ++k) {
-        const double Sv = __ldcg(S + ((size_t)b * K + k) * C + c);  // accumulated by other CTAs' atomics: read at L2
-        const double sv = __ldcg(s + b * K + k);
-        dw[k] += Sv * gam + sv * bet;
-        dgam += Sv * (double)w[k];
-        dbet += (double)w[k] * sv;
-      }
-      if (Kp) {
-        dfb_g += dgam;
-        dfb_b += dbet;
-        dg[(size_t)b * C + c] = dgam;
-        db[(size_t)b * C + c] = dbet;
-#pragma unroll
-        for (int j = 0; j < RHSEG_MAX_K; ++j)
-          if (j < Kp) {
-            dfw_g[j] += dgam * cond[b * Kp + j];
-            dfw_b[j] += dbet * cond[b * Kp + j];
-          }
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < K; ++k) pt.d_head_w[(size_t)k * C + c] = (float)dw[k];
-    if (Kp) {
-      pt.d_film_b[c] = (float)dfb_g;
-      pt.d_film_b[C + c] = (float)dfb_b;
-#pragma unroll
-      for (int j = 0; j < RHSEG_MAX_K; ++j)
-        if (j < Kp) {
-          pt.d_film_w[(size_t)c * Kp + j] = (float)dfw_g[j];
-          pt.d_film_w[(size_t)(C + c) * Kp + j] = (float)dfw_b[j];
-        }
-    }
-  }
-  if (tid < K) {
-    double acc = 0.0;
-    for (int b = 0; b < B; ++b) acc += __ldcg(s + b * K + tid);
-    pt.d_head_b[tid] = (float)acc;
-  }
-  if (Kp == 0) return;
+  if (tid == 0) last_cta = (atomicAdd(pt.ticket, 1u) == gridDim.x - 1) ? 1 : 0;
   consumer_sync(nthr);
-  // phase 2: g_prev[b][j] = sum_c film_w[c][j] dgamma[b][c] + film_w[C+c][j] dbeta[b][c]: one warp per (b, j) pair
-  for (int p = warp; p < B * Kp; p += nwarp) {
-    const int b = p / Kp, j = p - b * Kp;
-    double acc = 0.0;
-    for (int c = lane; c < C; c += 32)
-      acc += (double)pt.film_w[(size_t)c * Kp + j] * dg[(size_t)b * C + c] + (double)pt.film_w[(size_t)(C + c) * Kp + j] * db[(size_t)b * C + c];
-    acc = warp_sum(acc);
-    if (lane == 0) pt.g_prev[p] = acc;
+  if (last_cta) {
+    __threadfence();
+    for (int i = tid; i < K * C; i += nthr) {
+      double a = 0.0;
+      for (int bb = 0; bb < pt.B; ++bb) a += __ldcg(S + (size_t)bb * K * C + i);  // accumulated by other CTAs: read at L2
+      pt.d_head_w[i] = (float)a;
+    }
+    if (tid < K) {
+      double a = 0.0;
+      for (int bb = 0; bb < pt.B; ++bb) a += __ldcg(s + bb * K + tid);
+      pt.d_head_b[tid] = (float)a;
+    }
+    if (tid == 0) *pt.ticket = 0u;  // ready for the next launch / graph replay
   }
 }
 
@@ -167,15 +105,7 @@ conv_bwd_kernel(const FT* __restrict__ feats, const float* __restrict__ dz, cons
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long u_begin = units_total * blockIdx.x / gridDim.x;
   const long u_end = units_total * (blockIdx.x + 1) / gridDim.x;
-
-  if (tid == 0) {
-    for (int i = 0; i < NS; ++i) {
-      mbar_init(smem_u32(&bars[i]), CFG::NPW);
-      mbar_init(smem_u32(&bars[NS + i]), CFG::NCW);
-    }
-    mbar_fence_init();
-  }
-  __syncthreads();
+  ring_bars_init<NS>(bars, CFG::NPW, CFG::NCW);
 
   // Unit order: sample b -> GROUP of `group` consecutive pixel tiles -> channel stage -> tile of the group.
   // group >= n_tiles is the plain order (b, stage, tile).  Large planes x large batches (UNet 1024^2, batch 8..64) use
@@ -334,19 +264,7 @@ conv_bwd_kernel(const FT* __restrict__ feats, const float* __restrict__ dz, cons
     auto channel = [&](int cc, int offv, float& acc_out) {
       const FT* row = stage_base + cc * ROWP;
       float w[KP];
-      if constexpr (KP == 4) {
-        const float4 t = *reinterpret_cast<const float4*>(w_s + cc * KP);
-        w[0] = t.x; w[1] = t.y; w[2] = t.z; w[3] = t.w;
-      } else if constexpr (KP == 8) {
-        const float4 t0 = *reinterpret_cast<const float4*>(w_s + cc * KP);
-        const float4 t1 = *reinterpret_cast<const float4*>(w_s + cc * KP + 4);
-        w[0] = t0.x; w[1] = t0.y; w[2] = t0.z; w[3] = t0.w; w[4] = t1.x; w[5] = t1.y; w[6] = t1.z; w[7] = t1.w;
-      } else if constexpr (KP == 2) {
-        const float2 t = *reinterpret_cast<const float2*>(w_s + cc * KP);
-        w[0] = t.x; w[1] = t.y;
-      } else {
-        w[0] = w_s[cc];
-      }
+      ld_wvec<KP>(w_s + cc * KP, w);
       float part[KP];
 #pragma unroll
       for (int k = 0; k < KP; ++k) part[k] = 0.f;
@@ -413,48 +331,7 @@ conv_bwd_kernel(const FT* __restrict__ feats, const float* __restrict__ dz, cons
     advance();
   }
   if (cur_seg >= 0) flush();
-  // Level WITHOUT FiLM (level 0): its parameter gradients are plain sums over the batch, d_head_w = sum_b S_b and
-  // d_head_b = sum_b s_b.  The last CTA to finish forms them here (a few thousand L2 loads) instead of a second kernel
-  // at the very end of the step.  (The FiLM'd levels keep the separate 12-CTA kernel: their tail is the slower form.)
-  if (pt.ticket != nullptr && pt.film_w == nullptr) {
-    __shared__ int last_cta;
-    __threadfence();
-    consumer_sync(NCONS);
-    if (tid == 0) last_cta = (atomicAdd(pt.ticket, 1u) == gridDim.x - 1) ? 1 : 0;
-    consumer_sync(NCONS);
-    if (last_cta) {
-      __threadfence();
-      for (int i = tid; i < K * C; i += NCONS) {
-        double a = 0.0;
-        for (int bb = 0; bb < pt.B; ++bb) a += __ldcg(S + (size_t)bb * K * C + i);  // accumulated by other CTAs: read at L2
-        pt.d_head_w[i] = (float)a;
-      }
-      if (tid < K) {
-        double a = 0.0;
-        for (int bb = 0; bb < pt.B; ++bb) a += __ldcg(s + bb * K + tid);
-        pt.d_head_b[tid] = (float)a;
-      }
-      if (tid == 0) *pt.ticket = 0u;  // ready for the next launch / graph replay
-    }
-  }
-#ifdef RHSEG_WITH_PARAM_TAIL
-  // Compiled out by default: measured slower than the separate 12-CTA kernel (25 us against 8.6 us at C = 720), and the
-  // call into the tail raised the 128-bit instance of this kernel from 96 to 128 registers, i.e. from two CTAs per SM
-  // to one (UNet conv backward 0.81 -> 0.75 of the HBM peak).
-  if (pt.ticket != nullptr && pt.film_w != nullptr) {
-    // last CTA done: S / s are complete -> parameter gradients (the ring is free: its memory holds the pool-gradient sums)
-    __shared__ int is_last;
-    __threadfence();
-    consumer_sync(NCONS);
-    if (tid == 0) is_last = (atomicAdd(pt.ticket, 1u) == gridDim.x - 1) ? 1 : 0;
-    consumer_sync(NCONS);
-    if (is_last) {
-      __threadfence();
-      param_grads_tail<K>(pt, S, s, C, reinterpret_cast<double*>(ring), tid, NCONS);
-      if (tid == 0) *pt.ticket = 0u;  // ready for the next launch / graph replay
-    }
-  }
-#endif
+  if (pt.ticket != nullptr) level0_param_tail<K>(pt, S, s, C, NCONS);
 }
 
 template <typename FT, int K, int VEC, int J, typename CFG>
@@ -486,11 +363,27 @@ static int launch_conv_bwd(const FT* feats, const float* dz, const float* eff_w,
   return RHSEG_OK;
 }
 
-// conv backward with bf16 features and dfeats (head_bwd_bf16.cu): K dispatch and ring shapes included
-int conv_bwd_bf16(int K, const uint16_t* feats, const float* dz, const float* eff_w, int B, int C, int N, uint16_t* dfeats,
-                  double* S, double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt);
-
 using BwdCfgV4 = PipeCfg<8, 8, 3>;  // 8 consumer warps x float4 -> T = 1024 px, 4 KB row copies, 33 KB stages
 using BwdCfgS1 = PipeCfg<8, 16, 2>;  // scalar rows: T = 256*J px, 66 KB stages (dz reused over 16 channels)
+
+// Conv backward of NCHW features and dfeats [B,C,N], K dispatch and ring shapes included.  Instances: fp32 in
+// head_bwd.cu, bf16 (feats / dfeats = bf16 bit patterns, 2-byte aligned) in head_bwd_bf16.cu.
+template <typename FT>
+int conv_bwd_nchw(int K, const FT* feats, const float* dz, const float* eff_w, int B, int C, int N, FT* dfeats, double* S,
+                  double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt) {
+  const bool v4 = (N % FeatElem<FT>::G == 0) &&
+                  (((reinterpret_cast<uintptr_t>(feats) | reinterpret_cast<uintptr_t>(dz) | reinterpret_cast<uintptr_t>(dfeats)) & 15u) == 0);
+  RHSEG_DISPATCH_K(K, {
+    if (v4) return launch_conv_bwd<FT, KK, 4, 1, BwdCfgV4>(feats, dz, eff_w, B, C, N, dfeats, S, s, sm_count, st, w_shared, pt);
+    return launch_conv_bwd<FT, KK, 1, (KK <= 4 ? 4 : 2), BwdCfgS1>(feats, dz, eff_w, B, C, N, dfeats, S, s, sm_count, st, w_shared,
+                                                                   pt);
+  });
+  return RHSEG_OK;
+}
+
+// conv backward of channels-last features and dfeats [B,N,C] (head_bwd_nhwc.cu): K dispatch included
+template <typename FT>
+int conv_bwd_nhwc(int K, const FT* feats, const float* dz, const float* eff_w, int B, int C, int N, FT* dfeats, double* S,
+                  double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt);
 
 }  // namespace rhseg

@@ -9,9 +9,11 @@
 
 namespace rhseg {
 
-// conv backward for channels-last features and dfeats (head_bwd_nhwc.cu): K dispatch included
-int conv_bwd_nhwc(bool bf16, int K, const void* feats, const float* dz, const float* eff_w, int B, int C, int N,
-                  void* dfeats, double* S, double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt);
+// the fp32 instances of the NCHW conv backward compile here, the bf16 ones in head_bwd_bf16.cu
+template int conv_bwd_nchw<float>(int, const float*, const float*, const float*, int, int, int, float*, double*, double*, int,
+                                  cudaStream_t, int, const ParamTail&);
+extern template int conv_bwd_nchw<uint16_t>(int, const uint16_t*, const float*, const float*, int, int, int, uint16_t*, double*,
+                                            double*, int, cudaStream_t, int, const ParamTail&);
 
 // ------------------------------------------------------------------------------------
 // activation backward, output resolution, elementwise
@@ -88,11 +90,6 @@ act_bwd_kernel(const float* __restrict__ logits, const float* __restrict__ prev_
     for (int v = 0; v < VEC; ++v) o.v[v] = dz[k][v];
     *reinterpret_cast<Vec<VEC>*>(dz_out + base + (size_t)k * N) = o;
   }
-}
-
-static int tune_env(const char* name) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : 0;
 }
 
 // ------------------------------------------------------------------------------------
@@ -243,48 +240,25 @@ static int conv_bwd_impl(const void* feats_v, const float* dz, const float* eff_
     RHSEG_CUDA(cudaMemsetAsync(S, 0, sizeof(double) * (size_t)B * K * C, st));
     RHSEG_CUDA(cudaMemsetAsync(s, 0, sizeof(double) * (size_t)B * K, st));
   }
+  const bool nhwc = (zero_sums & RHSEG_FEATS_NHWC) != 0, bf16 = (zero_sums & RHSEG_FEATS_BF16) != 0;
+  const uintptr_t addr = reinterpret_cast<uintptr_t>(feats_v) | reinterpret_cast<uintptr_t>(dfeats_v);
+  if (nhwc) {
+    if (((size_t)C * (bf16 ? 2 : 4)) % 16 != 0 || (addr & 15u) != 0) return RHSEG_ERR_UNSUPPORTED;
+  } else if (bf16 && (addr & 1u)) {
+    return RHSEG_ERR_ARG;
+  }
   const int sms = device_sm_count();
-  if (zero_sums & RHSEG_FEATS_NHWC) {
-    const bool bf16 = (zero_sums & RHSEG_FEATS_BF16) != 0;
-    if (((size_t)C * (bf16 ? 2 : 4)) % 16 != 0 ||
-        ((reinterpret_cast<uintptr_t>(feats_v) | reinterpret_cast<uintptr_t>(dfeats_v)) & 15u) != 0)
-      return RHSEG_ERR_UNSUPPORTED;
-    return conv_bwd_nhwc(bf16, K, feats_v, dz, eff_w, B, C, n_pix, dfeats_v, S, s, sms, st, w_shared, pt);
-  }
-  if (zero_sums & RHSEG_FEATS_BF16) {
-    if ((reinterpret_cast<uintptr_t>(feats_v) | reinterpret_cast<uintptr_t>(dfeats_v)) & 1u) return RHSEG_ERR_ARG;
-    return conv_bwd_bf16(K, static_cast<const uint16_t*>(feats_v), dz, eff_w, B, C, n_pix, static_cast<uint16_t*>(dfeats_v),
-                         S, s, sms, st, w_shared, pt);
-  }
-  const float* feats = static_cast<const float*>(feats_v);
-  float* dfeats = static_cast<float*>(dfeats_v);
-  RHSEG_DISPATCH_K(K, {
-    const bool v4 = (n_pix % 4 == 0) && ((reinterpret_cast<uintptr_t>(feats) & 15u) == 0) &&
-                    ((reinterpret_cast<uintptr_t>(dz) & 15u) == 0) && ((reinterpret_cast<uintptr_t>(dfeats) & 15u) == 0);
-    if (v4) {
-      if constexpr (KK == 4) {
-        const int t = tune_env("RHSEG_TUNE_BWD_V4");
-        if (t == 1) return launch_conv_bwd<float, KK, 4, 1, PipeCfg<4, 8, 3>>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-        if (t == 2) return launch_conv_bwd<float, KK, 4, 1, PipeCfg<8, 16, 2>>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-        if (t == 3) return launch_conv_bwd<float, KK, 4, 1, PipeCfg<8, 16, 3>>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-      }
-      return launch_conv_bwd<float, KK, 4, 1, BwdCfgV4>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-    }
-    if constexpr (KK == 4) {
-      const int t = tune_env("RHSEG_TUNE_BWD_S1");
-      if (t == 1) return launch_conv_bwd<float, KK, 1, 4, PipeCfg<8, 16, 3>>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-      if (t == 2) return launch_conv_bwd<float, KK, 1, 4, PipeCfg<8, 24, 2>>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-      if (t == 3) return launch_conv_bwd<float, KK, 1, 4, PipeCfg<8, 16, 2>>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-    }
-    return launch_conv_bwd<float, KK, 1, (KK <= 4 ? 4 : 2), BwdCfgS1>(feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
-  });
-  return RHSEG_OK;
+  auto conv = [&](auto feats, auto dfeats) {
+    return nhwc ? conv_bwd_nhwc(K, feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt)
+                : conv_bwd_nchw(K, feats, dz, eff_w, B, C, n_pix, dfeats, S, s, sms, st, w_shared, pt);
+  };
+  return bf16 ? conv(static_cast<const uint16_t*>(feats_v), static_cast<uint16_t*>(dfeats_v))
+              : conv(static_cast<const float*>(feats_v), static_cast<float*>(dfeats_v));
 }
 
 extern "C" int rhseg_head_conv_bwd(const void* feats, const float* dz, const float* eff_w, int B, int C, int K,
                                    int n_pix, void* dfeats, double* S, double* s, int zero_sums, void* stream) {
-  ParamTail none{};
-  return conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, zero_sums, stream, none);
+  return conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, zero_sums, stream, ParamTail{});
 }
 
 extern "C" int rhseg_head_conv_bwd_params(const void* feats, const float* dz, const float* eff_w, int B, int C, int K,
@@ -297,32 +271,16 @@ extern "C" int rhseg_head_conv_bwd_params(const void* feats, const float* dz, co
     if (!gamma_beta || !prev_psum || !d_film_w || !d_film_b || !g_prev || n_pix_out <= 0) return RHSEG_ERR_ARG;
     if (K_prev < 1 || K_prev > RHSEG_MAX_K) return RHSEG_ERR_UNSUPPORTED;
   }
-  // Measured (HRNet-W48 tl, B = 4): the single-CTA tail costs 25 us per launch against 8.6 us for the 12-CTA
-  // rhseg_head_param_grads kernel behind a programmatic dependent launch, so the two-kernel form is the default;
-  // RHSEG_PARAM_TAIL=1 selects the tail (kept for small C / B where one CTA is enough).
-  static int use_tail = -1;
-#ifdef RHSEG_WITH_PARAM_TAIL
-  if (use_tail < 0) { const char* e = getenv("RHSEG_PARAM_TAIL"); use_tail = (e && e[0] == '1') ? 1 : 0; }
-#else
-  use_tail = 0;
-#endif
   // level 0 of a narrow donor: the batch sums are formed by the conv kernel's last CTA.  Measured: UNet (K*C*B = 1024 sums)
   // 0.5507 vs 0.5538 ms per step with the separate kernel; HRNet-W48 (11520 sums through one CTA) 0.4207 vs 0.4166 -> kept
   // for small heads only.
-  if (!film_w && (long)K * C * B <= 4096 && !getenv("RHSEG_NO_L0_TAIL")) {
-    ParamTail pt{ticket, head_w, nullptr, nullptr, nullptr, n_pix_out, B, 0, d_head_w, d_head_b, nullptr, nullptr, nullptr};
-    return conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, flags, stream, pt);
-  }
-  if (!use_tail || (film_w && ((long)B * K_prev + 2L * B * C) * 8 > 60 * 1024)) {
-    ParamTail none{};
-    const int rc = conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, flags, stream, none);
-    if (rc != RHSEG_OK) return rc;
-    // g_prev: the caller's buffer is zero on entry when bit 2 (value 4) of flags is set (part of a larger zero fill)
-    return rhseg_head_param_grads(S, s, head_w, film_w, gamma_beta, prev_psum, n_pix_out, B, C, K, K_prev, d_head_w, d_head_b,
-                                  d_film_w, d_film_b, g_prev, (flags & 4) ? 1 : 0, stream);
-  }
-  ParamTail pt{ticket, head_w, film_w, gamma_beta, prev_psum, n_pix_out, B, K_prev, d_head_w, d_head_b, d_film_w, d_film_b, g_prev};
-  return conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, flags, stream, pt);
+  if (!film_w && (long)K * C * B <= 4096 && !getenv("RHSEG_NO_L0_TAIL"))
+    return conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, flags, stream, ParamTail{ticket, B, d_head_w, d_head_b});
+  const int rc = conv_bwd_impl(feats, dz, eff_w, B, C, K, n_pix, dfeats, S, s, flags, stream, ParamTail{});
+  if (rc != RHSEG_OK) return rc;
+  // g_prev: the caller's buffer is zero on entry when bit 2 (value 4) of flags is set (part of a larger zero fill)
+  return rhseg_head_param_grads(S, s, head_w, film_w, gamma_beta, prev_psum, n_pix_out, B, C, K, K_prev, d_head_w, d_head_b,
+                                d_film_w, d_film_b, g_prev, (flags & 4) ? 1 : 0, stream);
 }
 
 extern "C" int rhseg_head_param_grads(const double* S, const double* s, const float* head_w, const float* film_w,

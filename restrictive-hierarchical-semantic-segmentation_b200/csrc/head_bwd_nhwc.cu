@@ -51,15 +51,7 @@ conv_bwd_nhwc_kernel(const FT* __restrict__ feats, const float* __restrict__ dz,
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long u_begin = units_total * blockIdx.x / gridDim.x;
   const long u_end = units_total * (blockIdx.x + 1) / gridDim.x;
-
-  if (tid == 0) {
-    for (int i = 0; i < NS; ++i) {
-      mbar_init(smem_u32(&bars[i]), 1);
-      mbar_init(smem_u32(&bars[NS + i]), ncw);
-    }
-    mbar_fence_init();
-  }
-  __syncthreads();
+  ring_bars_init<NS>(bars, 1, ncw);
 
   if (warp >= ncw) {
     // ------------------------------ producer ------------------------------
@@ -176,29 +168,7 @@ conv_bwd_nhwc_kernel(const FT* __restrict__ feats, const float* __restrict__ dz,
     if (++slot == NS) { slot = 0; phase ^= 1u; }
   }
   if (cur_b >= 0) flush(cur_b);
-  // level without FiLM of a narrow donor: d_head_w = sum_b S_b, d_head_b = sum_b s_b formed by the last CTA (as
-  // conv_bwd_kernel does)
-  if (pt.ticket != nullptr) {
-    __shared__ int last_cta;
-    __threadfence();
-    consumer_sync(ncons);
-    if (tid == 0) last_cta = (atomicAdd(pt.ticket, 1u) == gridDim.x - 1) ? 1 : 0;
-    consumer_sync(ncons);
-    if (last_cta) {
-      __threadfence();
-      for (int i = tid; i < K * C; i += ncons) {
-        double a = 0.0;
-        for (int bb = 0; bb < pt.B; ++bb) a += __ldcg(S + (size_t)bb * K * C + i);
-        pt.d_head_w[i] = (float)a;
-      }
-      if (tid < K) {
-        double a = 0.0;
-        for (int bb = 0; bb < pt.B; ++bb) a += __ldcg(s + bb * K + tid);
-        pt.d_head_b[tid] = (float)a;
-      }
-      if (tid == 0) *pt.ticket = 0u;
-    }
-  }
+  if (pt.ticket != nullptr) level0_param_tail<K>(pt, S, s, C, ncons);
 }
 
 template <typename FT, int K>
@@ -207,7 +177,6 @@ static int launch_conv_bwd_nhwc(const FT* feats, const float* dz, const float* e
   constexpr int VC = 16 / (int)sizeof(FT);
   const int NG = C / VC;
   if (NG > BWD_NHWC_MAX_CONS) return RHSEG_ERR_UNSUPPORTED;
-  if (pt.ticket != nullptr && pt.film_w != nullptr) return RHSEG_ERR_UNSUPPORTED;  // only the level-0 tail
   const int PL = BWD_NHWC_MAX_CONS / NG;
   const int ncons = (PL * NG + 31) / 32 * 32;
   const size_t pix_bytes = (size_t)C * sizeof(FT);
@@ -226,16 +195,17 @@ static int launch_conv_bwd_nhwc(const FT* feats, const float* dz, const float* e
   return RHSEG_OK;
 }
 
-int conv_bwd_nhwc(bool bf16, int K, const void* feats, const float* dz, const float* eff_w, int B, int C, int N,
-                  void* dfeats, double* S, double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt) {
+template <typename FT>
+int conv_bwd_nhwc(int K, const FT* feats, const float* dz, const float* eff_w, int B, int C, int N, FT* dfeats, double* S,
+                  double* s, int sm_count, cudaStream_t st, int w_shared, const ParamTail& pt) {
   RHSEG_DISPATCH_K(K, {
-    if (bf16)
-      return launch_conv_bwd_nhwc<uint16_t, KK>(static_cast<const uint16_t*>(feats), dz, eff_w, B, C, N,
-                                                static_cast<uint16_t*>(dfeats), S, s, sm_count, st, w_shared, pt);
-    return launch_conv_bwd_nhwc<float, KK>(static_cast<const float*>(feats), dz, eff_w, B, C, N, static_cast<float*>(dfeats),
-                                           S, s, sm_count, st, w_shared, pt);
+    return launch_conv_bwd_nhwc<FT, KK>(feats, dz, eff_w, B, C, N, dfeats, S, s, sm_count, st, w_shared, pt);
   });
   return RHSEG_OK;
 }
+template int conv_bwd_nhwc<float>(int, const float*, const float*, const float*, int, int, int, float*, double*, double*, int,
+                                  cudaStream_t, int, const ParamTail&);
+template int conv_bwd_nhwc<uint16_t>(int, const uint16_t*, const float*, const float*, int, int, int, uint16_t*, double*,
+                                     double*, int, cudaStream_t, int, const ParamTail&);
 
 }  // namespace rhseg

@@ -1,6 +1,6 @@
-// Pieces shared by head_fwd.cu (feature-streaming forward conv) and head_up.cu (output-resolution upsample +
+// Pieces shared by the feature-streaming forward conv (head_fwd*.cu) and head_up.cu (output-resolution upsample +
 // activation + fused evaluation): the activation epilogue, the FiLM-pool block sum, the evaluation arguments and
-// the dispatcher of the hi-res pass.  Two translation units so that they compile in parallel.
+// the dispatchers of both passes.  Separate translation units so that they compile in parallel.
 #pragma once
 #include "common.cuh"
 
@@ -28,21 +28,20 @@ int fwd_upsampled_dispatch(int K, int act_arg, const float* z_lo, const float* p
                            int Hf, int Wf, int H, int W, int K_prev, float* logits, float* probs, double* psum,
                            cudaStream_t st, const EvalArgs* ea, bool* need_eval);
 
-// feature conv of the level forward for bf16 features (head_fwd_bf16.cu).  z_lo == nullptr: a head at feature
+// Feature conv of the level forward, FT = float or uint16_t (bf16 bit patterns).  z_lo == nullptr: a head at feature
 // resolution, conv + activation into logits / probs / psum; otherwise the low-res conv of an upsampled head into
-// z_lo [B,K,Nf] (zeroed by the caller when zlo_zeroed).  feats = bf16 bit patterns, 2-byte aligned.
-int level_conv_bf16(const uint16_t* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
-                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
-
-// the same for channels-last features [B,Nf,C] (head_fwd_nhwc.cu, head_fwd_nhwc_bf16.cu): C * element size and the base
-// address are multiples of 16 bytes (checked by the caller)
-int level_conv_nhwc(const float* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
-                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
-int level_conv_nhwc(const uint16_t* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
-                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st);
+// z_lo [B,K,Nf] (zeroed by the caller when zlo_zeroed).  K dispatch and tile shapes included.
+// NCHW features [B,C,Nf], element-aligned (head_fwd_kernel.cuh; instances in head_fwd.cu, head_fwd_bf16.cu):
+template <typename FT>
+int level_conv_nchw(const FT* feats, const float* eff_w, const float* eff_b, const float* prev_probs, const int32_t* table,
+                    int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo, bool zlo_zeroed, float* logits,
+                    float* probs, double* psum, int w_shared, cudaStream_t st);
+// channels-last features [B,Nf,C], C * element size and the base address multiples of 16 bytes (head_fwd_nhwc.cuh;
+// instances in head_fwd_nhwc.cu, head_fwd_nhwc_bf16.cu):
+template <typename FT>
+int level_conv_nhwc(const FT* feats, const float* eff_w, const float* eff_b, const float* prev_probs, const int32_t* table,
+                    int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo, bool zlo_zeroed, float* logits,
+                    float* probs, double* psum, int w_shared, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------
 // Activation epilogue shared by the fused and the upsampled path.  P pixels per thread.

@@ -2,8 +2,6 @@
 // low-resolution conv of upsampled heads (HRNet; the hi-res pass lives in head_up.cu).
 // Reference semantics: Models/models.py:58-77 (FiLM), :177-184/:268/:280 (1x1 heads),
 // :269/:288-302 (sigmoid, restrictive softmax, composition, concat), :766/:776 (upsample).
-#include <algorithm>
-#include <cstdlib>
 #include "head_fwd_kernel.cuh"
 
 namespace rhseg {
@@ -61,27 +59,12 @@ __global__ void film_fold_kernel(const float* __restrict__ head_w, const float* 
   }
 }
 
-static int tune_env(const char* name) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : 0;
-}
-
-template <int K, int MODE>
-static int fwd_fullres(const float* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                       const int32_t* table, int B, int C, int N, int K_prev, float* logits, float* probs,
-                       double* psum, cudaStream_t st, int w_shared) {
-  const bool v4 = rows_vec4(feats, N) && rows_vec4(logits, N) && rows_vec4(probs, N) && (!prev_probs || rows_vec4(prev_probs, N));
-  if (v4) {
-    if constexpr (K == 4) {
-      const int t = tune_env("RHSEG_TUNE_FWD_V4");
-      if (t == 1) return launch_fwd<float, K, 4, 1, MODE, PipeCfg<4, 8, 4>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-      if (t == 2) return launch_fwd<float, K, 4, 1, MODE, PipeCfg<8, 16, 2>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-      if (t == 3) return launch_fwd<float, K, 4, 1, MODE, PipeCfg<8, 16, 3>>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-    }
-    return launch_fwd<float, K, 4, 1, MODE, FwdCfgV4>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-  }
-  return launch_fwd<float, K, 1, 2, MODE, FwdCfgS1>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits, probs, psum, st, false, w_shared);
-}
+// the fp32 instances of the NCHW feature conv compile here, the bf16 ones in head_fwd_bf16.cu
+template int level_conv_nchw<float>(const float*, const float*, const float*, const float*, const int32_t*, int, int, int,
+                                    int, int, int, float*, bool, float*, float*, double*, int, cudaStream_t);
+extern template int level_conv_nchw<uint16_t>(const uint16_t*, const float*, const float*, const float*, const int32_t*,
+                                              int, int, int, int, int, int, float*, bool, float*, float*, double*, int,
+                                              cudaStream_t);
 
 }  // namespace rhseg
 
@@ -123,56 +106,24 @@ static int level_fwd_impl(const void* feats_v, const float* eff_w, const float* 
   if (ea && !up) return RHSEG_ERR_UNSUPPORTED;
   if (act_mode == RHSEG_ACT_GROUPED && table == nullptr) return RHSEG_ERR_ARG;
   const int Nf = Hf * Wf;
-  if (zero_psum & RHSEG_FEATS_NHWC) {
-    const bool bf16 = (zero_psum & RHSEG_FEATS_BF16) != 0;
-    const size_t esz = bf16 ? 2 : 4;
-    if (((size_t)C * esz) % 16 != 0 || (reinterpret_cast<uintptr_t>(feats_v) & 15u) != 0) return RHSEG_ERR_UNSUPPORTED;
-    if (up && !z_lo) return RHSEG_ERR_ARG;
-    const int rc = bf16 ? level_conv_nhwc(static_cast<const uint16_t*>(feats_v), eff_w, eff_b, prev_probs, table, B, C, Nf, K,
-                                          K_prev, act_mode, up ? z_lo : nullptr, zlo_zeroed, logits, probs, psum, w_shared, st)
-                        : level_conv_nhwc(static_cast<const float*>(feats_v), eff_w, eff_b, prev_probs, table, B, C, Nf, K,
-                                          K_prev, act_mode, up ? z_lo : nullptr, zlo_zeroed, logits, probs, psum, w_shared, st);
-    if (rc != RHSEG_OK || !up) return rc;
-  } else if (zero_psum & RHSEG_FEATS_BF16) {
-    const uint16_t* fb = static_cast<const uint16_t*>(feats_v);
-    if (reinterpret_cast<uintptr_t>(fb) & 1u) return RHSEG_ERR_ARG;
-    if (up && !z_lo) return RHSEG_ERR_ARG;
-    const int rc = level_conv_bf16(fb, eff_w, eff_b, prev_probs, table, B, C, Nf, K, K_prev, act_mode, up ? z_lo : nullptr,
-                                   zlo_zeroed, logits, probs, psum, w_shared, st);
-    if (rc != RHSEG_OK || !up) return rc;
-  } else {
-    const float* feats = static_cast<const float*>(feats_v);
-    if (!up) {
-      RHSEG_DISPATCH_K(K, {
-        if (act_mode == RHSEG_ACT_SIGMOID)
-          return fwd_fullres<KK, RHSEG_ACT_SIGMOID>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
-        if (act_mode == RHSEG_ACT_GROUPED)
-          return fwd_fullres<KK, RHSEG_ACT_GROUPED>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
-        return fwd_fullres<KK, RHSEG_ACT_ZEROS>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits, probs, psum, st, w_shared);
-      });
-    }
-    if (!z_lo) return RHSEG_ERR_ARG;
-    RHSEG_DISPATCH_K(K, {
-      int rc;
-      if (rows_vec4(feats, Nf) && rows_vec4(z_lo, Nf)) {
-        rc = launch_fwd<float, KK, 4, 1, MODE_CONV_ONLY, FwdCfgV4>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
-      } else {
-        int t = 0;
-        if constexpr (KK == 4) t = tune_env("RHSEG_TUNE_FWD_S1");
-        if constexpr (KK == 4) {
-          if (t == 1) rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, PipeCfg<8, 16, 3, 2>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
-          else if (t == 2) rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, PipeCfg<8, 8, 4, 2>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
-          else if (t == 3) rc = launch_fwd<float, KK, 1, 4, MODE_CONV_ONLY, PipeCfg<4, 16, 4, 1>>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, false, w_shared);
-          else rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, FwdCfgS1>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
-        } else {
-          rc = launch_fwd<float, KK, 1, 2, MODE_CONV_ONLY, FwdCfgS1>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
-        }
-      }
-      if (rc != RHSEG_OK) return rc;
-    });
+  const bool nhwc = (zero_psum & RHSEG_FEATS_NHWC) != 0, bf16 = (zero_psum & RHSEG_FEATS_BF16) != 0;
+  if (nhwc) {
+    if (((size_t)C * (bf16 ? 2 : 4)) % 16 != 0 || (reinterpret_cast<uintptr_t>(feats_v) & 15u) != 0) return RHSEG_ERR_UNSUPPORTED;
+  } else if (bf16 && (reinterpret_cast<uintptr_t>(feats_v) & 1u)) {
+    return RHSEG_ERR_ARG;
   }
+  if (up && !z_lo) return RHSEG_ERR_ARG;
+  float* conv_out = up ? z_lo : nullptr;  // the feature conv of an upsampled head writes z_lo
+  auto conv = [&](auto feats) {
+    return nhwc ? level_conv_nhwc(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K, K_prev, act_mode, conv_out, zlo_zeroed,
+                                  logits, probs, psum, w_shared, st)
+                : level_conv_nchw(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K, K_prev, act_mode, conv_out, zlo_zeroed,
+                                  logits, probs, psum, w_shared, st);
+  };
+  int rc = bf16 ? conv(static_cast<const uint16_t*>(feats_v)) : conv(static_cast<const float*>(feats_v));
+  if (rc != RHSEG_OK || !up) return rc;
   bool ne = false;
-  const int rc = fwd_upsampled_dispatch(K, act_arg, z_lo, prev_probs, table, B, Hf, Wf, H, W, K_prev, logits, probs, psum, st, ea, &ne);
+  rc = fwd_upsampled_dispatch(K, act_arg, z_lo, prev_probs, table, B, Hf, Wf, H, W, K_prev, logits, probs, psum, st, ea, &ne);
   if (need_eval) *need_eval = ne;
   return rc;
 }

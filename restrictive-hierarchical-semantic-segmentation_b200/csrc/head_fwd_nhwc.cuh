@@ -3,12 +3,13 @@
 //
 // Same work decomposition as head_fwd_kernel (unit = sample, pixel tile of T pixels, channel stage of CH = 8 channels;
 // the unit space split evenly over one resident wave), same arithmetic: a logit starts at the bias and takes one fmaf
-// per channel in ascending order, so logits and probabilities equal the NCHW kernel's bit for bit.  What differs is the
-// stage: the producer copies a [T pixels x 8 channels] box of the [C, N, B] tensor map (pixel rows of 32 bytes fp32,
-// swizzled, or 16 bytes bf16), and consumer thread tid owns the pixels j*NCONS + tid, reading each pixel's 8 channels
-// with one or two 128-bit shared loads.  Where the NCHW kernel gives a thread 4 consecutive pixels (16-byte rows,
-// XCHG), the finished logits pass through shared memory to that ownership before the epilogue, so that the per-thread
-// probability sums (psum, the FiLM pool of the next level) add the same pixels in the same order.  DESIGN.md 3.8.
+// per channel in ascending order, so logits and probabilities equal the NCHW kernel's bit for bit.  The split, the
+// cursor, the weight staging and the epilogue are head_fwd_kernel.cuh's.  What differs is the stage: the producer
+// copies a [T pixels x 8 channels] box of the [C, N, B] tensor map (pixel rows of 32 bytes fp32, swizzled, or 16 bytes
+// bf16), and consumer thread tid owns the pixels j*NCONS + tid, reading each pixel's 8 channels with one or two 128-bit
+// shared loads.  Where the NCHW kernel gives a thread 4 consecutive pixels (16-byte rows, XCHG), the finished logits
+// pass through shared memory to that ownership before the epilogue, so that the per-thread probability sums (psum, the
+// FiLM pool of the next level) add the same pixels in the same order.  DESIGN.md 3.8.
 #pragma once
 #include <algorithm>
 #include "feats_nhwc.cuh"
@@ -37,8 +38,6 @@ head_fwd_nhwc_kernel(const __grid_constant__ CUtensorMap fmap, const float* __re
   constexpr int STAGE = T * IB;
   constexpr int NS = CFG::NS;
   // epilogue ownership: 4 consecutive pixels (XCHG, as head_fwd_kernel with VEC = 4) or the pixels j*NCONS + tid
-  constexpr int VE = XCHG ? 4 : 1;
-  constexpr int JE = XCHG ? 1 : J;
   static_assert(!XCHG || J == 4, "the exchange regroups 4 pixels per thread");
   static_assert(T % BOX == 0 && (IB == 16 || IB == 32), "stage shape");
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -52,36 +51,9 @@ head_fwd_nhwc_kernel(const __grid_constant__ CUtensorMap fmap, const float* __re
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   long u_begin, u_end;
-  if constexpr (MODE == MODE_CONV_ONLY) {
-    u_begin = units_total * blockIdx.x / gridDim.x;
-    u_end = units_total * (blockIdx.x + 1) / gridDim.x;
-  } else {
-    const long tiles_total = units_total / n_stages;
-    u_begin = (tiles_total * blockIdx.x / gridDim.x) * n_stages;
-    u_end = (tiles_total * (blockIdx.x + 1) / gridDim.x) * n_stages;
-  }
-  if (tid == 0) {
-    for (int i = 0; i < NS; ++i) {
-      mbar_init(smem_u32(&bars[i]), CFG::NPW);
-      mbar_init(smem_u32(&bars[NS + i]), CFG::NCW);
-    }
-    mbar_fence_init();
-  }
-  __syncthreads();
-
-  int stage, tile, b;
-  {
-    const long tile_lin = u_begin / n_stages;
-    stage = (int)(u_begin - tile_lin * n_stages);
-    b = (int)(tile_lin / n_tiles);
-    tile = (int)(tile_lin - (long)b * n_tiles);
-  }
-  auto advance = [&]() {
-    if (++stage == n_stages) {
-      stage = 0;
-      if (++tile == n_tiles) { tile = 0; ++b; }
-    }
-  };
+  fwd_units<MODE>(units_total, n_stages, u_begin, u_end);
+  ring_bars_init<NS>(bars, CFG::NPW, CFG::NCW);
+  FwdCursor at(u_begin, n_tiles, n_stages);
 
   if (warp >= CFG::NCW) {
     // ------------------------------ producers ------------------------------
@@ -91,24 +63,23 @@ head_fwd_nhwc_kernel(const __grid_constant__ CUtensorMap fmap, const float* __re
       uint32_t phase = 1;
       for (long u = u_begin; u < u_end; ++u) {
         mbar_wait(smem_u32(&bars[NS + slot]), phase);
-        const int p0 = tile * T;
+        const int p0 = at.tile * T;
         uint32_t bytes = 0;
         for (int i = pw; i < NBOX; i += CFG::NPW) {
           if (p0 + i * BOX >= N) break;  // boxes wholly past the plane: nothing of them is read
-          tma_load_3d(smem_u32(ring + (size_t)slot * STAGE + i * BOX * IB), &fmap, stage * CH, p0 + i * BOX, b,
+          tma_load_3d(smem_u32(ring + (size_t)slot * STAGE + i * BOX * IB), &fmap, at.stage * CH, p0 + i * BOX, at.b,
                       smem_u32(&bars[slot]));
           bytes += BOX * IB;
         }
         mbar_arrive_expect_tx(smem_u32(&bars[slot]), bytes);
         if (++slot == NS) { slot = 0; phase ^= 1u; }
-        advance();
+        at.advance();
       }
     }
     return;
   }
 
   // -------------------------------- consumers --------------------------------
-  auto csync = [] { consumer_sync(NCONS); };
   LevelInfo li;
   if constexpr (MODE != MODE_CONV_ONLY) li = load_level_info<K>(MODE == RHSEG_ACT_GROUPED ? table : nullptr);
   int cur_b = -1;
@@ -124,37 +95,12 @@ head_fwd_nhwc_kernel(const __grid_constant__ CUtensorMap fmap, const float* __re
   int slot = 0;
   uint32_t phase = 0;
   for (long u = u_begin; u < u_end; ++u) {
-    const int p0 = tile * T;
+    const int p0 = at.tile * T;
     const int t_act = min(T, N - p0);
-    if (stage == 0 || u == u_begin) {
-      if (b != cur_b) {
-        if constexpr (MODE != MODE_CONV_ONLY) {
-          if (cur_b >= 0) {
-            block_psum<K, CFG::NCW>(ps, psum + (size_t)cur_b * K, red, csync);
-#pragma unroll
-            for (int k = 0; k < K; ++k) ps[k] = 0.f;
-          }
-        }
-        csync();
-        const float* wsrc = w_shared ? eff_w : eff_w + (size_t)b * K * C;
-        for (int k = 0; k < K; ++k)
-          for (int c = tid; c < C; c += NCONS) w_t[c * KP + k] = wsrc[(size_t)k * C + c];
-        if constexpr (KP > K)
-          for (int k = K; k < KP; ++k)
-            for (int c = tid; c < C; c += NCONS) w_t[c * KP + k] = 0.f;
-#pragma unroll
-        for (int k = 0; k < K; ++k) bias[k] = eff_b[(w_shared ? 0 : b * K) + k];
-        cur_b = b;
-        csync();
-      }
-      from_stage0 = stage == 0;
-#pragma unroll
-      for (int k = 0; k < K; ++k)
-#pragma unroll
-        for (int j = 0; j < J; ++j) acc[k][j] = from_stage0 ? bias[k] : 0.f;
-    }
+    if (at.stage == 0 || u == u_begin)  // first unit of this tile in this CTA (uniform)
+      from_stage0 = fwd_tile_begin<K, J, MODE, CFG>(at, tid, cur_b, eff_w, eff_b, C, w_shared, w_t, red, psum, bias, ps, acc);
 
-    const int c0 = stage * CH;
+    const int c0 = at.stage * CH;
     const int ccnt = min(CH, C - c0);
     const float* wrow = w_t + (size_t)c0 * KP;
     mbar_wait(smem_u32(&bars[slot]), phase);
@@ -176,19 +122,7 @@ head_fwd_nhwc_kernel(const __grid_constant__ CUtensorMap fmap, const float* __re
 
     auto channel = [&](int cc) {
       float w[KP];
-      if constexpr (KP == 4) {
-        const float4 t = *reinterpret_cast<const float4*>(wrow + cc * KP);
-        w[0] = t.x; w[1] = t.y; w[2] = t.z; w[3] = t.w;
-      } else if constexpr (KP == 8) {
-        const float4 t0 = *reinterpret_cast<const float4*>(wrow + cc * KP);
-        const float4 t1 = *reinterpret_cast<const float4*>(wrow + cc * KP + 4);
-        w[0] = t0.x; w[1] = t0.y; w[2] = t0.z; w[3] = t0.w; w[4] = t1.x; w[5] = t1.y; w[6] = t1.z; w[7] = t1.w;
-      } else if constexpr (KP == 2) {
-        const float2 t = *reinterpret_cast<const float2*>(wrow + cc * KP);
-        w[0] = t.x; w[1] = t.y;
-      } else {
-        w[0] = wrow[cc];
-      }
+      ld_wvec<KP>(wrow + cc * KP, w);
 #pragma unroll
       for (int j = 0; j < J; ++j)
 #pragma unroll
@@ -203,96 +137,27 @@ head_fwd_nhwc_kernel(const __grid_constant__ CUtensorMap fmap, const float* __re
         if (cc < ccnt) channel(cc);
     }
 
-    if (stage == n_stages - 1 || u == u_end - 1) {  // last unit of this tile in this CTA: epilogue
-      float e[K][JE * VE];
-      if constexpr (XCHG) {
+    if (at.stage == n_stages - 1 || u == u_end - 1) {  // last unit of this tile in this CTA: epilogue
+      if constexpr (XCHG) {  // regroup: 4 consecutive pixels per thread
+        float e[K][4];
 #pragma unroll
         for (int k = 0; k < K; ++k) {
-          csync();
+          consumer_sync(NCONS);
 #pragma unroll
           for (int j = 0; j < J; ++j) xbuf[j * NCONS + tid] = acc[k][j];
-          csync();
+          consumer_sync(NCONS);
           const float4 t = *reinterpret_cast<const float4*>(xbuf + 4 * tid);
           e[k][0] = t.x; e[k][1] = t.y; e[k][2] = t.z; e[k][3] = t.w;
         }
+        fwd_epilogue<K, 1, 4, MODE, NCONS>(e, at, tid, from_stage0, li, N, p0, t_act, K_prev, prev_probs, logits, probs, ps);
       } else {
-#pragma unroll
-        for (int k = 0; k < K; ++k)
-#pragma unroll
-          for (int j = 0; j < J; ++j) e[k][j] = acc[k][j];
-      }
-      constexpr int PE = JE * VE;
-      int lp[JE];
-      bool ok[JE];
-#pragma unroll
-      for (int j = 0; j < JE; ++j) {
-        lp[j] = (j * NCONS + tid) * VE;
-        ok[j] = lp[j] < t_act;
-      }
-      float* zb = logits + (size_t)b * K * N + p0;
-      if constexpr (MODE == MODE_CONV_ONLY) {
-        const bool complete = from_stage0 && stage == n_stages - 1;
-#pragma unroll
-        for (int j = 0; j < JE; ++j) {
-          if (!ok[j]) continue;
-#pragma unroll
-          for (int k = 0; k < K; ++k) {
-            float* dst = zb + (size_t)k * N + lp[j];
-            if (complete) *dst = e[k][j];
-            else atomicAdd(dst, e[k][j]);
-          }
-        }
-      } else {
-        float pp[K][PE];
-        if constexpr (MODE == RHSEG_ACT_GROUPED) {
-          const float* pb = prev_probs + (size_t)b * K_prev * N + p0;
-#pragma unroll
-          for (int k = 0; k < K; ++k) {
-            if ((li.start_mask >> k) & 1) {
-#pragma unroll
-              for (int j = 0; j < JE; ++j) {
-                Vec<VE> t;
-                if (ok[j]) t = ld_cached<VE>(pb + (size_t)li.parent[k] * N + lp[j]);
-                else {
-#pragma unroll
-                  for (int v = 0; v < VE; ++v) t.v[v] = 0.f;
-                }
-#pragma unroll
-                for (int v = 0; v < VE; ++v) pp[k][j * VE + v] = t.v[v];
-              }
-            } else {
-#pragma unroll
-              for (int p = 0; p < PE; ++p) pp[k][p] = pp[k > 0 ? k - 1 : 0][p];
-            }
-          }
-        }
-        float prob[K][PE];
-        activate<K, PE, MODE>(e, pp, li.start_mask, prob);
-        float* pb_out = probs + (size_t)b * K * N + p0;
-#pragma unroll
-        for (int k = 0; k < K; ++k) {
-#pragma unroll
-          for (int j = 0; j < JE; ++j) {
-            if (!ok[j]) continue;
-            Vec<VE> zo, po;
-#pragma unroll
-            for (int v = 0; v < VE; ++v) {
-              zo.v[v] = e[k][j * VE + v];
-              po.v[v] = prob[k][j * VE + v];
-              ps[k] += po.v[v];
-            }
-            *reinterpret_cast<Vec<VE>*>(zb + (size_t)k * N + lp[j]) = zo;
-            *reinterpret_cast<Vec<VE>*>(pb_out + (size_t)k * N + lp[j]) = po;
-          }
-        }
+        fwd_epilogue<K, J, 1, MODE, NCONS>(acc, at, tid, from_stage0, li, N, p0, t_act, K_prev, prev_probs, logits, probs, ps);
       }
     }
     if (++slot == NS) { slot = 0; phase ^= 1u; }
-    advance();
+    at.advance();
   }
-  if constexpr (MODE != MODE_CONV_ONLY) {
-    if (cur_b >= 0) block_psum<K, CFG::NCW>(ps, psum + (size_t)cur_b * K, red, csync);
-  }
+  fwd_flush_psum<K, MODE, CFG>(cur_b, ps, red, psum);
 }
 
 template <typename FT, int K, int J, int MODE, typename CFG, bool XCHG>
@@ -304,23 +169,15 @@ static int launch_fwd_nhwc(const FT* feats, const float* eff_w, const float* eff
   constexpr int IB = NHWC_CH * (int)sizeof(FT);
   const size_t smem = 1024 + 128 + (size_t)CFG::NS * T * IB + ((size_t)C * KP + CFG::NCW * K + (XCHG ? T : 0)) * sizeof(float);
   auto kern = head_fwd_nhwc_kernel<FT, K, J, MODE, CFG, XCHG>;
-  int per_sm = 0;
-  RHSEG_CUDA(cached_launch_prep(reinterpret_cast<const void*>(kern), CFG::THREADS, smem, smem, &per_sm));
-  if (per_sm < 1) return RHSEG_ERR_UNSUPPORTED;
   CUtensorMap map;
-  const int rc = encode_feats_map<FT>(&map, feats, B, C, N, NHWC_CH, T < 256 ? T : 256);
+  int rc = encode_feats_map<FT>(&map, feats, B, C, N, NHWC_CH, T < 256 ? T : 256);
   if (rc != RHSEG_OK) return rc;
-  const int n_tiles = (N + T - 1) / T;
-  const int n_stages = (C + NHWC_CH - 1) / NHWC_CH;
-  const long tiles_total = (long)B * n_tiles;
-  const long units_total = tiles_total * n_stages;
-  long grid = (long)device_sm_count() * per_sm;
-  grid = std::min<long>(grid, tiles_total);
-  if (grid < 1) grid = 1;
-  if (MODE == MODE_CONV_ONLY && grid > 1 && !out_prezeroed)
-    RHSEG_CUDA(cudaMemsetAsync(logits, 0, sizeof(float) * (size_t)B * K * N, st));
-  launch_pdl(kern, dim3((unsigned)grid), dim3(CFG::THREADS), smem, st, map, eff_w, eff_b, prev_probs, table, C, N, K_prev,
-             n_tiles, n_stages, units_total, w_shared, logits, probs, psum);
+  FwdGrid g;
+  rc = fwd_grid<MODE>(reinterpret_cast<const void*>(kern), CFG::THREADS, smem, B, C, N, K, T, NHWC_CH, logits, out_prezeroed,
+                      st, g);
+  if (rc != RHSEG_OK) return rc;
+  launch_pdl(kern, dim3((unsigned)g.ctas), dim3(CFG::THREADS), smem, st, map, eff_w, eff_b, prev_probs, table, C, N, K_prev,
+             g.n_tiles, g.n_stages, g.units_total, w_shared, logits, probs, psum);
   RHSEG_LAUNCH_CHECK();
   return RHSEG_OK;
 }
@@ -328,45 +185,48 @@ static int launch_fwd_nhwc(const FT* feats, const float* eff_w, const float* eff
 // Ring shapes.  Each mirrors the NCHW kernel's for the same plane (FwdCfgV4 / FwdCfgS1: consumers, producers, tile
 // size, about the same shared memory), so that both kernels get the same resident wave and split the pixel tiles
 // between CTAs alike: the psum of a level then adds the same pixels per thread and per CTA.
-using FwdNhwcCfgV4 = FwdCfgV4;               // T = 1024 px: 3 stages of 32 KB (fp32) / 16 KB (bf16)
+using FwdNhwcCfgV4 = FwdCfgV4;                   // T = 1024 px: 3 stages of 32 KB (fp32) / 16 KB (bf16)
 using FwdNhwcCfgS1 = PipeCfg<4, NHWC_CH, 8, 2>;  // T = 128*J px: 8 stages of 8 KB (fp32, J = 2) / 8 KB (bf16, J = 4)
-template <typename FT> constexpr int fwd_nhwc_s1_j() { return sizeof(FT) == 4 ? 2 : 4; }
 
-template <typename FT, int K, int MODE>
-static int fwd_fullres_nhwc(bool v4, const FT* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                            const int32_t* table, int B, int C, int N, int K_prev, float* logits, float* probs, double* psum,
-                            cudaStream_t st, int w_shared) {
-  if (v4)
-    return launch_fwd_nhwc<FT, K, 4, MODE, FwdNhwcCfgV4, true>(feats, eff_w, eff_b, prev_probs, table, B, C, N, K_prev, logits,
-                                                               probs, psum, st, false, w_shared);
-  return launch_fwd_nhwc<FT, K, fwd_nhwc_s1_j<FT>(), MODE, FwdNhwcCfgS1, false>(feats, eff_w, eff_b, prev_probs, table, B, C,
-                                                                                N, K_prev, logits, probs, psum, st, false,
-                                                                                w_shared);
-}
-
-// Level conv for NHWC features: z_lo == nullptr, conv + activation at feature resolution; otherwise the low-res conv of
-// an upsampled head into z_lo [B,K,Nf].  The tile shape follows what the NCHW path picks for the same plane.
+// z_lo == nullptr: conv + activation at feature resolution; otherwise the low-res conv of an upsampled head into z_lo
+// [B,K,Nf].  The tile shape follows what the NCHW path picks for the same plane.
 template <typename FT>
-int level_conv_nhwc_impl(const FT* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                         const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
-                         bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st) {
+int level_conv_nhwc(const FT* feats, const float* eff_w, const float* eff_b, const float* prev_probs, const int32_t* table,
+                    int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo, bool zlo_zeroed, float* logits,
+                    float* probs, double* psum, int w_shared, cudaStream_t st) {
+  constexpr int J1 = s1_j<FT>();
   if (z_lo == nullptr) {
     const bool v4 = Nf % FeatElem<FT>::G == 0 && rows_vec4(logits, Nf) && rows_vec4(probs, Nf) &&
                     (!prev_probs || rows_vec4(prev_probs, Nf));
     RHSEG_DISPATCH_K(K, {
+      if (v4) {
+        if (act_mode == RHSEG_ACT_SIGMOID)
+          return launch_fwd_nhwc<FT, KK, 4, RHSEG_ACT_SIGMOID, FwdNhwcCfgV4, true>(feats, eff_w, eff_b, prev_probs, table, B, C,
+                                                                                  Nf, K_prev, logits, probs, psum, st, false,
+                                                                                  w_shared);
+        if (act_mode == RHSEG_ACT_GROUPED)
+          return launch_fwd_nhwc<FT, KK, 4, RHSEG_ACT_GROUPED, FwdNhwcCfgV4, true>(feats, eff_w, eff_b, prev_probs, table, B, C,
+                                                                                  Nf, K_prev, logits, probs, psum, st, false,
+                                                                                  w_shared);
+        return launch_fwd_nhwc<FT, KK, 4, RHSEG_ACT_ZEROS, FwdNhwcCfgV4, true>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf,
+                                                                              K_prev, logits, probs, psum, st, false, w_shared);
+      }
       if (act_mode == RHSEG_ACT_SIGMOID)
-        return fwd_fullres_nhwc<FT, KK, RHSEG_ACT_SIGMOID>(v4, feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits,
-                                                           probs, psum, st, w_shared);
+        return launch_fwd_nhwc<FT, KK, J1, RHSEG_ACT_SIGMOID, FwdNhwcCfgS1, false>(feats, eff_w, eff_b, prev_probs, table, B, C,
+                                                                                  Nf, K_prev, logits, probs, psum, st, false,
+                                                                                  w_shared);
       if (act_mode == RHSEG_ACT_GROUPED)
-        return fwd_fullres_nhwc<FT, KK, RHSEG_ACT_GROUPED>(v4, feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits,
-                                                           probs, psum, st, w_shared);
-      return fwd_fullres_nhwc<FT, KK, RHSEG_ACT_ZEROS>(v4, feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K_prev, logits,
-                                                       probs, psum, st, w_shared);
+        return launch_fwd_nhwc<FT, KK, J1, RHSEG_ACT_GROUPED, FwdNhwcCfgS1, false>(feats, eff_w, eff_b, prev_probs, table, B, C,
+                                                                                  Nf, K_prev, logits, probs, psum, st, false,
+                                                                                  w_shared);
+      return launch_fwd_nhwc<FT, KK, J1, RHSEG_ACT_ZEROS, FwdNhwcCfgS1, false>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf,
+                                                                              K_prev, logits, probs, psum, st, false, w_shared);
     });
   }
   RHSEG_DISPATCH_K(K, {
-    return launch_fwd_nhwc<FT, KK, fwd_nhwc_s1_j<FT>(), MODE_CONV_ONLY, FwdNhwcCfgS1, false>(
-        feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf, K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed, w_shared);
+    return launch_fwd_nhwc<FT, KK, J1, MODE_CONV_ONLY, FwdNhwcCfgS1, false>(feats, eff_w, eff_b, nullptr, nullptr, B, C, Nf,
+                                                                           K_prev, z_lo, nullptr, nullptr, st, zlo_zeroed,
+                                                                           w_shared);
   });
   return RHSEG_OK;
 }

@@ -4,11 +4,7 @@
 
 namespace rhseg {
 
-int level_conv_nhwc(const uint16_t* feats, const float* eff_w, const float* eff_b, const float* prev_probs,
-                    const int32_t* table, int B, int C, int Nf, int K, int K_prev, int act_mode, float* z_lo,
-                    bool zlo_zeroed, float* logits, float* probs, double* psum, int w_shared, cudaStream_t st) {
-  return level_conv_nhwc_impl<uint16_t>(feats, eff_w, eff_b, prev_probs, table, B, C, Nf, K, K_prev, act_mode, z_lo,
-                                        zlo_zeroed, logits, probs, psum, w_shared, st);
-}
+template int level_conv_nhwc<uint16_t>(const uint16_t*, const float*, const float*, const float*, const int32_t*, int, int,
+                                       int, int, int, int, float*, bool, float*, float*, double*, int, cudaStream_t);
 
 }  // namespace rhseg

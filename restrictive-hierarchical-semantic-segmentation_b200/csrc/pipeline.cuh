@@ -62,6 +62,19 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   while (!mbar_try_wait(bar, parity)) {
   }
 }
+// Barriers of an NS-stage ring: full[i] = bars[i] completes on `producers` arrivals (plus the copied bytes), empty[i] =
+// bars[NS + i] on `consumer_warps` arrivals.  Called by the whole CTA.
+template <int NS>
+__device__ __forceinline__ void ring_bars_init(uint64_t* bars, uint32_t producers, uint32_t consumer_warps) {
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < NS; ++i) {
+      mbar_init(smem_u32(&bars[i]), producers);
+      mbar_init(smem_u32(&bars[NS + i]), consumer_warps);
+    }
+    mbar_fence_init();
+  }
+  __syncthreads();
+}
 // L2 policy for read-once streams: do not let 300-400 MB of features evict the small tensors
 // (logits, targets, probabilities) that the following kernels re-read.
 __device__ __forceinline__ uint64_t l2_evict_first_policy() {
