@@ -33,6 +33,7 @@ extern "C" {
 #define RHSEG_KERNEL_MAX_K 8     /* channels per level the fused kernels are built for    */
 #define RHSEG_TABLE_INTS (4 + 5 * RHSEG_MAX_K)
 #define RHSEG_EVAL_PREZEROED 1   /* rhseg_level_eval / rhseg_head_level_fwd_eval flag       */
+#define RHSEG_EVAL_COMPOSED 0x40 /* rhseg_head_level_fwd_eval flag: validation evaluation     */
 /* Feature element type flag of rhseg_head_level_fwd (zero_psum), rhseg_head_level_fwd_eval (flags),
  * rhseg_head_conv_bwd (zero_sums) and rhseg_head_conv_bwd_params (flags): set, feats (and dfeats) are
  * bf16 [B,C,Hf,Wf], 2-byte aligned (autocast-trained donors); clear, fp32.  Each bf16 value is converted
@@ -146,6 +147,11 @@ int rhseg_head_level_fwd_eval(const void* feats, const float* eff_w, const float
                               const float* parent_targets, long pt_bstride, long pt_cstride,
                               const unsigned char* prev_idx, void* out_words, unsigned char* idx_out,
                               int flags, void* stream);
+/* flags & RHSEG_EVAL_COMPOSED: the pass evaluates what rhseg_level_eval_composed evaluates (the reference's test(),
+ * train.py:324-339) instead of the training evaluation: the confusion matrix of ProcessClasses over the composed
+ * probabilities against the raw targets, and on grouped levels the consistency sums of the probabilities against
+ * prev_probs, the parent probabilities the activation reads anyway.  parent_targets, prev_idx and idx_out are
+ * ignored.  Shapes the band kernel does not take run rhseg_level_eval_composed after the forward.               */
 
 /* ---------------------------------------------------------------------------------------
  * (2') head, backward (what autograd does for the reference; closed forms in DESIGN.md).
@@ -335,6 +341,26 @@ int rhseg_level_eval(const float* logits, const float* targets, long t_bstride, 
                      const float* parent_targets, long pt_bstride, long pt_cstride,
                      const unsigned char* prev_idx, const int32_t* table, int B, int K, int n_pix,
                      int child, void* out_words, unsigned char* idx_out, int flags, void* stream);
+
+/* Fused per-level VALIDATION evaluation: what the reference's test() computes for one level
+ * (train.py:324-339), which differs from the training evaluation above:
+ *   - confusion: ProcessClasses (first maximum, NaN wins, the prepended "nothing positive" channel on
+ *     child levels) over the COMPOSED probabilities `probs` against the RAW ternary targets; child levels
+ *     drop target class 0, level 0 counts every pixel;
+ *   - consistency: per group g of `table`, sum over pixels of |sum_{c in g} probs_c - prev_probs[parent(g)]|
+ *     on the real probabilities, without an ignore mask (rhseg_consistency_sums' sums), so that
+ *     rhseg_step_finalize turns them into the test() term unchanged;
+ *   - statistics: rhseg_level_eval's CE/Dice statistics of `logits`.
+ * No prediction index map is read or written.
+ *   logits, probs [B,K,n_pix] contiguous; prev_probs [B,K_prev,n_pix] contiguous (NULL: no consistency
+ *   sums; ignored at level 0); targets strided as everywhere.  out_words, flags and child as in
+ *   rhseg_level_eval (child: 0 / 1, optionally | RHSEG_GROUP_HINT(gsz)).  A bulk-copy pipeline serves
+ *   16-byte aligned planes with n_pix % 4 == 0 and target strides that are multiples of 4; any other
+ *   shape takes a one-pixel-per-thread kernel with the same results.                            */
+int rhseg_level_eval_composed(const float* logits, const float* probs, const float* prev_probs,
+                              const float* targets, long t_bstride, long t_cstride, const int32_t* table,
+                              int B, int K, int K_prev, int n_pix, int child, void* out_words, int flags,
+                              void* stream);
 
 /* Flat -> hierarchy stitching (predictEval.py:85-185, :381-388): `leaves` [B,n_leaves,n_pix] are the
  * flat model's leaf channels (predictions or targets); `out` [B,n_out,n_pix] gets one channel per tree

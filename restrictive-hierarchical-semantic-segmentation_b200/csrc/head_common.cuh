@@ -19,6 +19,7 @@ struct EvalArgs {
   double* cons;
   unsigned long long* conf;
   unsigned char* idx_out;
+  int composed;  // RHSEG_EVAL_COMPOSED: the validation evaluation (parent_targets / prev_idx / idx_out unused)
 };
 
 // hi-res pass of an upsampled head (head_up.cu): K / activation mode dispatch included.  act_arg = activation mode |

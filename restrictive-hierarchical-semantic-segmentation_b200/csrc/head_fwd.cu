@@ -151,13 +151,19 @@ extern "C" int rhseg_head_level_fwd_eval(const void* feats, const float* eff_w, 
   if (!(flags & RHSEG_EVAL_PREZEROED)) RHSEG_CUDA(cudaMemsetAsync(out_words, 0, words * 8, (cudaStream_t)stream));
   double* stats = reinterpret_cast<double*>(out_words);
   double* cons = stats + (size_t)B * K * RHSEG_NSTAT;
+  const bool composed = (flags & RHSEG_EVAL_COMPOSED) != 0;
+  if (composed) parent_targets = nullptr, prev_idx = nullptr, idx_out = nullptr;
   EvalArgs ea{targets, t_bstride, t_cstride, parent_targets, pt_bstride, pt_cstride, prev_idx, child, stats, cons,
-              reinterpret_cast<unsigned long long*>(cons + RHSEG_MAX_K), idx_out};
+              reinterpret_cast<unsigned long long*>(cons + RHSEG_MAX_K), idx_out, composed ? 1 : 0};
   bool need_eval = false;
   const int rc = level_fwd_impl(feats, eff_w, eff_b, prev_probs, table, B, C, Hf, Wf, H, W, K, K_prev, act_mode, z_lo, logits,
                                 probs, psum, (flags & (2 | 4 | RHSEG_FEATS_BF16 | RHSEG_FEATS_NHWC)), stream, &ea, &need_eval);
   if (rc != RHSEG_OK || !need_eval) return rc;
   // shapes the band kernel does not take: the evaluation runs as its own kernel on the finished logits
+  if (composed)
+    return rhseg_level_eval_composed(logits, probs, child ? prev_probs : nullptr, targets, t_bstride, t_cstride, table, B, K,
+                                     K_prev, H * W, child | RHSEG_GROUP_HINT(RHSEG_GROUP_HINT_OF(act_mode)), out_words,
+                                     RHSEG_EVAL_PREZEROED, stream);
   return rhseg_level_eval(logits, targets, t_bstride, t_cstride, parent_targets, pt_bstride, pt_cstride, prev_idx, table, B, K,
                           H * W, child | RHSEG_GROUP_HINT(RHSEG_GROUP_HINT_OF(act_mode)), out_words, idx_out,
                           RHSEG_EVAL_PREZEROED, stream);

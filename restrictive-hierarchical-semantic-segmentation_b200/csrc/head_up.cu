@@ -3,6 +3,7 @@
 // Reference semantics: Models/models.py:766/:776 (upsample), :767/:779-796 (activation, composition).
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 #include "common.cuh"
 #include "hires.cuh"
 #include "head_common.cuh"
@@ -113,9 +114,12 @@ upsample_band_kernel(const float* __restrict__ z_lo, const float* __restrict__ p
                      int band, int lok, int ns, int a0, float* __restrict__ logits, float* __restrict__ probs,
                      double* __restrict__ psum, EvalArgs ea) {
   constexpr bool EVAL = EVALK != 0, GROUPED = MODE == RHSEG_ACT_GROUPED;
-  constexpr int CT = !GROUPED ? 0 : (EVALK == 2 ? 2 : 1);
-  constexpr bool CONS = EVAL && CT == 2;
-  using Acc = EvalAcc<K, CT, GSZ>;
+  // EVALK 3: the validation evaluation (ValAcc) on the composed probabilities; its consistency term reads the parent
+  // probabilities the activation already streams, so it needs no input beyond the targets
+  constexpr bool COMPOSED = EVALK == 3;
+  constexpr int CT = !GROUPED ? 0 : (EVALK == 2 || COMPOSED ? 2 : 1);
+  constexpr bool CONS = EVAL && CT == 2 && !COMPOSED;
+  using Acc = std::conditional_t<COMPOSED, ValAcc<K, CT, GSZ>, EvalAcc<K, CT, GSZ>>;
   constexpr int NG = Groups<K, GSZ>::NG;
   constexpr int MAXCW = VEC == 4 ? 6 : 12;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -336,7 +340,14 @@ upsample_band_kernel(const float* __restrict__ z_lo, const float* __restrict__ p
 #pragma unroll
         for (int k = 0; k < K; ++k) prob[k][v] = group_value<K, GSZ>(pg, gr, k) * q[k];
       }
-      if constexpr (EVAL) {
+      if constexpr (COMPOSED) {
+        float tt[K], P[K], pp[NG];
+#pragma unroll
+        for (int k = 0; k < K; ++k) { tt[k] = t[k][v]; P[k] = prob[k][v]; }
+#pragma unroll
+        for (int g = 0; g < NG; ++g) pp[g] = GROUPED ? ppg[g][v] : 0.f;
+        ev.pixel(zz, p, mx + log_fast(sum), tt, P, pp, ok, gr);  // lanes past the row end hold the row start: finite
+      } else if constexpr (EVAL) {
         float tt[K], pt[NG];
 #pragma unroll
         for (int k = 0; k < K; ++k) tt[k] = t[k][v];
@@ -355,7 +366,7 @@ upsample_band_kernel(const float* __restrict__ z_lo, const float* __restrict__ p
         *reinterpret_cast<Vec<VEC>*>(logits + ((size_t)b * K + k) * N + px) = zo;
         *reinterpret_cast<Vec<VEC>*>(probs + ((size_t)b * K + k) * N + px) = po;
       }
-      if constexpr (EVAL) {
+      if constexpr (EVAL && !COMPOSED) {
         if (ea.idx_out) {
           unsigned char* dst = ea.idx_out + (size_t)b * N + px;
           if constexpr (VEC == 4) *reinterpret_cast<unsigned*>(dst) = my_idx;
@@ -397,12 +408,24 @@ upsample_band_kernel(const float* __restrict__ z_lo, const float* __restrict__ p
         if (lane == 0 && v) atomicAdd(&cred[g], v);
       }
     }
+    if constexpr (COMPOSED) {
+#pragma unroll
+      for (int g = 0; g < Acc::NCS; ++g) {
+        const float v = warp_sum(ev.cs[g]);
+        if (lane == 0) red[warp * NACC + K * RHSEG_NSTAT + g] = v;
+      }
+    }
     ev.cc.flush(hist);
     csync();
     for (int i = tid; i < NACC; i += ncons) {  // narrow images run a single consumer warp
       double acc = 0.0;
       for (int w = 0; w < ncw; ++w) acc += (double)red[w * NACC + i];
-      atomicAdd(&ea.stats[(size_t)b * K * RHSEG_NSTAT + i], acc);
+      if constexpr (COMPOSED) {
+        if (i < K * RHSEG_NSTAT) atomicAdd(&ea.stats[(size_t)b * K * RHSEG_NSTAT + i], acc);
+        else if (acc != 0.0) atomicAdd(&ea.cons[i - K * RHSEG_NSTAT], acc);
+      } else {
+        atomicAdd(&ea.stats[(size_t)b * K * RHSEG_NSTAT + i], acc);
+      }
     }
     if constexpr (CONS) {
       if (tid < NG && cred[tid]) atomicAdd(&ea.cons[tid], (double)cred[tid]);
@@ -478,7 +501,7 @@ static int fwd_upsampled(const float* z_lo, const float* prev_probs, const int32
     if (band_ok) {
       const EvalArgs none{};
       const EvalArgs& e = ea ? *ea : none;
-      const int evalk = !ea ? 0 : ((MODE == RHSEG_ACT_GROUPED && ea->prev_idx && ea->parent_targets) ? 2 : 1);
+      const int evalk = !ea ? 0 : ea->composed ? 3 : ((MODE == RHSEG_ACT_GROUPED && ea->prev_idx && ea->parent_targets) ? 2 : 1);
       // pixels per thread: 4 when three low-res columns cover them (sx <= 1/3), else 2
       const bool v4 = 3.0f * sx <= 0.999f && tune_vec != 2;
       const bool v2 = 1.0f * sx <= 0.999f;
@@ -493,18 +516,18 @@ static int fwd_upsampled(const float* z_lo, const float* prev_probs, const int32
         }                                                     \
       } while (0)
       if constexpr (MODE == RHSEG_ACT_SIGMOID) {
-        if (evalk == 0) RHSEG_BAND_V(0, K); else RHSEG_BAND_V(1, K);
+        if (evalk == 0) RHSEG_BAND_V(0, K); else if (evalk == 3) RHSEG_BAND_V(3, K); else RHSEG_BAND_V(1, K);
       } else {
         const bool single = hint == K;
         bool uniform2 = false;
         if constexpr (K == 4) uniform2 = hint == 2;  // two parents with two children each (extended tree, level 2)
         if (single) {
-          if (evalk == 0) RHSEG_BAND_V(0, K); else if (evalk == 1) RHSEG_BAND_V(1, K); else RHSEG_BAND_V(2, K);
+          if (evalk == 0) RHSEG_BAND_V(0, K); else if (evalk == 1) RHSEG_BAND_V(1, K); else if (evalk == 3) RHSEG_BAND_V(3, K); else RHSEG_BAND_V(2, K);
         } else if (uniform2) {
-          if constexpr (K == 4) { if (evalk == 0) RHSEG_BAND_V(0, 2); else if (evalk == 1) RHSEG_BAND_V(1, 2); else RHSEG_BAND_V(2, 2); }
+          if constexpr (K == 4) { if (evalk == 0) RHSEG_BAND_V(0, 2); else if (evalk == 1) RHSEG_BAND_V(1, 2); else if (evalk == 3) RHSEG_BAND_V(3, 2); else RHSEG_BAND_V(2, 2); }
         } else {
           if (evalk == 0) RHSEG_BAND_V(0, 0);
-          else if constexpr (K <= 6) { if (evalk == 1) RHSEG_BAND_V(1, 0); else RHSEG_BAND_V(2, 0); }
+          else if constexpr (K <= 6) { if (evalk == 1) RHSEG_BAND_V(1, 0); else if (evalk == 3) RHSEG_BAND_V(3, 0); else RHSEG_BAND_V(2, 0); }
           // K > 6 with a table-driven group layout and the fused evaluation would spill: generic kernel + rhseg_level_eval
         }
       }

@@ -302,6 +302,109 @@ struct EvalAcc {
 };
 
 // ------------------------------------------------------------------------------------------------
+// Per-pixel VALIDATION evaluation (the reference's test(), train.py:324-339, for one level): the CE/Dice statistics
+// of EvalAcc, the confusion cell of ProcessClasses over the composed probabilities P against the RAW ternary targets
+// (no one-hot, no -1 -> 0), and per group g the consistency |sum_{c in g} P_c - P_prev[parent(g)]| of the real
+// probabilities, without an ignore mask.  Level kinds (CT) as in EvalAcc.  Kept apart from EvalAcc so that the
+// training instances keep their code.
+// ------------------------------------------------------------------------------------------------
+template <int K, int CT, int GSZ>
+struct ValAcc {
+  static constexpr int NS = RHSEG_NSTAT;
+  static constexpr bool CHILD = CT >= 1, CONS = CT == 2;
+  static constexpr int NC = CHILD ? K + 1 : K;
+  static constexpr int NCELL = NC * NC;
+  static constexpr int NG = Groups<K, GSZ>::NG;
+  static constexpr int NCS = CONS ? NG : 0;
+  static constexpr int NACC = K * NS + NCS;  // statistics, then one consistency partial per group
+  float a[K][NS];
+  float cs[CONS ? NG : 1];
+  CellCounter<NCELL> cc;
+
+  __device__ __forceinline__ void init() {
+    cc.init();
+#pragma unroll
+    for (int g = 0; g < (CONS ? NG : 1); ++g) cs[g] = 0.f;
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+#pragma unroll
+      for (int j = 0; j < NS; ++j) a[k][j] = 0.f;
+  }
+
+  // z, p, mlse, t, ok as in EvalAcc::pixel (t: the raw ternary targets); P: the level's composed probabilities,
+  // pp: the previous level's probability of each group's parent (CT 2).  Out-of-range pixels (ok == false) must
+  // arrive with finite P.  All lanes of the warp call it (ballots).
+  __device__ __forceinline__ void pixel(const float (&z)[K], const float (&p)[K], float mlse, const float (&t)[K],
+                                        const float (&P)[K], const float (&pp)[NG], bool ok, const Groups<K, GSZ>& gr) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const bool m = ok && t[k] != -1.0f;
+      const float mf = m ? 1.0f : 0.0f;
+      const float et = m ? t[k] : 0.0f;
+      const float lp = z[k] - mlse;
+      a[k][0] = fmaf(et, lp, a[k][0]);
+      a[k][1] += mf;
+      a[k][2] = fmaf(p[k], et, a[k][2]);
+      a[k][3] = fmaf(p[k], mf, a[k][3]);
+      a[k][4] += et;
+    }
+    const int pc = process_class2<K, CHILD>(P);
+    const int tc = process_class2<K, CHILD>(t);
+    const bool counted = ok && !(CHILD && tc == 0);  // torchmetrics ignore_index=0 on child levels
+    cc.add(counted ? tc * NC + pc : -1);
+    if constexpr (CONS) {
+#pragma unroll
+      for (int g = 0; g < NG; ++g) {
+        float s = 0.f;
+        if constexpr (GSZ > 0) {
+#pragma unroll
+          for (int j = 0; j < GSZ; ++j) s += P[g * GSZ + j];
+        } else {
+#pragma unroll
+          for (int k = 0; k < K; ++k) s += (gr.group_of(k) == g) ? P[k] : 0.0f;
+        }
+        cs[g] += (ok && g < gr.n) ? fabsf(s - pp[g]) : 0.0f;
+      }
+    }
+  }
+
+  // Block reduction + one fp64 / int64 atomic per CTA and quantity, then the accumulators are cleared.
+  //   red: shared float[NWARP][NACC]; hist: shared int[NCELL] (zeroed by the caller before the first pixel and left
+  //   zeroed here); cons: the level's consistency slots, indexed by group.  sync / tid / nthreads as in EvalAcc.
+  template <int NWARP, typename SyncFn>
+  __device__ __forceinline__ void finish(float* red, int* hist, double* __restrict__ stats_b, double* __restrict__ cons,
+                                         unsigned long long* __restrict__ conf, int tid, int nthreads, SyncFn sync) {
+    const int lane = tid & 31, warp = tid >> 5;
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+#pragma unroll
+      for (int j = 0; j < NS; ++j) {
+        const float v = warp_sum(a[k][j]);
+        if (lane == 0) red[warp * NACC + k * NS + j] = v;
+        a[k][j] = 0.f;
+      }
+#pragma unroll
+    for (int g = 0; g < NCS; ++g) {
+      const float v = warp_sum(cs[g]);
+      if (lane == 0) red[warp * NACC + K * NS + g] = v;
+      cs[g] = 0.f;
+    }
+    cc.flush(hist);
+    sync();
+    if (tid < NACC) {
+      double acc = 0.0;
+#pragma unroll
+      for (int w = 0; w < NWARP; ++w) acc += (double)red[w * NACC + tid];
+      if (tid < K * NS) atomicAdd(&stats_b[tid], acc);
+      else if (acc != 0.0) atomicAdd(&cons[tid - K * NS], acc);
+    }
+    for (int i = tid; i < NCELL; i += nthreads)
+      if (hist[i]) { atomicAdd(&conf[i], (unsigned long long)hist[i]); hist[i] = 0; }
+    sync();
+  }
+};
+
+// ------------------------------------------------------------------------------------------------
 // Shared-memory stage ring.  bars[0..NS) = "full" (expect_tx bytes of the stage's copies, one producer arrival),
 // bars[NS..2NS) = "empty" (one arrival per consumer warp).  The producer is one elected lane.
 // ------------------------------------------------------------------------------------------------

@@ -364,6 +364,183 @@ static int launch_eval_pipe(const float* logits, const float* targets, long t_bs
 }
 
 // ------------------------------------------------------------------------------------
+// Per-level VALIDATION evaluation (the reference's test(), train.py:324-339; hires.cuh: ValAcc), ONE pass over the
+// logits, the composed probabilities, the ternary targets and, for the consistency term, the previous level's
+// probability plane of each group's parent.  Nothing is written but the fp64 / int64 sums.
+//   level_val_pipe_kernel  bulk-copy pipeline (16-byte aligned planes and target strides, N % 4 == 0): the same
+//                          even split and producer warp as level_eval_pipe_kernel; a consumer thread takes the stage's
+//                          pixels tid, tid + 256, ... straight from shared memory (conflict-free 4-byte reads), so
+//                          only one pixel's values are in registers at a time.
+//   level_val_kernel       any alignment and size: one pixel per thread, the group layout read from the table.
+// ------------------------------------------------------------------------------------
+template <int K, int CT, int GSZ>
+__host__ __device__ constexpr int vp_planes() { return 3 * K + (CT == 2 ? Groups<K, GSZ>::NG : 0); }
+// pixels per stage: a stage stays within 64 KB, so that three of them fit one CTA's shared memory
+template <int K, int CT, int GSZ>
+__host__ __device__ constexpr int vp_px() { return vp_planes<K, CT, GSZ>() <= 16 ? 1024 : 512; }
+constexpr int VP_STAGES = 3;
+
+template <int K, int CT, int GSZ>
+__global__ void __launch_bounds__(EVP_THREADS)
+level_val_pipe_kernel(const float* __restrict__ logits, const float* __restrict__ probs, const float* __restrict__ prev_probs,
+                      int K_prev, const float* __restrict__ targets, long t_bstride, long t_cstride,
+                      const int32_t* __restrict__ table, long N, long units_total, double* __restrict__ stats,
+                      double* __restrict__ cons, unsigned long long* __restrict__ conf) {
+  using Acc = ValAcc<K, CT, GSZ>;
+  constexpr bool CONS = CT == 2;
+  constexpr int NG = Groups<K, GSZ>::NG;
+  constexpr int PX = vp_px<K, CT, GSZ>(), PPT = PX / EVP_CONSUMERS;
+  constexpr int STAGE = vp_planes<K, CT, GSZ>() * PX * 4;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  __shared__ float red[EVP_CW * Acc::NACC];
+  __shared__ int hist[Acc::NCELL];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  StageRing ring;
+  ring.init(reinterpret_cast<uint64_t*>(smem_raw), VP_STAGES, EVP_CW);
+  unsigned char* stage0 = smem_raw + 128;
+  for (int i = tid; i < Acc::NCELL; i += EVP_THREADS) hist[i] = 0;
+  Groups<K, GSZ> gr;
+  gr.load(CT >= 1 ? table : nullptr);  // uploaded once per device: not produced by the previous kernel
+  const long g0 = (units_total * blockIdx.x / gridDim.x) * 4, g1 = (units_total * (blockIdx.x + 1) / gridDim.x) * 4;
+  int b = (int)(g0 / N);
+  long off = g0 - (long)b * N;
+  __syncthreads();
+  pdl_wait();
+
+  if (warp == EVP_CW) {
+    // ------------------------------ producer ------------------------------
+    if (lane == 0) {
+      int slot = 0;
+      uint32_t phase = 1;
+      for (long cur = g0; cur < g1;) {
+        const int len = (int)min((long)PX, min(N - off, g1 - cur));
+        mbar_wait(ring.empty(slot), phase);
+        const uint32_t dst = smem_u32(stage0 + (size_t)slot * STAGE), bar = ring.full(slot);
+        const uint32_t bytes = (uint32_t)len * 4u;
+        uint32_t total = 0;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+          bulk_g2s_plain(dst + k * PX * 4, logits + ((size_t)b * K + k) * N + off, bytes, bar);
+          bulk_g2s_plain(dst + (K + k) * PX * 4, probs + ((size_t)b * K + k) * N + off, bytes, bar);
+          bulk_g2s_plain(dst + (2 * K + k) * PX * 4, targets + (size_t)b * t_bstride + (size_t)k * t_cstride + off, bytes, bar);
+          total += 3 * bytes;
+        }
+        if constexpr (CONS) {
+#pragma unroll
+          for (int g = 0; g < NG; ++g)
+            if (g < gr.n) {
+              bulk_g2s_plain(dst + (3 * K + g) * PX * 4, prev_probs + ((size_t)b * K_prev + gr.parent[g]) * N + off, bytes, bar);
+              total += bytes;
+            }
+        }
+        mbar_arrive_expect_tx(bar, total);
+        if (++slot == VP_STAGES) { slot = 0; phase ^= 1u; }
+        cur += len;
+        off += len;
+        if (off == N) { off = 0; ++b; }
+      }
+    }
+    return;
+  }
+
+  // -------------------------------- consumers --------------------------------
+  auto csync = [] { consumer_sync(EVP_CONSUMERS); };
+  Acc ev;
+  ev.init();
+  int cur_b = b, slot = 0;
+  uint32_t phase = 0;
+  for (long cur = g0; cur < g1;) {
+    const int len = (int)min((long)PX, min(N - off, g1 - cur));
+    if (b != cur_b) {  // the range crosses into the next sample: hand over the finished sample's sums
+      ev.template finish<EVP_CW>(red, hist, stats + (size_t)cur_b * K * RHSEG_NSTAT, cons, conf, tid, EVP_CONSUMERS, csync);
+      cur_b = b;
+    }
+    mbar_wait(ring.full(slot), phase);
+    const float* sf = reinterpret_cast<const float*>(stage0 + (size_t)slot * STAGE);
+#pragma unroll 1
+    for (int v = 0; v < PPT; ++v) {
+      const int i = tid + v * EVP_CONSUMERS;
+      const bool ok = i < len;
+      float z[K], P[K], t[K], pp[NG], p[K], mx, sum;
+#pragma unroll
+      for (int k = 0; k < K; ++k) {  // stale shared memory past `len` may hold NaNs
+        z[k] = ok ? sf[k * PX + i] : 0.f;
+        P[k] = ok ? sf[(K + k) * PX + i] : 0.f;
+        t[k] = ok ? sf[(2 * K + k) * PX + i] : -1.f;
+      }
+#pragma unroll
+      for (int g = 0; g < NG; ++g) pp[g] = (CONS && ok && g < gr.n) ? sf[(3 * K + g) * PX + i] : 0.f;
+      softmax_all<K>(z, p, mx, sum);
+      ev.pixel(z, p, mx + log_fast(sum), t, P, pp, ok, gr);
+    }
+    __syncwarp();
+    if (lane == 0) mbar_arrive(ring.empty(slot));  // the warp is done with the stage: the producer may refill it
+    if (++slot == VP_STAGES) { slot = 0; phase ^= 1u; }
+    cur += len;
+    off += len;
+    if (off == N) { off = 0; ++b; }
+  }
+  if (g0 < g1) ev.template finish<EVP_CW>(red, hist, stats + (size_t)cur_b * K * RHSEG_NSTAT, cons, conf, tid, EVP_CONSUMERS, csync);
+}
+
+template <int K, int CT, int GSZ>
+static int launch_val_pipe(const float* logits, const float* probs, const float* prev_probs, int K_prev, const float* targets,
+                           long t_bs, long t_cs, const int32_t* table, int B, long N, double* stats, double* cons,
+                           unsigned long long* conf, cudaStream_t st) {
+  auto kern = level_val_pipe_kernel<K, CT, GSZ>;
+  const size_t smem = 128 + (size_t)VP_STAGES * vp_planes<K, CT, GSZ>() * vp_px<K, CT, GSZ>() * 4;
+  int per_sm = 0;
+  RHSEG_CUDA(cached_launch_prep(reinterpret_cast<const void*>(kern), EVP_THREADS, smem, smem, &per_sm));
+  if (per_sm < 1) return RHSEG_ERR_UNSUPPORTED;
+  const long units = (long)B * N / 4;
+  // every CTA gets at least two full stages of work; one resident wave at most
+  const long grid = std::max<long>(1, std::min<long>((long)device_sm_count() * per_sm, units / (2 * vp_px<K, CT, GSZ>() / 4)));
+  launch_pdl(kern, dim3((unsigned)grid), dim3(EVP_THREADS), smem, st, logits, probs, prev_probs, K_prev, targets, t_bs, t_cs,
+             table, N, units, stats, cons, conf);
+  RHSEG_LAUNCH_CHECK();
+  return RHSEG_OK;
+}
+
+template <int K, int CT>
+__global__ void __launch_bounds__(256)
+level_val_kernel(const float* __restrict__ logits, const float* __restrict__ probs, const float* __restrict__ prev_probs,
+                 int K_prev, const float* __restrict__ targets, long t_bstride, long t_cstride,
+                 const int32_t* __restrict__ table, long N, double* __restrict__ stats, double* __restrict__ cons,
+                 unsigned long long* __restrict__ conf) {
+  using Acc = ValAcc<K, CT, 0>;
+  constexpr int NG = Groups<K, 0>::NG;
+  __shared__ float red[8 * Acc::NACC];
+  __shared__ int hist[Acc::NCELL];
+  const int tid = threadIdx.x, b = blockIdx.y;
+  for (int i = tid; i < Acc::NCELL; i += 256) hist[i] = 0;
+  Groups<K, 0> gr;
+  gr.load(CT >= 1 ? table : nullptr);
+  __syncthreads();
+  pdl_wait();
+  Acc ev;
+  ev.init();
+  const float* zb = logits + (size_t)b * K * N;
+  const float* Pb = probs + (size_t)b * K * N;
+  for (long px0 = (long)blockIdx.x * 256; px0 < N; px0 += (long)gridDim.x * 256) {  // uniform trip count: ballots
+    const long px = px0 + tid;
+    const bool ok = px < N;
+    float z[K], P[K], t[K], pp[NG], p[K], mx, sum;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      z[k] = ok ? zb[(size_t)k * N + px] : 0.f;
+      P[k] = ok ? Pb[(size_t)k * N + px] : 0.f;
+      t[k] = ok ? targets[(size_t)b * t_bstride + (size_t)k * t_cstride + px] : -1.f;
+    }
+#pragma unroll
+    for (int g = 0; g < NG; ++g)
+      pp[g] = (CT == 2 && ok && g < gr.n) ? prev_probs[((size_t)b * K_prev + gr.parent[g]) * N + px] : 0.f;
+    softmax_all<K>(z, p, mx, sum);
+    ev.pixel(z, p, mx + log_fast(sum), t, P, pp, ok, gr);
+  }
+  ev.template finish<8>(red, hist, stats + (size_t)b * K * RHSEG_NSTAT, cons, conf, tid, 256, [] { __syncthreads(); });
+}
+
+// ------------------------------------------------------------------------------------
 // Flat -> hierarchy stitching (predictEval.py:85-185, :381-388): the flat model predicts the
 // leaves only; every node of the tree becomes one output channel: a leaf copies its flat channel,
 // a parent is the union (any > 0) of its descendant leaves.  Table driven: one uint32 leaf mask
@@ -542,6 +719,58 @@ extern "C" int rhseg_level_eval(const float* logits, const float* targets, long 
       launch_pdl(level_eval_kernel<KK, 1, (KK > 6 ? 1 : 2), THREADS>, dim3(grid), dim3(THREADS), 0, st, logits, targets, t_bstride, t_cstride, parent_targets,
           pt_bstride, pt_cstride, prev_idx, table, N, child, stats, cons, conf, idx_out);
     }
+  });
+  RHSEG_LAUNCH_CHECK();
+  return RHSEG_OK;
+}
+
+extern "C" int rhseg_level_eval_composed(const float* logits, const float* probs, const float* prev_probs,
+                                         const float* targets, long t_bstride, long t_cstride, const int32_t* table,
+                                         int B, int K, int K_prev, int n_pix, int child_arg, void* out_words, int flags,
+                                         void* stream) {
+  if (!logits || !probs || !targets || !out_words || B <= 0 || n_pix <= 0) return RHSEG_ERR_ARG;
+  if (K < 1 || K > RHSEG_KERNEL_MAX_K) return RHSEG_ERR_UNSUPPORTED;
+  const int child = child_arg & 1, hint = RHSEG_GROUP_HINT_OF(child_arg);
+  if (child && !table) return RHSEG_ERR_ARG;
+  const bool cons_in = child && prev_probs != nullptr;
+  if (cons_in && (K_prev < 1 || K_prev > RHSEG_KERNEL_MAX_K)) return RHSEG_ERR_ARG;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int nc = child ? K + 1 : K;
+  const size_t words = (size_t)B * K * RHSEG_NSTAT + RHSEG_MAX_K + (size_t)nc * nc;
+  if (!(flags & RHSEG_EVAL_PREZEROED)) RHSEG_CUDA(cudaMemsetAsync(out_words, 0, words * 8, st));
+  double* stats = reinterpret_cast<double*>(out_words);
+  double* cons = stats + (size_t)B * K * RHSEG_NSTAT;
+  unsigned long long* conf = reinterpret_cast<unsigned long long*>(cons + RHSEG_MAX_K);
+  const long N = n_pix;
+  // bulk copies need 16-byte sizes and addresses: every plane and target slice starts on a 16-byte boundary and
+  // every stage boundary (a multiple of 4 pixels) stays on one
+  const bool pipe = N % 4 == 0 && aligned16(logits) && aligned16(probs) && aligned16(targets) && t_bstride % 4 == 0 &&
+                    t_cstride % 4 == 0 && (!cons_in || aligned16(prev_probs)) && !getenv("RHSEG_NO_EVAL_PIPE");
+  if (pipe) {
+    RHSEG_DISPATCH_K(K, {
+      if (!child)
+        return launch_val_pipe<KK, 0, KK>(logits, probs, nullptr, 0, targets, t_bstride, t_cstride, nullptr, B, N, stats, cons, conf, st);
+      if (hint == KK) {
+        if (cons_in) return launch_val_pipe<KK, 2, KK>(logits, probs, prev_probs, K_prev, targets, t_bstride, t_cstride, table, B, N, stats, cons, conf, st);
+        return launch_val_pipe<KK, 1, KK>(logits, probs, nullptr, 0, targets, t_bstride, t_cstride, table, B, N, stats, cons, conf, st);
+      }
+      if constexpr (KK == 4) {
+        if (hint == 2) {  // two parents with two children each (extended tree, level 2)
+          if (cons_in) return launch_val_pipe<KK, 2, 2>(logits, probs, prev_probs, K_prev, targets, t_bstride, t_cstride, table, B, N, stats, cons, conf, st);
+          return launch_val_pipe<KK, 1, 2>(logits, probs, nullptr, 0, targets, t_bstride, t_cstride, table, B, N, stats, cons, conf, st);
+        }
+      }
+      if (cons_in) return launch_val_pipe<KK, 2, 0>(logits, probs, prev_probs, K_prev, targets, t_bstride, t_cstride, table, B, N, stats, cons, conf, st);
+      return launch_val_pipe<KK, 1, 0>(logits, probs, nullptr, 0, targets, t_bstride, t_cstride, table, B, N, stats, cons, conf, st);
+    });
+  }
+  constexpr int THREADS = 256;
+  const int slots = std::max(1, device_sm_count() * 4 / B);  // CTAs per sample for about one resident wave
+  const dim3 grid((unsigned)balanced_grid((N + THREADS - 1) / THREADS, slots), B);
+  RHSEG_DISPATCH_K(K, {
+    if (!child) launch_pdl(level_val_kernel<KK, 0>, grid, dim3(THREADS), 0, st, logits, probs, prev_probs, K_prev, targets, t_bstride, t_cstride, table, N, stats, cons, conf);
+    else if (cons_in) launch_pdl(level_val_kernel<KK, 2>, grid, dim3(THREADS), 0, st, logits, probs, prev_probs, K_prev, targets, t_bstride, t_cstride, table, N, stats, cons, conf);
+    else launch_pdl(level_val_kernel<KK, 1>, grid, dim3(THREADS), 0, st, logits, probs, prev_probs, K_prev, targets, t_bstride, t_cstride, table, N, stats, cons, conf);
   });
   RHSEG_LAUNCH_CHECK();
   return RHSEG_OK;

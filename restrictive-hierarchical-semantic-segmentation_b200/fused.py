@@ -68,33 +68,71 @@ def _eval_layout(tree: ClassTree, B: int):
     return offs, off
 
 
+def _step_target(tree: ClassTree, target: torch.Tensor):
+    """The wide ternary target as the evaluation kernels read it (fp32, contiguous H*W planes) and each level's first
+    channel in it."""
+    native.require_cuda(target)
+    target = widen_targets(target)
+    if target.dim() != 4 or target.shape[1] != sum(tree.head_channels):
+        raise native.NativeError("target must be [B, sum(K_L), H, W] with sum(K_L) = %d, got %s"
+                                 % (sum(tree.head_channels), tuple(target.shape)))
+    if not (target.stride(3) == 1 and target.stride(2) == target.shape[3]):
+        target = target.contiguous()
+    ch_off = [0]
+    for k in tree.head_channels:
+        ch_off.append(ch_off[-1] + k)
+    return target, ch_off
+
+
+def _check_eval_dims(target, dims):
+    if dims[0] != target.shape[0] or (dims[4], dims[5]) != tuple(target.shape[2:]):
+        raise native.NativeError("target %s does not match the head output [%d, *, %d, %d]"
+                                 % (tuple(target.shape), dims[0], dims[4], dims[5]))
+
+
+def _finalize(tree: ClassTree, ws, offs, weights_all, smooth, B, n_pix, n_active, xchg_tail, st):
+    """rhseg_step_finalize over the levels' evaluation words: (scalars + ratios, backward coefficients, summary with
+    `xchg_tail` free slots behind it, per-level confusion views, per-level ratio views)."""
+    n = tree.num_levels
+    dev = ws.device
+    n_ratio = sum(5 * o[3] for o in offs)
+    scal_all = torch.empty((2 + 4 * n + n_ratio,), dtype=torch.float32, device=dev)
+    coef_all = torch.empty((B * sum(tree.head_channels) * 3,), dtype=torch.float32, device=dev)
+    # [summary | xchg_tail slots for the parameter gradients]: the data-parallel exchange buffer
+    summary = torch.empty((2 + 4 * n + sum(o[3] * o[3] for o in offs) + int(xchg_tail),), dtype=torch.float64, device=dev)
+    Ks = (_I32 * n)(*tree.head_channels)
+    Gs = (_I32 * n)(*[tree.group_count(L) for L in range(n)])
+    call("rhseg_step_finalize", ptr(ws), ptr(weights_all), B, n, Ks, Gs, float(smooth), n_pix, (1 << n_active) - 1,
+         ptr(scal_all), ptr(coef_all), ptr(summary), st)
+    conf, ratios, r_off = [], [], 2 + 4 * n
+    for L in range(n):
+        nc = offs[L][3]
+        conf.append(ws[offs[L][2]:offs[L][2] + nc * nc].view(torch.int64).view(nc, nc))
+        ratios.append(scal_all[r_off:r_off + 5 * nc].view(5, nc))
+        r_off += 5 * nc
+    return scal_all, coef_all, summary, conf, ratios
+
+
+def _n_active(n, level_cap):
+    return n if level_cap is None else max(1, min(n, int(level_cap) + 1))  # train.py:121-126
+
+
 class _FusedStepFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, tree: ClassTree, out_size, weights_all, smooth, xchg_tail, level_cap, dp, target, *tensors):
         n = tree.num_levels
-        n_active = n if level_cap is None else max(1, min(n, int(level_cap) + 1))  # train.py:121-126
-        native.require_cuda(target)
-        target = widen_targets(target)
-        if target.dim() != 4 or target.shape[1] != sum(tree.head_channels):
-            raise native.NativeError("target must be [B, sum(K_L), H, W] with sum(K_L) = %d, got %s"
-                                     % (sum(tree.head_channels), tuple(target.shape)))
-        if not (target.stride(3) == 1 and target.stride(2) == target.shape[3]):
-            target = target.contiguous()
+        n_active = _n_active(n, level_cap)
+        target, ch_off = _step_target(tree, target)
         dev = target.device
         B = target.shape[0]
         t_bs, t_cs = target.stride(0), target.stride(1)
         esz = target.element_size()
-        ch_off = [0]
-        for k in tree.head_channels:
-            ch_off.append(ch_off[-1] + k)
         offs, words = _eval_layout(tree, B)
         idx_maps = [torch.empty((B,) + tuple(target.shape[2:]), dtype=torch.uint8, device=dev) if L < n - 1 else None
                     for L in range(n)]
 
         def evaluate(L, dims, ws):  # ws: the zeroed statistics workspace (part of the forward's single fill)
-            if dims[0] != B or (dims[4], dims[5]) != tuple(target.shape[2:]):
-                raise native.NativeError("target %s does not match the head output [%d, *, %d, %d]"
-                                         % (tuple(target.shape), dims[0], dims[4], dims[5]))
+            _check_eval_dims(target, dims)
             return (target.data_ptr() + ch_off[L] * t_cs * esz, t_bs, t_cs,
                     target.data_ptr() + ch_off[L - 1] * t_cs * esz if L > 0 else None,
                     ptr(idx_maps[L - 1]) if L > 0 else None, ws.data_ptr() + offs[L][0] * 8, ptr(idx_maps[L]))
@@ -105,17 +143,9 @@ class _FusedStepFn(torch.autograd.Function):
         ws = r["workspace"]
         B, C, Hf, Wf, H, W = r["dims"]
         st = stream_of(r["feats"][0])
-        n_pix = H * W
-        n_ratio = sum(5 * o[3] for o in offs)
-        scal_all = torch.empty((2 + 4 * n + n_ratio,), dtype=torch.float32, device=dev)
+        scal_all, coef_all, summary, conf, ratios = _finalize(tree, ws, offs, weights_all, smooth, B, H * W, n_active,
+                                                              xchg_tail, st)
         scalars = scal_all[:2 + 4 * n]
-        coef_all = torch.empty((B * sum(tree.head_channels) * 3,), dtype=torch.float32, device=dev)
-        # [summary | xchg_tail slots for the parameter gradients]: the data-parallel exchange buffer
-        summary = torch.empty((2 + 4 * n + sum(o[3] * o[3] for o in offs) + int(xchg_tail),), dtype=torch.float64, device=dev)
-        Ks = (_I32 * n)(*tree.head_channels)
-        Gs = (_I32 * n)(*[tree.group_count(L) for L in range(n)])
-        call("rhseg_step_finalize", ptr(ws), ptr(weights_all), B, n, Ks, Gs, float(smooth), n_pix, (1 << n_active) - 1,
-             ptr(scal_all), ptr(coef_all), ptr(summary), st)
         # data-parallel: the summary is summed over ranks BETWEEN forward and backward (a few hundred bytes), because the
         # exact Dice gradient needs the global count of valid samples (dist.py, rhseg_dp_grad_scales)
         n_summary = summary.numel() - int(xchg_tail)
@@ -128,12 +158,6 @@ class _FusedStepFn(torch.autograd.Function):
                 raise native.NativeError("the data-parallel summary reduction must not overwrite the local summary")
             ctx.dp = (summary, gsum, int(world))
         ctx.n_active = n_active
-        conf, ratios, r_off = [], [], 2 + 4 * n
-        for L in range(n):
-            nc = offs[L][3]
-            conf.append(ws[offs[L][2]:offs[L][2] + nc * nc].view(torch.int64).view(nc, nc))
-            ratios.append(scal_all[r_off:r_off + 5 * nc].view(5, nc))
-            r_off += 5 * nc
         ctx.tree, ctx.dims, ctx.upsampled = tree, r["dims"], r["upsampled"]
         ctx.t_meta = (t_bs, t_cs, ch_off, esz)
         ctx.save_for_backward(target, coef_all, *r["feats"], *r["head_w"], *r["film_w"], *r["logits"], *r["probs"],
@@ -277,6 +301,49 @@ class FusedHierStep:
         return StepOutput(outs[0], outs[1], list(outs[2:2 + n]), list(outs[2 + n:2 + 2 * n]),
                           list(outs[2 + 2 * n:2 + 3 * n]), list(outs[2 + 3 * n:2 + 4 * n]), n,
                           xbuf[:xbuf.numel() - self.exchange_tail], xbuf, gsum if gsum.numel() else None)
+
+    def validate(self, feats, head_w, head_b, film_w, film_b, target, out_size: Optional[Tuple[int, int]] = None,
+                 level_cap: Optional[int] = None, keep_outputs: bool = False) -> StepOutput:
+        """Validation pass of one batch: the numbers the reference's test() reports (train.py:282-393, evaluation at
+        :324-339), which are not those of the training step (DESIGN.md 3.9):
+          * metrics: ProcessClasses over the COMPOSED probabilities against the raw ternary targets (the step: argmax
+            of softmax(z) over all K logits, one-hot masked where the target is -1, against -1 -> 0 targets);
+          * consistency: on the real probabilities (the step: on the masked one-hots);
+          * CE and Dice: the same as the step's.
+        Arguments, level_cap, int8 targets and bf16 / channels-last features as in __call__.  Never records autograd,
+        whatever the grad mode (out.loss.requires_grad is False), allocates no backward buffers and never synchronises
+        with the host, so it can be captured in a CUDA graph.  keep_outputs=False: out.probs / out.logits are None and
+        only the previous level's probabilities stay alive while a level runs; True returns every level's.
+        out.summary is additive over batches and ranks: dist.unpack_global(sum of the summaries) gives the epoch's
+        numbers.  With data_parallel set, out.global_summary = reduce_fn(out.summary)."""
+        n = self.tree.num_levels
+        if not (len(feats) == len(head_w) == len(head_b) == n and len(film_w) == len(film_b) == n - 1):
+            raise native.NativeError("expected %d levels of features/heads and %d FiLMs" % (n, n - 1))
+        native.require_cuda(feats[0], target)
+        with torch.no_grad(), torch.cuda.device(feats[0].device):
+            tree = self.tree
+            target, ch_off = _step_target(tree, target)
+            B = target.shape[0]
+            t_bs, t_cs, esz = target.stride(0), target.stride(1), target.element_size()
+            offs, words = _eval_layout(tree, B)
+
+            def evaluate(L, dims, ws):
+                _check_eval_dims(target, dims)
+                return target.data_ptr() + ch_off[L] * t_cs * esz, t_bs, t_cs, ws.data_ptr() + offs[L][0] * 8
+
+            r = forward_levels(tree, out_size, (*feats, *head_w, *head_b, *film_w, *film_b), evaluate, zero_words=words,
+                               composed=True, keep_outputs=keep_outputs)
+            B, C, Hf, Wf, H, W = r["dims"]
+            scal_all, _, summary, conf, ratios = _finalize(tree, r["workspace"], offs, self.weights(target.device),
+                                                           self.smooth, B, H * W, _n_active(n, level_cap), 0,
+                                                           stream_of(r["feats"][0]))
+            gsum = None
+            if self._dp is not None:
+                gsum = self._dp[0](summary)
+                if gsum.data_ptr() == summary.data_ptr():
+                    raise native.NativeError("the data-parallel summary reduction must not overwrite the local summary")
+        probs, logits = (r["probs"], r["logits"]) if keep_outputs else ([None] * n, [None] * n)
+        return StepOutput(scal_all[0], scal_all[:2 + 4 * n], conf, ratios, probs, logits, n, summary, summary, gsum)
 
 
 class _FusedFlatFn(torch.autograd.Function):

@@ -60,6 +60,10 @@ _SIDE_STREAMS = {}
 #   "last": only the last level (nothing is left to overlap with)     "root": also level 0     "all": every level
 # Measured (DESIGN.md 6): HRNet-W48 tl "root" = "all" 0.420 ms vs "last" 0.428 ms; extended tree "all" is slower than "last".
 _FUSE_EVAL = os.environ.get("RHSEG_FUSE_EVAL", "root")
+# The same choice for the validation pass (forward_levels(composed=True), rhseg_head_level_fwd_eval with
+# RHSEG_EVAL_COMPOSED); the last level is always evaluated in its band kernel.  Measured (DESIGN.md 3.9, graph replay):
+# HRNet-W48 ext "all" 0.316 ms vs "root" 0.326 ms; tl the same for both (two levels: root and last)
+_FUSE_EVAL_VAL = os.environ.get("RHSEG_FUSE_EVAL", "all")
 
 
 def _side_stream(dev):
@@ -70,7 +74,8 @@ def _side_stream(dev):
     return _SIDE_STREAMS[key]
 
 
-def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words: int = 0, with_backward: bool = False):
+def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words: int = 0, with_backward: bool = False,
+                   composed: bool = False, keep_outputs: bool = True):
     """Runs the per-level forward kernels.  `tensors` = feats[n] + head_w[n] + head_b[n] + film_w[n-1] +
     film_b[n-1]; the features are fp32 or bf16, contiguous or channels-last (_feats_c), everything else fp32.
     Returns a dict with the inputs (as the kernels read them) and probs / logits / psums / eff_w /
@@ -80,7 +85,14 @@ def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words
     inside the hi-res forward kernel (upsampled heads) or right after the level's forward (feature-resolution heads).
     `zero_words` extra fp64 words are zeroed by the same fill as the pool sums / low-res logits and handed to
     `evaluate` as its third argument (the fused step's statistics workspace).  with_backward: the same fill also
-    zeroes the accumulators of the backward pass (r["bwd"], see backward_buffers): ONE fill per training step."""
+    zeroes the accumulators of the backward pass (r["bwd"], see backward_buffers): ONE fill per training step.
+    composed (validation, FusedHierStep.validate): `evaluate(L, dims, ws)` returns (targets_ptr, t_bs, t_cs,
+    out_words_ptr) and the level is evaluated on its logits, its probabilities and the previous level's: by
+    rhseg_level_eval_composed, every level but the last on the side stream, concurrent with the next level's forward, or
+    (upsampled heads, the last level and the levels _FUSE_EVAL_VAL names) inside the band forward
+    (rhseg_head_level_fwd_eval with RHSEG_EVAL_COMPOSED).
+    keep_outputs=False: each level's logits and probabilities are released as soon as nothing queued later reads
+    them (r["probs"] / r["logits"] hold None), so at most two levels' outputs are alive at a time."""
     n = tree.num_levels
     feats, fflags = _feats_c(tensors[0:n])
     head_w = [_f32c(t) for t in tensors[n:2 * n]]
@@ -140,6 +152,36 @@ def forward_levels(tree: ClassTree, out_size, tensors, evaluate=None, zero_words
             zlo_off += B * K * Hf * Wf
         ev = evaluate(L, (B, C, Hf, Wf, H, W), workspace) if evaluate is not None else None
         hint = tree.group_hint(L)  # uniform group size: kernels with the group layout fixed at compile time
+        if composed:
+            p_prev = probs[L - 1] if L > 0 else None
+            fused = ev is not None and upsampled and (L == n - 1 or _FUSE_EVAL_VAL == "all" or (_FUSE_EVAL_VAL == "root" and L == 0))
+            if fused:  # evaluated inside the band kernel while z, P and the parent probabilities are in registers
+                t_ptr, t_bs, t_cs, words_ptr = ev
+                call("rhseg_head_level_fwd_eval", ptr(f), ptr(eff_w), ptr(eff_b), ptr(p_prev), ptr(tables[L]),
+                     B, C, Hf, Wf, H, W, K, K_prev, tree.act_mode[L] | hint, ptr(z_lo), ptr(z), ptr(p), ptr(psum),
+                     t_ptr, t_bs, t_cs, None, 0, 0, None, words_ptr, None, native.EVAL_COMPOSED | 1 | 2 | shared | fbf, st)
+            else:
+                call("rhseg_head_level_fwd", ptr(f), ptr(eff_w), ptr(eff_b), ptr(p_prev), ptr(tables[L]),
+                     B, C, Hf, Wf, H, W, K, K_prev, tree.act_mode[L] | hint, ptr(z_lo), ptr(z), ptr(p), ptr(psum), (2 if upsampled else 0) | shared | fbf, st)
+            if ev is not None and not fused:
+                t_ptr, t_bs, t_cs, words_ptr = ev
+                eval_st = st
+                if L < n - 1:  # nothing downstream waits for the sums: overlap with the next level's forward
+                    side = _side_stream(dev)
+                    side.wait_stream(torch.cuda.current_stream(dev))
+                    eval_st, used_side = side.cuda_stream, True
+                    if not keep_outputs:  # the caching allocator must not hand these out before the side stream is done
+                        for t in (z, p, p_prev):
+                            if t is not None:
+                                t.record_stream(side)
+                call("rhseg_level_eval_composed", ptr(z), ptr(p), ptr(p_prev), t_ptr, t_bs, t_cs, ptr(tables[L]),
+                     B, K, K_prev, n_pix, (1 if L > 0 else 0) | hint, words_ptr, 1, eval_st)
+            if not keep_outputs:
+                z = None
+                if L > 0:
+                    probs[L - 1] = None
+            probs.append(p); logits.append(z); psums.append(psum); eff_ws.append(eff_w); gbs.append(gb)
+            continue
         # The evaluation of level L only needs its logits (and the previous level's index map): for all
         # but the last level it runs on a side stream, overlapping the (memory-bound) forward of the next
         # level; the last level's evaluation is fused into its hi-res forward kernel when there is one.

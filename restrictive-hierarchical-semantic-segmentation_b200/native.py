@@ -18,6 +18,7 @@ TABLE_INTS = 4 + 5 * MAX_K
 NSTAT = 5
 XCHG_HANDLE_BYTES = 64
 DZ_PREZEROED = 1
+EVAL_COMPOSED = 0x40  # RHSEG_EVAL_COMPOSED: rhseg_head_level_fwd_eval evaluates what rhseg_level_eval_composed does
 FEATS_BF16 = 0x10  # RHSEG_FEATS_BF16: the feature (and dfeats) tensors of the call are bf16
 FEATS_NHWC = 0x20  # RHSEG_FEATS_NHWC: the feature (and dfeats) tensors of the call are channels-last [B,H,W,C]
 ACT_SIGMOID, ACT_GROUPED, ACT_ZEROS = 0, 1, 2
@@ -60,6 +61,7 @@ SIGNATURES = {
     "rhseg_step_finalize": [_P, _P, _I, _I, _P, _P, _D, _L, _U, _P, _P, _P, _P],
     "rhseg_dp_grad_scales": [_P, _P, _I, _I, _P, _P, _P],
     "rhseg_level_eval": [_P, _P, _L, _L, _P, _L, _L, _P, _P, _I, _I, _I, _I, _P, _P, _I, _P],
+    "rhseg_level_eval_composed": [_P, _P, _P, _P, _L, _L, _P, _I, _I, _I, _I, _I, _P, _I, _P],
     "rhseg_targets_i8_to_f32": [_P, _L, _P, _P],
     "rhseg_concat_image_logits": [_P, _I, _P, _I, _I, _I, _P, _P],
     "rhseg_stitch_levels": [_P, _I, _I, _I, _P, _I, _P, _P],
