@@ -50,6 +50,14 @@ extern "C" {
  * order, and dfeats too for the same dz; see DESIGN.md 3.8 for when they are bit-identical.  The
  * low-resolution logits of upsampled heads and the fp64 sums agree to rounding.                */
 #define RHSEG_FEATS_NHWC 0x20
+/* Logit element type flag, OR-ed into the `flags` of rhseg_level_eval, the `act_mode` of rhseg_head_dz_fullres_fused and
+ * the `logits_input` of rhseg_loss_stats and rhseg_loss_bwd: set, the logits (outs) are bf16 and dz / dz_out is written
+ * as bf16 (a flat head run under bf16 autocast); clear, both are fp32.  Each bf16 logit is converted to fp32 exactly
+ * when it is loaded; every other tensor and every sum keeps its type, and the gradient is formed in fp32 and rounded to
+ * bf16 (nearest even) once, when stored.  So the results equal the fp32 path's on the upcast logits.  Only the flat
+ * model's calls take it: rhseg_level_eval at the root level (child 0, no parent targets, prev_idx or idx_out) and
+ * rhseg_head_dz_fullres_fused with RHSEG_ACT_ZEROS; any other combination returns RHSEG_ERR_UNSUPPORTED.          */
+#define RHSEG_LOGITS_BF16 0x80
 #define RHSEG_NSTAT 5            /* per (sample, class) loss statistics, see loss_stats   */
 #define RHSEG_MAX_LEVELS 8       /* tree depth rhseg_step_finalize handles in one launch  */
 #define RHSEG_STITCH_MAX_LEAVES 16 /* leaf channels of a flat model rhseg_stitch_levels reads */
@@ -236,8 +244,9 @@ int rhseg_head_param_grads(const double* S, const double* s, const float* head_w
  *   [0] sum_m t*lp   [1] |m|   [2] sum_m p*t   [3] sum_m p   [4] sum_m t,   m = (t != -1)
  * logits_input != 0: lp = log_softmax(outs), p = softmax(outs) over the K channels;
  * otherwise lp = p = outs (the modules' logits_input=False mode).  Zeroes `stats` first.
+ * logits_input & RHSEG_LOGITS_BF16: outs is bf16 (either mode).
  * targets: element (b,k,n) at targets[b*t_bstride + k*t_cstride + n].                    */
-int rhseg_loss_stats(const float* outs, const float* targets, long t_bstride, long t_cstride,
+int rhseg_loss_stats(const void* outs, const float* targets, long t_bstride, long t_cstride,
                      int B, int K, int n_pix, int logits_input, double* stats, void* stream);
 
 /* Scalars from the statistics (one tiny launch):
@@ -252,9 +261,10 @@ int rhseg_loss_finalize(const double* stats, const float* weights, int B, int K,
 
 /* d(g_ce*CE + g_dice*Dice)/d outs -> dz [B,K,n_pix] (written, not accumulated).
  * g_ce / g_dice are DEVICE scalars (autograd's upstream gradients; NULL -> 0).            */
-int rhseg_loss_bwd(const float* outs, const float* targets, long t_bstride, long t_cstride,
+int rhseg_loss_bwd(const void* outs, const float* targets, long t_bstride, long t_cstride,
                    const float* coef, const float* g_ce, const float* g_dice,
-                   int B, int K, int n_pix, int logits_input, float* dz, void* stream);
+                   int B, int K, int n_pix, int logits_input, void* dz, void* stream);
+/* logits_input & RHSEG_LOGITS_BF16: outs and dz are bf16.                                  */
 
 /* Consistency term of one (level, parent-group set): for each group g of `table`,
  * sums[g] = sum_{b,n} | sum_{c in g} cur[b,c,n] - prev[b,parent(g),n] |  (fp64, zeroed here).
@@ -294,12 +304,13 @@ int rhseg_confusion_from_logits(const float* logits, const float* targets, long 
                                 int B, int K, int n_pix, int child, int64_t* conf, void* stream);
 
 /* Same fused gradient for full-resolution heads (UNet): dz_out [B,K,n_pix] written once. */
-int rhseg_head_dz_fullres_fused(const float* logits, const float* targets, long t_bstride, long t_cstride,
+int rhseg_head_dz_fullres_fused(const void* logits, const float* targets, long t_bstride, long t_cstride,
                                 const float* coef, const float* g_ce, const float* g_dice,
                                 const float* prev_probs, const int32_t* table, const double* g_uniform,
                                 double inv_npix, const float* dp_pix, uint32_t pix_mask,
                                 int B, int K, int K_prev, int n_pix, int act_mode,
-                                float* dz_out, float* dp_prev, void* stream);
+                                void* dz_out, float* dp_prev, void* stream);
+/* act_mode & RHSEG_LOGITS_BF16: logits and dz_out are bf16 (RHSEG_ACT_ZEROS only).          */
 
 /* All levels of one training step from the rhseg_level_eval workspaces (stored back to back in
  * level order), one launch:  out[0] = total = sum_L (CE_L + Dice_L) + consistency
@@ -335,9 +346,10 @@ int rhseg_dp_grad_scales(const double* local_summary, const double* global_summa
  *   out_words (8-byte words, zeroed here):
  *     [B*K*RHSEG_NSTAT fp64 statistics][RHSEG_MAX_K fp64 consistency sums][nc*nc int64 confusion]
  *   idx_out: uint8 [B,n_pix] prediction index map (NULL when no deeper level needs it).
- *   flags: RHSEG_EVAL_PREZEROED = the caller already zeroed out_words (one fill for all levels).
+ *   flags: RHSEG_EVAL_PREZEROED = the caller already zeroed out_words (one fill for all levels);
+ *          RHSEG_LOGITS_BF16 = logits are bf16 (level 0 only).
  *   child: 0 / 1, optionally | RHSEG_GROUP_HINT(gsz).                                          */
-int rhseg_level_eval(const float* logits, const float* targets, long t_bstride, long t_cstride,
+int rhseg_level_eval(const void* logits, const float* targets, long t_bstride, long t_cstride,
                      const float* parent_targets, long pt_bstride, long pt_cstride,
                      const unsigned char* prev_idx, const int32_t* table, int B, int K, int n_pix,
                      int child, void* out_words, unsigned char* idx_out, int flags, void* stream);

@@ -4,6 +4,7 @@
 // :150-177 (hierarchical_consistency_loss).
 #include <math.h>
 #include "common.cuh"
+#include "logits_io.cuh"
 
 namespace rhseg {
 
@@ -12,10 +13,11 @@ __device__ __forceinline__ bool vec_ok_ptr(const void* p) { return (reinterpret_
 // ------------------------------------------------------------------------------------
 // statistics pass.  grid = (chunks, B); each thread handles ITER vectors of VEC pixels.
 // per (b, c): [0] sum_m t*lp  [1] |m|  [2] sum_m p*t  [3] sum_m p  [4] sum_m t
+// LT: logit element type (float, or uint16_t = bf16 bits, widened at the load: logits_io.cuh)
 // ------------------------------------------------------------------------------------
-template <int K, int VEC, int ITER, int THREADS, bool LOGITS>
+template <int K, int VEC, int ITER, int THREADS, bool LOGITS, typename LT = float>
 __global__ void __launch_bounds__(THREADS)
-loss_stats_kernel(const float* __restrict__ outs, const float* __restrict__ targets, long t_bstride,
+loss_stats_kernel(const LT* __restrict__ outs, const float* __restrict__ targets, long t_bstride,
                   long t_cstride, long N, double* __restrict__ stats) {
   pdl_wait();
   constexpr int NWARP = THREADS / 32;
@@ -28,7 +30,7 @@ loss_stats_kernel(const float* __restrict__ outs, const float* __restrict__ targ
 #pragma unroll
     for (int j = 0; j < NS; ++j) a[k][j] = 0.f;
 
-  const float* ob = outs + (size_t)b * K * N;
+  const LT* ob = outs + (size_t)b * K * N;
   const float* tb = targets + (size_t)b * t_bstride;
   const long chunk0 = (long)blockIdx.x * (THREADS * VEC * ITER);
 #pragma unroll
@@ -416,11 +418,11 @@ step_finalize_kernel(const double* __restrict__ ws, const float* __restrict__ we
 //   logits:  dz_k = (a_k - p_k sum_c a_c) + p_k (g_k - sum_c g_c p_c)
 //   raw:     dz_k = a_k + g_k
 // ------------------------------------------------------------------------------------
-template <int K, int VEC, int THREADS, bool LOGITS>
+template <int K, int VEC, int THREADS, bool LOGITS, typename LT = float>
 __global__ void __launch_bounds__(THREADS)
-loss_bwd_kernel(const float* __restrict__ outs, const float* __restrict__ targets, long t_bstride,
+loss_bwd_kernel(const LT* __restrict__ outs, const float* __restrict__ targets, long t_bstride,
                 long t_cstride, const float* __restrict__ coef, const float* __restrict__ g_ce,
-                const float* __restrict__ g_dice, long N, float* __restrict__ dz) {
+                const float* __restrict__ g_dice, long N, LT* __restrict__ dz) {
   pdl_wait();
   const int b = blockIdx.y;
   const long px = ((long)blockIdx.x * THREADS + threadIdx.x) * VEC;
@@ -434,7 +436,7 @@ loss_bwd_kernel(const float* __restrict__ outs, const float* __restrict__ target
     Bc[k] = gdi * __ldg(cf + 1);
     Cc[k] = gdi * __ldg(cf + 2);
   }
-  const float* ob = outs + (size_t)b * K * N + px;
+  const LT* ob = outs + (size_t)b * K * N + px;
   const float* tb = targets + (size_t)b * t_bstride + px;
   float z[K][VEC], t[K][VEC];
 #pragma unroll
@@ -454,13 +456,13 @@ loss_bwd_kernel(const float* __restrict__ outs, const float* __restrict__ target
 #pragma unroll
     for (int k = 0; k < K; ++k) o[k][v] = ov[k];
   }
-  float* db = dz + (size_t)b * K * N + px;
+  LT* db = dz + (size_t)b * K * N + px;
 #pragma unroll
   for (int k = 0; k < K; ++k) {
     Vec<VEC> r;
 #pragma unroll
     for (int v = 0; v < VEC; ++v) r.v[v] = o[k][v];
-    *reinterpret_cast<Vec<VEC>*>(db + (size_t)k * N) = r;  // consumed right away by the head backward
+    st_grad<VEC>(db + (size_t)k * N, r);  // consumed right away by the head backward
   }
 }
 
@@ -528,27 +530,58 @@ static bool can_vec4(const void* a, const void* b, long s0, long s1, long N) {
 
 using namespace rhseg;
 
-extern "C" int rhseg_loss_stats(const float* outs, const float* targets, long t_bstride, long t_cstride, int B,
+namespace rhseg {
+template <typename LT>
+static int loss_stats_launch(const LT* outs, const float* targets, long t_bstride, long t_cstride, int B, int K, long N,
+                             bool logits, double* stats, cudaStream_t st) {
+  constexpr int THREADS = 256, ITER = 4;
+  RHSEG_DISPATCH_K(K, {
+    if (can_vec4(outs, targets, t_bstride, t_cstride, N)) {
+      dim3 grid((unsigned)((N + THREADS * 4 * ITER - 1) / (THREADS * 4 * ITER)), B);
+      if (logits) launch_pdl(loss_stats_kernel<KK, 4, ITER, THREADS, true, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
+      else launch_pdl(loss_stats_kernel<KK, 4, ITER, THREADS, false, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
+    } else {
+      dim3 grid((unsigned)((N + THREADS * ITER - 1) / (THREADS * ITER)), B);
+      if (logits) launch_pdl(loss_stats_kernel<KK, 1, ITER, THREADS, true, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
+      else launch_pdl(loss_stats_kernel<KK, 1, ITER, THREADS, false, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
+    }
+  });
+  RHSEG_LAUNCH_CHECK();
+  return RHSEG_OK;
+}
+
+template <typename LT>
+static int loss_bwd_launch(const LT* outs, const float* targets, long t_bstride, long t_cstride, const float* coef,
+                           const float* g_ce, const float* g_dice, int B, int K, long N, bool logits, LT* dz,
+                           cudaStream_t st) {
+  constexpr int THREADS = 256;
+  RHSEG_DISPATCH_K(K, {
+    if (can_vec4(outs, targets, t_bstride, t_cstride, N) && ((reinterpret_cast<uintptr_t>(dz) & 15u) == 0)) {
+      dim3 grid((unsigned)((N / 4 + THREADS - 1) / THREADS), B);
+      if (logits) launch_pdl(loss_bwd_kernel<KK, 4, THREADS, true, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
+      else launch_pdl(loss_bwd_kernel<KK, 4, THREADS, false, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
+    } else {
+      dim3 grid((unsigned)((N + THREADS - 1) / THREADS), B);
+      if (logits) launch_pdl(loss_bwd_kernel<KK, 1, THREADS, true, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
+      else launch_pdl(loss_bwd_kernel<KK, 1, THREADS, false, LT>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
+    }
+  });
+  RHSEG_LAUNCH_CHECK();
+  return RHSEG_OK;
+}
+}  // namespace rhseg
+
+// logits_input: 0 / 1 (outs are probabilities / logits), optionally | RHSEG_LOGITS_BF16
+extern "C" int rhseg_loss_stats(const void* outs, const float* targets, long t_bstride, long t_cstride, int B,
                                 int K, int n_pix, int logits_input, double* stats, void* stream) {
   if (!outs || !targets || !stats || B <= 0 || n_pix <= 0) return RHSEG_ERR_ARG;
   if (K < 1 || K > RHSEG_KERNEL_MAX_K) return RHSEG_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
   RHSEG_CUDA(cudaMemsetAsync(stats, 0, sizeof(double) * (size_t)B * K * RHSEG_NSTAT, st));
-  const long N = n_pix;
-  constexpr int THREADS = 256, ITER = 4;
-  RHSEG_DISPATCH_K(K, {
-    if (can_vec4(outs, targets, t_bstride, t_cstride, N)) {
-      dim3 grid((unsigned)((N + THREADS * 4 * ITER - 1) / (THREADS * 4 * ITER)), B);
-      if (logits_input) launch_pdl(loss_stats_kernel<KK, 4, ITER, THREADS, true>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
-      else launch_pdl(loss_stats_kernel<KK, 4, ITER, THREADS, false>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
-    } else {
-      dim3 grid((unsigned)((N + THREADS * ITER - 1) / (THREADS * ITER)), B);
-      if (logits_input) launch_pdl(loss_stats_kernel<KK, 1, ITER, THREADS, true>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
-      else launch_pdl(loss_stats_kernel<KK, 1, ITER, THREADS, false>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, N, stats);
-    }
-  });
-  RHSEG_LAUNCH_CHECK();
-  return RHSEG_OK;
+  const bool logits = (logits_input & ~RHSEG_LOGITS_BF16) != 0;
+  if (logits_input & RHSEG_LOGITS_BF16)
+    return loss_stats_launch(static_cast<const uint16_t*>(outs), targets, t_bstride, t_cstride, B, K, n_pix, logits, stats, st);
+  return loss_stats_launch(static_cast<const float*>(outs), targets, t_bstride, t_cstride, B, K, n_pix, logits, stats, st);
 }
 
 extern "C" int rhseg_loss_finalize(const double* stats, const float* weights, int B, int K, double smooth,
@@ -559,27 +592,18 @@ extern "C" int rhseg_loss_finalize(const double* stats, const float* weights, in
   return RHSEG_OK;
 }
 
-extern "C" int rhseg_loss_bwd(const float* outs, const float* targets, long t_bstride, long t_cstride,
+extern "C" int rhseg_loss_bwd(const void* outs, const float* targets, long t_bstride, long t_cstride,
                               const float* coef, const float* g_ce, const float* g_dice, int B, int K, int n_pix,
-                              int logits_input, float* dz, void* stream) {
+                              int logits_input, void* dz, void* stream) {
   if (!outs || !targets || !coef || !dz || B <= 0 || n_pix <= 0) return RHSEG_ERR_ARG;
   if (K < 1 || K > RHSEG_KERNEL_MAX_K) return RHSEG_ERR_UNSUPPORTED;
   cudaStream_t st = (cudaStream_t)stream;
-  const long N = n_pix;
-  constexpr int THREADS = 256;
-  RHSEG_DISPATCH_K(K, {
-    if (can_vec4(outs, targets, t_bstride, t_cstride, N) && ((reinterpret_cast<uintptr_t>(dz) & 15u) == 0)) {
-      dim3 grid((unsigned)((N / 4 + THREADS - 1) / THREADS), B);
-      if (logits_input) launch_pdl(loss_bwd_kernel<KK, 4, THREADS, true>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
-      else launch_pdl(loss_bwd_kernel<KK, 4, THREADS, false>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
-    } else {
-      dim3 grid((unsigned)((N + THREADS - 1) / THREADS), B);
-      if (logits_input) launch_pdl(loss_bwd_kernel<KK, 1, THREADS, true>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
-      else launch_pdl(loss_bwd_kernel<KK, 1, THREADS, false>, dim3(grid), dim3(THREADS), 0, st, outs, targets, t_bstride, t_cstride, coef, g_ce, g_dice, N, dz);
-    }
-  });
-  RHSEG_LAUNCH_CHECK();
-  return RHSEG_OK;
+  const bool logits = (logits_input & ~RHSEG_LOGITS_BF16) != 0;
+  if (logits_input & RHSEG_LOGITS_BF16)
+    return loss_bwd_launch(static_cast<const uint16_t*>(outs), targets, t_bstride, t_cstride, coef, g_ce, g_dice, B, K, n_pix,
+                           logits, static_cast<uint16_t*>(dz), st);
+  return loss_bwd_launch(static_cast<const float*>(outs), targets, t_bstride, t_cstride, coef, g_ce, g_dice, B, K, n_pix,
+                         logits, static_cast<float*>(dz), st);
 }
 
 extern "C" int rhseg_consistency_sums(const float* cur, const float* prev, const int32_t* table, int B, int K,

@@ -7,6 +7,7 @@
 #include "common.cuh"
 #include "eval_accum.cuh"
 #include "hires.cuh"
+#include "logits_io.cuh"
 
 namespace rhseg {
 
@@ -152,10 +153,11 @@ __global__ void metric_ratios_kernel(const long long* __restrict__ conf, int nc,
 //     (losses.py:150-177 as train_epoch calls it, train.py:237-239)
 // so neither the one-hot tensors nor the eval targets are ever materialised.
 // out layout (8-byte words): [B*K*5 fp64 stats][RHSEG_MAX_K fp64 consistency sums][nc*nc int64 confusion]
+// LT: logit element type (float, or uint16_t = bf16 bits of a flat head under autocast, widened at the load)
 // ------------------------------------------------------------------------------------
-template <int K, int VEC, int MINB, int THREADS, int CT = -1>
+template <int K, int VEC, int MINB, int THREADS, int CT = -1, typename LT = float>
 __global__ void __launch_bounds__(THREADS, MINB)
-level_eval_kernel(const float* __restrict__ logits, const float* __restrict__ targets, long t_bstride, long t_cstride,
+level_eval_kernel(const LT* __restrict__ logits, const float* __restrict__ targets, long t_bstride, long t_cstride,
                   const float* __restrict__ parent_targets, long pt_bstride, long pt_cstride,
                   const unsigned char* __restrict__ prev_idx, const int32_t* __restrict__ table, long N, int child,
                   double* __restrict__ stats, double* __restrict__ cons, unsigned long long* __restrict__ conf,
@@ -166,7 +168,7 @@ level_eval_kernel(const float* __restrict__ logits, const float* __restrict__ ta
   const int b = blockIdx.y, tid = threadIdx.x;
   EvalAccum<K, CT> ev;
   ev.init(child, child && prev_idx != nullptr && parent_targets != nullptr, table, hist, THREADS);
-  const float* zb = logits + (size_t)b * K * N;
+  const LT* zb = logits + (size_t)b * K * N;
   // persistent over the sample's pixel vectors: one resident wave, statistics reduced once per CTA
   for (long px0 = (long)blockIdx.x * (THREADS * VEC); px0 < N; px0 += (long)gridDim.x * (THREADS * VEC)) {
     const long px = px0 + (long)tid * VEC;
@@ -206,14 +208,16 @@ level_eval_kernel(const float* __restrict__ logits, const float* __restrict__ ta
 // ------------------------------------------------------------------------------------
 constexpr int EVP_CW = 8, EVP_CONSUMERS = EVP_CW * 32, EVP_THREADS = EVP_CONSUMERS + 32, EVP_PX = EVP_CONSUMERS * 4;
 
-template <int K, int CT, int GSZ>
+// stage layout: K logit planes (EVP_PX elements of LT each), then K target planes, the NG parent target planes and the
+// index map (fp32 / uint8)
+template <int K, int CT, int GSZ, typename LT = float>
 __host__ __device__ constexpr int evp_stage_bytes() {
-  return (2 * K + (CT == 2 ? Groups<K, GSZ>::NG : 0)) * EVP_PX * 4 + (CT == 2 ? EVP_PX : 0);
+  return K * EVP_PX * (int)sizeof(LT) + (K + (CT == 2 ? Groups<K, GSZ>::NG : 0)) * EVP_PX * 4 + (CT == 2 ? EVP_PX : 0);
 }
 
-template <int K, int CT, int GSZ>
+template <int K, int CT, int GSZ, typename LT = float>
 __global__ void __launch_bounds__(EVP_THREADS)
-level_eval_pipe_kernel(const float* __restrict__ logits, const float* __restrict__ targets, long t_bstride, long t_cstride,
+level_eval_pipe_kernel(const LT* __restrict__ logits, const float* __restrict__ targets, long t_bstride, long t_cstride,
                        const float* __restrict__ parent_targets, long pt_bstride, long pt_cstride,
                        const unsigned char* __restrict__ prev_idx, const int32_t* __restrict__ table, long N,
                        long units_total, int ns, double* __restrict__ stats, double* __restrict__ cons,
@@ -221,7 +225,8 @@ level_eval_pipe_kernel(const float* __restrict__ logits, const float* __restrict
   using Acc = EvalAcc<K, CT, GSZ>;
   constexpr bool CONS = CT == 2;
   constexpr int NG = Groups<K, GSZ>::NG;
-  constexpr int STAGE = evp_stage_bytes<K, CT, GSZ>();
+  constexpr int STAGE = evp_stage_bytes<K, CT, GSZ, LT>();
+  constexpr int ZF = K * EVP_PX * (int)sizeof(LT) / 4;  // 4-byte words of a stage's logit planes
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ float red[EVP_CW * Acc::NACC];
   __shared__ int hist[Acc::NCELL];
@@ -249,23 +254,23 @@ level_eval_pipe_kernel(const float* __restrict__ logits, const float* __restrict
         const int len = (int)min((long)EVP_PX, min(N - off, g1 - cur));
         mbar_wait(ring.empty(slot), phase);
         const uint32_t dst = smem_u32(stage0 + (size_t)slot * STAGE), bar = ring.full(slot);
-        const uint32_t bytes = (uint32_t)len * 4u;
+        const uint32_t bytes = (uint32_t)len * 4u, zbytes = (uint32_t)len * (uint32_t)sizeof(LT);
         uint32_t total = 0;
 #pragma unroll
         for (int k = 0; k < K; ++k) {
-          bulk_g2s_plain(dst + k * EVP_PX * 4, logits + ((size_t)b * K + k) * N + off, bytes, bar);
-          bulk_g2s_plain(dst + (K + k) * EVP_PX * 4, targets + (size_t)b * t_bstride + (size_t)k * t_cstride + off, bytes, bar);
-          total += 2 * bytes;
+          bulk_g2s_plain(dst + k * EVP_PX * (int)sizeof(LT), logits + ((size_t)b * K + k) * N + off, zbytes, bar);
+          bulk_g2s_plain(dst + (ZF + k * EVP_PX) * 4, targets + (size_t)b * t_bstride + (size_t)k * t_cstride + off, bytes, bar);
+          total += zbytes + bytes;
         }
         if constexpr (CONS) {
 #pragma unroll
           for (int g = 0; g < NG; ++g)
             if (g < gr.n) {
-              bulk_g2s_plain(dst + (2 * K + g) * EVP_PX * 4,
+              bulk_g2s_plain(dst + (ZF + (K + g) * EVP_PX) * 4,
                              parent_targets + (size_t)b * pt_bstride + (size_t)gr.parent[g] * pt_cstride + off, bytes, bar);
               total += bytes;
             }
-          bulk_g2s_plain(dst + (2 * K + NG) * EVP_PX * 4, prev_idx + (size_t)b * N + off, (uint32_t)len, bar);
+          bulk_g2s_plain(dst + (ZF + (K + NG) * EVP_PX) * 4, prev_idx + (size_t)b * N + off, (uint32_t)len, bar);
           total += (uint32_t)len;
         }
         mbar_arrive_expect_tx(bar, total);
@@ -300,21 +305,26 @@ level_eval_pipe_kernel(const float* __restrict__ logits, const float* __restrict
       unsigned pidx4 = 0u;
 #pragma unroll
       for (int k = 0; k < K; ++k) {
-        const float4 zv = *reinterpret_cast<const float4*>(sf + k * EVP_PX + tid * 4);
-        const float4 tv = *reinterpret_cast<const float4*>(sf + (K + k) * EVP_PX + tid * 4);
-        z[k][0] = zv.x; z[k][1] = zv.y; z[k][2] = zv.z; z[k][3] = zv.w;
+        if constexpr (std::is_same_v<LT, float>) {
+          const float4 zv = *reinterpret_cast<const float4*>(sf + k * EVP_PX + tid * 4);
+          z[k][0] = zv.x; z[k][1] = zv.y; z[k][2] = zv.z; z[k][3] = zv.w;
+        } else {  // bf16: four logits in 8 bytes, widened exactly
+          const uint2 zv = *reinterpret_cast<const uint2*>(reinterpret_cast<const uint16_t*>(sf) + k * EVP_PX + tid * 4);
+          z[k][0] = bf16_lo(zv.x); z[k][1] = bf16_hi(zv.x); z[k][2] = bf16_lo(zv.y); z[k][3] = bf16_hi(zv.y);
+        }
+        const float4 tv = *reinterpret_cast<const float4*>(sf + ZF + k * EVP_PX + tid * 4);
         t[k][0] = tv.x; t[k][1] = tv.y; t[k][2] = tv.z; t[k][3] = tv.w;
       }
 #pragma unroll
       for (int g = 0; g < NG; ++g) {
         if (CONS && g < gr.n) {
-          const float4 pv = *reinterpret_cast<const float4*>(sf + (2 * K + g) * EVP_PX + tid * 4);
+          const float4 pv = *reinterpret_cast<const float4*>(sf + ZF + (K + g) * EVP_PX + tid * 4);
           ptg[g][0] = pv.x; ptg[g][1] = pv.y; ptg[g][2] = pv.z; ptg[g][3] = pv.w;
         } else {
           ptg[g][0] = ptg[g][1] = ptg[g][2] = ptg[g][3] = -1.0f;
         }
       }
-      if constexpr (CONS) pidx4 = *reinterpret_cast<const unsigned*>(reinterpret_cast<const unsigned char*>(sf + (2 * K + NG) * EVP_PX) + tid * 4);
+      if constexpr (CONS) pidx4 = *reinterpret_cast<const unsigned*>(reinterpret_cast<const unsigned char*>(sf + ZF + (K + NG) * EVP_PX) + tid * 4);
       __syncwarp();
       if (lane == 0) mbar_arrive(ring.empty(slot));  // the stage is in registers: the producer may refill the slot
       unsigned my_idx = 0u;
@@ -341,12 +351,12 @@ level_eval_pipe_kernel(const float* __restrict__ logits, const float* __restrict
   if (g0 < g1) ev.template finish<EVP_CW>(red, cred, hist, stats + (size_t)cur_b * K * RHSEG_NSTAT, cons, conf, tid, EVP_CONSUMERS, csync);
 }
 
-template <int K, int CT, int GSZ>
-static int launch_eval_pipe(const float* logits, const float* targets, long t_bs, long t_cs, const float* parent_targets,
+template <int K, int CT, int GSZ, typename LT = float>
+static int launch_eval_pipe(const LT* logits, const float* targets, long t_bs, long t_cs, const float* parent_targets,
                             long pt_bs, long pt_cs, const unsigned char* prev_idx, const int32_t* table, int B, long N,
                             double* stats, double* cons, unsigned long long* conf, unsigned char* idx_out, cudaStream_t st) {
-  auto kern = level_eval_pipe_kernel<K, CT, GSZ>;
-  constexpr int STAGE = evp_stage_bytes<K, CT, GSZ>();
+  auto kern = level_eval_pipe_kernel<K, CT, GSZ, LT>;
+  constexpr int STAGE = evp_stage_bytes<K, CT, GSZ, LT>();
   static int tune = -1;
   if (tune < 0) { const char* e = getenv("RHSEG_TUNE_EVAL"); tune = e ? atoi(e) : 0; }
   const int ns = tune == 1 ? 3 : (tune == 2 ? 4 : 2);
@@ -611,6 +621,29 @@ static int confusion_launch(const float* probs, long p_bs, long p_cs, const floa
   return RHSEG_OK;
 }
 
+// generic path of rhseg_level_eval: any alignment, any size (level kind decided at run time)
+template <typename LT>
+static int launch_eval_generic(const LT* logits, const float* targets, long t_bstride, long t_cstride,
+                               const float* parent_targets, long pt_bstride, long pt_cstride, const unsigned char* prev_idx,
+                               const int32_t* table, int B, int K, long N, int child, bool v4, double* stats, double* cons,
+                               unsigned long long* conf, unsigned char* idx_out, cudaStream_t st) {
+  constexpr int THREADS = 256;
+  const int slots = std::max(1, device_sm_count() * 2 / B);  // CTAs per sample for one resident wave
+  RHSEG_DISPATCH_K(K, {
+    if (v4 && KK <= 4) {  // 4 pixels per thread spill beyond K = 4 at two CTAs per SM: wider levels take one pixel per thread
+      dim3 grid((unsigned)balanced_grid((N + THREADS * 4 - 1) / (THREADS * 4), slots), B);
+      launch_pdl(level_eval_kernel<(KK <= 4 ? KK : 1), 4, 2, THREADS, -1, LT>, dim3(grid), dim3(THREADS), 0, st, logits, targets, t_bstride, t_cstride,
+          parent_targets, pt_bstride, pt_cstride, prev_idx, table, N, child, stats, cons, conf, idx_out);
+    } else {
+      dim3 grid((unsigned)balanced_grid((N + THREADS - 1) / THREADS, slots), B);
+      launch_pdl(level_eval_kernel<KK, 1, (KK > 6 ? 1 : 2), THREADS, -1, LT>, dim3(grid), dim3(THREADS), 0, st, logits, targets, t_bstride, t_cstride,
+          parent_targets, pt_bstride, pt_cstride, prev_idx, table, N, child, stats, cons, conf, idx_out);
+    }
+  });
+  RHSEG_LAUNCH_CHECK();
+  return RHSEG_OK;
+}
+
 }  // namespace rhseg
 
 using namespace rhseg;
@@ -663,13 +696,16 @@ extern "C" int rhseg_metric_ratios(const int64_t* conf, int nc, float* out5, voi
   return RHSEG_OK;
 }
 
-extern "C" int rhseg_level_eval(const float* logits, const float* targets, long t_bstride, long t_cstride,
+extern "C" int rhseg_level_eval(const void* logits_in, const float* targets, long t_bstride, long t_cstride,
                                 const float* parent_targets, long pt_bstride, long pt_cstride,
                                 const unsigned char* prev_idx, const int32_t* table, int B, int K, int n_pix,
                                 int child_arg, void* out_words, unsigned char* idx_out, int flags, void* stream) {
-  if (!logits || !targets || !out_words || B <= 0 || n_pix <= 0) return RHSEG_ERR_ARG;
+  if (!logits_in || !targets || !out_words || B <= 0 || n_pix <= 0) return RHSEG_ERR_ARG;
   if (K < 1 || K > RHSEG_KERNEL_MAX_K) return RHSEG_ERR_UNSUPPORTED;
   const int child = child_arg & 1, hint = RHSEG_GROUP_HINT_OF(child_arg);
+  // bf16 logits come from the flat model: its one (root) level only, no consistency inputs or index map
+  const bool bf16 = (flags & RHSEG_LOGITS_BF16) != 0;
+  if (bf16 && (child || parent_targets || prev_idx || idx_out)) return RHSEG_ERR_UNSUPPORTED;
   if (child && !table) return RHSEG_ERR_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   const int nc = child ? K + 1 : K;
@@ -679,12 +715,17 @@ extern "C" int rhseg_level_eval(const float* logits, const float* targets, long 
   double* cons = stats + (size_t)B * K * RHSEG_NSTAT;
   unsigned long long* conf = reinterpret_cast<unsigned long long*>(cons + RHSEG_MAX_K);
   const long N = n_pix;
-  constexpr int THREADS = 256;
-  bool v4 = (N % 4 == 0) && aligned16(logits) && aligned16(targets) && t_bstride % 4 == 0 && t_cstride % 4 == 0 &&
+  bool v4 = (N % 4 == 0) && aligned16(logits_in) && aligned16(targets) && t_bstride % 4 == 0 && t_cstride % 4 == 0 &&
             (reinterpret_cast<uintptr_t>(prev_idx) % 4 == 0) && (reinterpret_cast<uintptr_t>(idx_out) % 4 == 0);
   if (parent_targets) v4 = v4 && aligned16(parent_targets) && pt_bstride % 4 == 0 && pt_cstride % 4 == 0;
   const bool cons_in = child && prev_idx != nullptr && parent_targets != nullptr;
   const bool pipe = v4 && N % 16 == 0 && aligned16(prev_idx) && (long)B * N >= 4 * EVP_PX && !getenv("RHSEG_NO_EVAL_PIPE");
+  if (bf16) {
+    const uint16_t* z16 = static_cast<const uint16_t*>(logits_in);
+    if (pipe) RHSEG_DISPATCH_K(K, return (launch_eval_pipe<KK, 0, KK, uint16_t>(z16, targets, t_bstride, t_cstride, nullptr, 0, 0, nullptr, nullptr, B, N, stats, cons, conf, nullptr, st)));
+    return launch_eval_generic(z16, targets, t_bstride, t_cstride, nullptr, 0, 0, nullptr, table, B, K, N, 0, v4, stats, cons, conf, nullptr, st);
+  }
+  const float* logits = static_cast<const float*>(logits_in);
   if (pipe) {
     // level kind and group structure fixed at compile time: no flag tests per pixel
     RHSEG_DISPATCH_K(K, {
@@ -707,21 +748,8 @@ extern "C" int rhseg_level_eval(const float* logits, const float* targets, long 
       return launch_eval_pipe<KK, 1, 0>(logits, targets, t_bstride, t_cstride, nullptr, 0, 0, nullptr, table, B, N, stats, cons, conf, idx_out, st);
     });
   }
-  // generic path: any alignment, any size (level kind decided at run time)
-  const int slots = std::max(1, device_sm_count() * 2 / B);  // CTAs per sample for one resident wave
-  RHSEG_DISPATCH_K(K, {
-    if (v4 && KK <= 4) {  // 4 pixels per thread spill beyond K = 4 at two CTAs per SM: wider levels take one pixel per thread
-      dim3 grid((unsigned)balanced_grid((N + THREADS * 4 - 1) / (THREADS * 4), slots), B);
-      launch_pdl(level_eval_kernel<(KK <= 4 ? KK : 1), 4, 2, THREADS>, dim3(grid), dim3(THREADS), 0, st, logits, targets, t_bstride, t_cstride, parent_targets,
-          pt_bstride, pt_cstride, prev_idx, table, N, child, stats, cons, conf, idx_out);
-    } else {
-      dim3 grid((unsigned)balanced_grid((N + THREADS - 1) / THREADS, slots), B);
-      launch_pdl(level_eval_kernel<KK, 1, (KK > 6 ? 1 : 2), THREADS>, dim3(grid), dim3(THREADS), 0, st, logits, targets, t_bstride, t_cstride, parent_targets,
-          pt_bstride, pt_cstride, prev_idx, table, N, child, stats, cons, conf, idx_out);
-    }
-  });
-  RHSEG_LAUNCH_CHECK();
-  return RHSEG_OK;
+  return launch_eval_generic(logits, targets, t_bstride, t_cstride, parent_targets, pt_bstride, pt_cstride, prev_idx, table, B, K, N,
+                             child, v4, stats, cons, conf, idx_out, st);
 }
 
 extern "C" int rhseg_level_eval_composed(const float* logits, const float* probs, const float* prev_probs,

@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include "common.cuh"
 #include "hires.cuh"
+#include "logits_io.cuh"
 
 namespace rhseg {
 
@@ -550,10 +551,11 @@ static int launch_dz_band(const float* dz_hi, const FusedDzArgs& fa, int B, int 
   return RHSEG_OK;
 }
 
-// Full-resolution donors (UNet): the same fused per-pixel gradient, written out once as dz.
-template <int K, int VEC, int MODE, int THREADS>
+// Full-resolution donors (UNet): the same fused per-pixel gradient, written out once as dz.  LT: logit and dz element
+// type (float, or uint16_t = bf16 bits: fa.logits then points at bf16 values; RHSEG_ACT_ZEROS only).
+template <int K, int VEC, int MODE, int THREADS, typename LT = float>
 __global__ void __launch_bounds__(THREADS)
-dz_fullres_fused_kernel(FusedDzArgs fa, long N, float* __restrict__ dz_out) {
+dz_fullres_fused_kernel(FusedDzArgs fa, long N, LT* __restrict__ dz_out) {
   pdl_wait();
   const int b = blockIdx.y;
   const long px = ((long)blockIdx.x * THREADS + threadIdx.x) * VEC;
@@ -573,7 +575,7 @@ dz_fullres_fused_kernel(FusedDzArgs fa, long N, float* __restrict__ dz_out) {
   float z[K][VEC], t[K][VEC], e[K][VEC], pp[K][VEC], o[K][VEC], dpar[K][VEC];
 #pragma unroll
   for (int k = 0; k < K; ++k) {
-    const Vec<VEC> zv = ld_stream<VEC>(fa.logits + ((size_t)b * K + k) * N + px);
+    const Vec<VEC> zv = ld_stream<VEC>(reinterpret_cast<const LT*>(fa.logits) + ((size_t)b * K + k) * N + px);
     const Vec<VEC> tv = ld_cached<VEC>(fa.targets + (size_t)b * fa.t_bstride + (size_t)k * fa.t_cstride + px);
     Vec<VEC> ev;
 #pragma unroll
@@ -612,7 +614,7 @@ dz_fullres_fused_kernel(FusedDzArgs fa, long N, float* __restrict__ dz_out) {
     Vec<VEC> r;
 #pragma unroll
     for (int v = 0; v < VEC; ++v) r.v[v] = o[k][v];
-    *reinterpret_cast<Vec<VEC>*>(dz_out + ((size_t)b * K + k) * N + px) = r;  // re-read by the conv backward: keep cached
+    st_grad<VEC>(dz_out + ((size_t)b * K + k) * N + px, r);  // re-read by the conv backward: keep cached
   }
   if constexpr (MODE == RHSEG_ACT_GROUPED) {
     if (has_act && fa.dp_prev) {
@@ -737,35 +739,47 @@ extern "C" int rhseg_head_dz_lowres_fused(const float* logits, const float* targ
   return RHSEG_OK;
 }
 
-extern "C" int rhseg_head_dz_fullres_fused(const float* logits, const float* targets, long t_bstride, long t_cstride,
+extern "C" int rhseg_head_dz_fullres_fused(const void* logits, const float* targets, long t_bstride, long t_cstride,
                                            const float* coef, const float* g_ce, const float* g_dice,
                                            const float* prev_probs, const int32_t* table, const double* g_uniform,
                                            double inv_npix, const float* dp_pix, uint32_t pix_mask, int B, int K,
-                                           int K_prev, int n_pix, int act_mode, float* dz_out, float* dp_prev,
+                                           int K_prev, int n_pix, int act_mode, void* dz_out, float* dp_prev,
                                            void* stream) {
   if (!logits || !targets || !coef || !dz_out || B <= 0 || n_pix <= 0) return RHSEG_ERR_ARG;
   if (K < 1 || K > RHSEG_KERNEL_MAX_K) return RHSEG_ERR_UNSUPPORTED;
-  act_mode &= 0xff;
+  const bool bf16 = (act_mode & RHSEG_LOGITS_BF16) != 0;
+  act_mode &= 0xff & ~RHSEG_LOGITS_BF16;
+  if (bf16 && act_mode != RHSEG_ACT_ZEROS) return RHSEG_ERR_UNSUPPORTED;  // only the flat model's logits are bf16
   if (act_mode == RHSEG_ACT_GROUPED && (!prev_probs || !table)) return RHSEG_ERR_ARG;
-  FusedDzArgs fa{logits, targets, t_bstride, t_cstride, coef, g_ce, g_dice, prev_probs, table, g_uniform,
-                 (float)inv_npix, dp_pix, pix_mask, dp_prev, K_prev};
+  // bf16: fa.logits carries the bf16 pointer; the kernel instance reads it as such
+  FusedDzArgs fa{static_cast<const float*>(logits), targets, t_bstride, t_cstride, coef, g_ce, g_dice, prev_probs, table,
+                 g_uniform, (float)inv_npix, dp_pix, pix_mask, dp_prev, K_prev};
   cudaStream_t st = (cudaStream_t)stream;
   const long N = n_pix;
   constexpr int THREADS = 256;
   auto al = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   const bool v4 = (N % 4 == 0) && al(logits) && al(targets) && t_bstride % 4 == 0 && t_cstride % 4 == 0 && al(dz_out) &&
                   al(prev_probs) && al(dp_pix) && al(dp_prev);
+  const dim3 grid((unsigned)(v4 ? (N / 4 + THREADS - 1) / THREADS : (N + THREADS - 1) / THREADS), B);
+  if (bf16) {
+    auto* dz = static_cast<uint16_t*>(dz_out);
+    RHSEG_DISPATCH_K(K, {
+      if (v4) launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_ZEROS, THREADS, uint16_t>, grid, dim3(THREADS), 0, st, fa, N, dz);
+      else launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_ZEROS, THREADS, uint16_t>, grid, dim3(THREADS), 0, st, fa, N, dz);
+    });
+    RHSEG_LAUNCH_CHECK();
+    return RHSEG_OK;
+  }
+  float* dz = static_cast<float*>(dz_out);
   RHSEG_DISPATCH_K(K, {
     if (v4) {
-      dim3 grid((unsigned)((N / 4 + THREADS - 1) / THREADS), B);
-      if (act_mode == RHSEG_ACT_SIGMOID) launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_SIGMOID, THREADS>, dim3(grid), dim3(THREADS), 0, st, fa, N, dz_out);
-      else if (act_mode == RHSEG_ACT_GROUPED) launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_GROUPED, THREADS>, dim3(grid), dim3(THREADS), 0, st, fa, N, dz_out);
-      else launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_ZEROS, THREADS>, dim3(grid), dim3(THREADS), 0, st, fa, N, dz_out);
+      if (act_mode == RHSEG_ACT_SIGMOID) launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_SIGMOID, THREADS>, grid, dim3(THREADS), 0, st, fa, N, dz);
+      else if (act_mode == RHSEG_ACT_GROUPED) launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_GROUPED, THREADS>, grid, dim3(THREADS), 0, st, fa, N, dz);
+      else launch_pdl(dz_fullres_fused_kernel<KK, 4, RHSEG_ACT_ZEROS, THREADS>, grid, dim3(THREADS), 0, st, fa, N, dz);
     } else {
-      dim3 grid((unsigned)((N + THREADS - 1) / THREADS), B);
-      if (act_mode == RHSEG_ACT_SIGMOID) launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_SIGMOID, THREADS>, dim3(grid), dim3(THREADS), 0, st, fa, N, dz_out);
-      else if (act_mode == RHSEG_ACT_GROUPED) launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_GROUPED, THREADS>, dim3(grid), dim3(THREADS), 0, st, fa, N, dz_out);
-      else launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_ZEROS, THREADS>, dim3(grid), dim3(THREADS), 0, st, fa, N, dz_out);
+      if (act_mode == RHSEG_ACT_SIGMOID) launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_SIGMOID, THREADS>, grid, dim3(THREADS), 0, st, fa, N, dz);
+      else if (act_mode == RHSEG_ACT_GROUPED) launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_GROUPED, THREADS>, grid, dim3(THREADS), 0, st, fa, N, dz);
+      else launch_pdl(dz_fullres_fused_kernel<KK, 1, RHSEG_ACT_ZEROS, THREADS>, grid, dim3(THREADS), 0, st, fa, N, dz);
     }
   });
   RHSEG_LAUNCH_CHECK();

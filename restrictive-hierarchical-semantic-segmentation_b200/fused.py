@@ -350,13 +350,13 @@ class _FusedFlatFn(torch.autograd.Function):
     """Flat model (model_type 0; Models/models.py:258-261, :754-757): weighted CE + Dice on the logits of ONE level of
     leaf classes, the train-path prediction and the confusion-matrix metrics, in three launches: rhseg_level_eval
     (statistics + bit-exact argmax(softmax) + confusion, one pass over logits and targets), rhseg_step_finalize,
-    and rhseg_head_dz_fullres_fused in the backward (closed-form gradient, one pass)."""
+    and rhseg_head_dz_fullres_fused in the backward (closed-form gradient, one pass).  bf16 logits (a flat head run under
+    bf16 autocast) are read as such (RHSEG_LOGITS_BF16): the results are those of the fp32 step on logits.float(), and
+    the gradient comes back as bf16, rounded once."""
 
     @staticmethod
     def forward(ctx, tree: ClassTree, weights, smooth, logits, target):
         native.require_cuda(logits, target)
-        if logits.dtype != torch.float32:
-            raise native.NativeError("flat step expects float32 logits, got %s" % logits.dtype)
         z = logits if logits.is_contiguous() else logits.contiguous()
         t = widen_targets(target)
         if not (t.stride(3) == 1 and t.stride(2) == t.shape[3]):
@@ -371,7 +371,7 @@ class _FusedFlatFn(torch.autograd.Function):
         ws = torch.zeros((words,), dtype=torch.float64, device=dev)
         tables = tree.device_tables(dev)
         call("rhseg_level_eval", ptr(z), ptr(t), t.stride(0), t.stride(1), None, 0, 0, None, ptr(tables[0]), B, K, n_pix, 0,
-             ptr(ws), None, 1, st)
+             ptr(ws), None, native.EVAL_PREZEROED | native.logits_flag(z), st)
         scal_all = torch.empty((2 + 4 + 5 * K,), dtype=torch.float32, device=dev)
         coef = torch.empty((B * K * 3,), dtype=torch.float32, device=dev)
         summary = torch.empty((2 + 4 + K * K,), dtype=torch.float64, device=dev)
@@ -396,7 +396,8 @@ class _FusedFlatFn(torch.autograd.Function):
         g = g if g.dtype == torch.float32 else g.float()
         dz = torch.empty_like(z)
         call("rhseg_head_dz_fullres_fused", ptr(z), ptr(t), t.stride(0), t.stride(1), ptr(coef), ptr(g), ptr(g), None, ptr(table),
-             None, 1.0 / (H * W), None, 0, B, K, 0, H * W, native.ACT_ZEROS, ptr(dz), None, stream_of(z))  # no activation path:
+             None, 1.0 / (H * W), None, 0, B, K, 0, H * W, native.ACT_ZEROS | native.logits_flag(z), ptr(dz), None,
+             stream_of(z))  # no activation path:
         # nothing but the loss reaches the flat logits (the instance without activation code: 108 vs 138 registers at K = 7)
         return None, None, None, dz, None
 
@@ -421,6 +422,9 @@ class FusedFlatStep:
         self.smooth = float(smooth)
 
     def __call__(self, logits, target) -> StepOutput:
+        """logits: float32, or bfloat16 (a flat head under bf16 autocast: the results are the fp32 step's on
+        logits.float(), and the gradient reaching the logits is bf16)."""
+        native.check_logits_dtype(logits, "flat step")
         key = str(logits.device)
         if key not in self._weights:
             self._weights[key] = torch.tensor(self._weights_host, dtype=torch.float32).to(logits.device)

@@ -47,10 +47,9 @@ def _plane_contiguous(t: torch.Tensor) -> torch.Tensor:
 class _LevelLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, outs, targets, weights, smooth, logits_input, token):
+        native.check_logits_dtype(outs, "losses")
         native.require_cuda(outs, targets, weights)
         ctx.token = token
-        if outs.dtype != torch.float32:
-            raise native.NativeError("losses expect float32 predictions, got %s" % outs.dtype)
         outs = outs if outs.is_contiguous() else outs.contiguous()
         targets = _plane_contiguous(targets)
         B, K = outs.shape[0], outs.shape[1]
@@ -64,7 +63,7 @@ class _LevelLossFn(torch.autograd.Function):
         out4 = torch.empty((4,), dtype=torch.float32, device=dev)
         coef = torch.empty((B, K, 3), dtype=torch.float32, device=dev)
         call("rhseg_loss_stats", ptr(outs), ptr(targets), targets.stride(0), targets.stride(1), B, K, n_pix,
-             1 if logits_input else 0, ptr(stats), st)
+             (1 if logits_input else 0) | native.logits_flag(outs), ptr(stats), st)
         call("rhseg_loss_finalize", ptr(stats), ptr(weights), B, K, float(smooth), ptr(out4), ptr(coef), st)
         ctx.save_for_backward(outs, targets, coef)
         ctx.logits_input = logits_input
@@ -88,9 +87,10 @@ class _LevelLossFn(torch.autograd.Function):
             return g if g.dtype == torch.float32 else g.float()
 
         g_ce, g_dice = scalar(g_ce), scalar(g_dice)
-        dz = torch.empty_like(outs)
+        dz = torch.empty_like(outs)  # bf16 predictions get a bf16 gradient
         call("rhseg_loss_bwd", ptr(outs), ptr(targets), targets.stride(0), targets.stride(1), ptr(coef),
-             ptr(g_ce), ptr(g_dice), B, K, n_pix, 1 if ctx.logits_input else 0, ptr(dz), stream_of(outs))
+             ptr(g_ce), ptr(g_dice), B, K, n_pix, (1 if ctx.logits_input else 0) | native.logits_flag(outs), ptr(dz),
+             stream_of(outs))
         return dz, None, None, None, None, None
 
 

@@ -18,9 +18,11 @@ TABLE_INTS = 4 + 5 * MAX_K
 NSTAT = 5
 XCHG_HANDLE_BYTES = 64
 DZ_PREZEROED = 1
+EVAL_PREZEROED = 1
 EVAL_COMPOSED = 0x40  # RHSEG_EVAL_COMPOSED: rhseg_head_level_fwd_eval evaluates what rhseg_level_eval_composed does
 FEATS_BF16 = 0x10  # RHSEG_FEATS_BF16: the feature (and dfeats) tensors of the call are bf16
 FEATS_NHWC = 0x20  # RHSEG_FEATS_NHWC: the feature (and dfeats) tensors of the call are channels-last [B,H,W,C]
+LOGITS_BF16 = 0x80  # RHSEG_LOGITS_BF16: the logits (and the gradient written for them) of the call are bf16
 ACT_SIGMOID, ACT_GROUPED, ACT_ZEROS = 0, 1, 2
 
 _c = ctypes
@@ -155,6 +157,18 @@ def require_cuda(*tensors):
         if t is not None and not t.is_cuda:
             raise NativeError("rhseg_b200 kernels need CUDA tensors (got a %s tensor); there is no CPU fallback"
                               % t.device.type)
+
+
+def check_logits_dtype(t, what):
+    """Logits / predictions the loss and flat-step kernels read: float32, or bfloat16 (a head run under bf16 autocast).
+    Checked before the device, so that a CPU tensor of another dtype names the dtype."""
+    if t.dtype not in (torch.float32, torch.bfloat16):
+        raise NativeError("%s: expected float32 or bfloat16 logits, got %s" % (what, t.dtype))
+
+
+def logits_flag(t) -> int:
+    """RHSEG_LOGITS_BF16 for a bf16 logit tensor, 0 for fp32."""
+    return LOGITS_BF16 if t.dtype == torch.bfloat16 else 0
 
 
 def call(name, *args):
